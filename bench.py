@@ -1,13 +1,13 @@
 #!/usr/bin/env python
 """bench.py — LLaMA-7B FP32 decode tokens/sec on B200 (BASELINE.json metric), one JSON line.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): LLaMA-7B FP32, context 512, predict 128 — a 384-token
 synthetic prompt is prefilled (untimed setup), then single-token decode steps are timed.
 A "step" = one decoded token per in-flight sequence (N sequences at N GPUs, see DESIGN.md §multi-GPU).
   value : whole-job decode tokens/s, tokens/KV/weights resident in HBM, K CUDA-graph replays timed
-          with CUDA events on the engine's stream (lb_decode_resident).
+          with CUDA events on the engine's stream (lb_decode_resident).  Every timed region is exactly K steps.
   e2e   : the same K steps through the public API lb_eval() with HOST buffers: token id H2D and
           128 KB logits D2H inside the timed region, one synchronous call per token.
   roofline    : dominant kernel = the decode megakernel (one launch per token): algorithmic bytes of a token
@@ -16,8 +16,11 @@ A "step" = one decoded token per in-flight sequence (N sequences at N GPUs, see 
   cpu_baseline: the reference's own binary (--avx, all host threads) on a bounded sample.
 --impl reference times the reference's own CPU implementation (oracle/_ref/llama-go-linux).
 Weights (26.4 GB/token) are far larger than L2 (126 MB): no flush needed between iterations.
+--dump-outputs DIR writes the logits of the last timed step of every measured decode path to DIR/<name>.npy
+(float32), so that two builds run with the same arguments (same seeded inputs) can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import shutil
@@ -64,6 +67,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(
                 ["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100", "-i", str(self.gpu)],
                 stdout=open(self.path, "w"), stderr=subprocess.DEVNULL)
+            atexit.register(self.proc.kill)      # a measurement that raises before stop() must not leave it running
         except Exception:
             self.proc = None
 
@@ -100,7 +104,7 @@ class ClockSampler:
 
 # --------------------------------------------------------------------------------------------- reference arm
 def _scratch_dir(need_bytes):
-    for d in ("/dev/shm", tempfile.gettempdir(), ROOT):
+    for d in ("/dev/shm", tempfile.gettempdir()):
         try:
             if shutil.disk_usage(d).free > need_bytes * 1.2:
                 return tempfile.mkdtemp(prefix="lb_ref_", dir=d)
@@ -319,13 +323,6 @@ def compare_with_reference_stream(llama, synth, model):
         return {"equal": None, "error": str(e)}
 
 
-def _repeats_for(K, est_ms_per_step, target_s=2.0, cap=64):
-    """How many times the K-step timed region is repeated so that the clocks sampler (100 ms period) sees
-    >= ~2 s of load even at the driver's --steps 20 (0.09 s per region).  Every region is exactly K steps,
-    bracketed by CUDA events; the reported time is the mean over the regions."""
-    return int(min(cap, max(1, np.ceil(target_s / max(1e-6, K * est_ms_per_step / 1e3)))))
-
-
 def measure_decode(llama, lib, hp, q8, ctx_size, K, W, sampler=None):
     """One single-GPU decode measurement: model (device RNG, seed 0) + context, prompt prefill, `value` (device
     resident, CUDA events) and `e2e` (lb_eval with host buffers).  Returns a dict that keeps model/lctx alive."""
@@ -343,44 +340,40 @@ def measure_decode(llama, lib, hp, q8, ctx_size, K, W, sampler=None):
     prefill_s = time.perf_counter() - t0
 
     # ---- value: device-resident decode, CUDA events on the engine's stream
-    w_ms = llama.DecodeResident(lctx, gen[:max(W, 1)], PROMPT_LEN)    # warm-up (also captures the CUDA graph)
-    w_ms = llama.DecodeResident(lctx, gen[:max(W, 1)], PROMPT_LEN)
+    llama.DecodeResident(lctx, gen[:max(W, 1)], PROMPT_LEN)    # warm-up (also captures the CUDA graph)
+    llama.DecodeResident(lctx, gen[:max(W, 1)], PROMPT_LEN)
     lib.lb_context_synchronize(lctx._h)
-    R = _repeats_for(K, w_ms / max(W, 1))
     if sampler:
         sampler.start()
     l0 = lib.lb_kernel_launches()
-    reps = [llama.DecodeResident(lctx, gen[W:W + K], PROMPT_LEN + W) for _ in range(R)]
+    ms = llama.DecodeResident(lctx, gen[W:W + K], PROMPT_LEN + W)
     lib.lb_context_synchronize(lctx._h)
-    launches = (lib.lb_kernel_launches() - l0) // R
-    ms = float(np.mean(reps))
+    launches = lib.lb_kernel_launches() - l0
     value = K / (ms / 1e3)
+    logits = llama.ReadLogits(lctx).copy()              # the last timed step's row, before e2e overwrites it
 
     # ---- e2e: public API, host buffers, one synchronous lb_eval per token
     for i in range(W):
         llama.Eval(lctx, gen[i:i + 1], PROMPT_LEN + i)
     lib.lb_context_synchronize(lctx._h)
-    e2e_reps = []
-    for _ in range(R):
-        t0 = time.perf_counter()
-        for i in range(K):
-            llama.Eval(lctx, gen[W + i:W + i + 1], PROMPT_LEN + W + i)
-        lib.lb_context_synchronize(lctx._h)
-        e2e_reps.append(time.perf_counter() - t0)
+    t0 = time.perf_counter()
+    for i in range(K):
+        llama.Eval(lctx, gen[W + i:W + i + 1], PROMPT_LEN + W + i)
+    lib.lb_context_synchronize(lctx._h)
+    e2e = K / (time.perf_counter() - t0)
     clocks = sampler.stop() if sampler else None
-    e2e = K / float(np.mean(e2e_reps))
     T_mid = PROMPT_LEN + W + K / 2.0
     bytes_per_token = model.weight_bytes_per_token + 2 * hp.layers * T_mid * hp.dim * 4 + 2 * hp.layers * hp.dim * 4 + 4 * hp.vocab
     return {"model": model, "lctx": lctx, "value": value, "ms": ms, "e2e": e2e, "launches": int(launches), "clocks": clocks,
             "decode_path": DECODE_PATHS.get(lib.lb_context_decode_path(lctx._h).decode(), "?"),
-            "repeats": R, "repeat_ms": [round(r, 3) for r in reps], "setup_s": t_setup, "bytes_per_token": int(bytes_per_token),
+            "logits": logits, "setup_s": t_setup, "bytes_per_token": int(bytes_per_token),
             "prefill": {"tokens": PROMPT_LEN, "ms": round(prefill_s * 1e3, 2), "tok_s": round(PROMPT_LEN / prefill_s, 1),
                         "what": "lb_eval of the %d-token prompt (host buffers, synchronous; tcgen05 3xTF32 GEMMs + prefill attention)" % PROMPT_LEN}}
 
 
 def sub_record(r, peak, what, K, W, extra=None):
     gbs = r["bytes_per_token"] * r["value"] / 1e9
-    rec = {"workload": what, "decode_path": r.get("decode_path"), "value": r["value"], "unit": UNIT, "ms_per_step": r["ms"] / K, "steps": K, "warmup": W, "repeats": r["repeats"],
+    rec = {"workload": what, "decode_path": r.get("decode_path"), "value": r["value"], "unit": UNIT, "ms_per_step": r["ms"] / K, "steps": K, "warmup": W,
            "e2e": r["e2e"], "gpu_launches": r["launches"], "clocks": r["clocks"], "prefill": r["prefill"],
            "roofline": {"bound": "hbm", "achieved": round(gbs, 1), "peak": peak, "unit": "GB/s", "frac": round(gbs / peak, 4),
                         "bytes_per_step": r["bytes_per_token"], "roofline_tok_s": round(peak * 1e9 / r["bytes_per_token"], 1)}}
@@ -398,16 +391,15 @@ def measure_pods(llama, lib, hp, B, ctx_size, K, W, sampler=None):
         llama.Eval(c, rs.randint(3, hp.vocab, size=PROMPT_LEN).astype(np.uint32), 0)
     gen = rs.randint(3, hp.vocab, size=(B, 2 * W + 2 * K)).astype(np.uint32)
     batch = llama.PodBatch(pods)
-    w_ms = batch.DecodeResident(gen[:, :W], [PROMPT_LEN] * B)
-    w_ms = batch.DecodeResident(gen[:, :W], [PROMPT_LEN] * B)
-    R = _repeats_for(K, w_ms / max(W, 1))
+    batch.DecodeResident(gen[:, :W], [PROMPT_LEN] * B)
+    batch.DecodeResident(gen[:, :W], [PROMPT_LEN] * B)
     if sampler:
         sampler.start()
     l0 = lib.lb_kernel_launches()
-    reps = [batch.DecodeResident(gen[:, W:W + K], [PROMPT_LEN + W] * B) for _ in range(R)]
-    launches = (lib.lb_kernel_launches() - l0) // R
-    ms = float(np.mean(reps))
+    ms = batch.DecodeResident(gen[:, W:W + K], [PROMPT_LEN + W] * B)
+    launches = lib.lb_kernel_launches() - l0
     value = B * K / (ms / 1e3)
+    logits = batch.ReadLogits()                         # [B][vocab] of the last timed step, before e2e overwrites it
     for i in range(W):
         batch.Eval(gen[:, W + K + i], [PROMPT_LEN + W + K + i] * B)
     t0 = time.perf_counter()
@@ -418,7 +410,7 @@ def measure_pods(llama, lib, hp, B, ctx_size, K, W, sampler=None):
     T_mid = PROMPT_LEN + W + K / 2.0
     bytes_per_step = model.weight_bytes_per_token + B * (2 * hp.layers * T_mid * hp.dim * 4 + 2 * hp.layers * hp.dim * 4 + 4 * hp.vocab)
     mega = os.environ.get("LB_NO_MEGA_PODS") is None
-    return {"value": value, "ms": ms, "e2e": e2e, "launches": int(launches), "clocks": clocks, "repeats": R,
+    return {"value": value, "ms": ms, "e2e": e2e, "launches": int(launches), "clocks": clocks, "logits": logits,
             "bytes_per_step": int(bytes_per_step), "B": B,
             "decode_path": ("pod-batch megakernel: one persistent launch per step, B-column MulMat on mma.sync tf32 (3xTF32)" if mega
                             else "per-op kernels, B-column GEMV, CUDA-graph replay")}
@@ -426,13 +418,20 @@ def measure_pods(llama, lib, hp, B, ctx_size, K, W, sampler=None):
 
 def pods_record(r, peak, peak_src, what, K, W):
     gbs = r["bytes_per_step"] * (r["value"] / r["B"]) / 1e9
-    return {"workload": what, "value": r["value"], "unit": UNIT, "ms_per_step": r["ms"] / K, "steps": K, "warmup": W, "repeats": r["repeats"],
+    return {"workload": what, "value": r["value"], "unit": UNIT, "ms_per_step": r["ms"] / K, "steps": K, "warmup": W,
             "sequences_in_flight": r["B"], "e2e": r["e2e"], "gpu_launches": r["launches"], "clocks": r["clocks"],
             "decode_path": r["decode_path"],
             "roofline": {"bound": "hbm", "kernel": "whole step", "achieved": round(gbs, 1), "peak": peak, "unit": "GB/s",
                          "frac": round(gbs / peak, 4), "bytes_per_step": r["bytes_per_step"], "peak_source": peak_src,
                          "roofline_tok_s": round(r["B"] * peak * 1e9 / r["bytes_per_step"], 1),
                          "note": "bytes per step = weights once + %d x (KV read/write + logits)" % r["B"]}}
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one float32 .npy per measured decode path, the logits its last timed step computed."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float32))
 
 
 def release(*objs):
@@ -461,7 +460,8 @@ def run_single_gpu(args):
     sampler = ClockSampler(0)
     r = measure_decode(llama, lib, hp, q8, ctx_size, K, W, sampler)
     model, lctx, value, ms, e2e, launches, clocks = r["model"], r["lctx"], r["value"], r["ms"], r["e2e"], r["launches"], r["clocks"]
-    t_setup, repeats, repeat_ms, prefill_rec = r["setup_s"], r["repeats"], r["repeat_ms"], r["prefill"]
+    t_setup, prefill_rec = r["setup_s"], r["prefill"]
+    outputs = {"logits": r["logits"]}
 
     # ---- roofline of the dominant kernel + per-kernel table (live CUDA-event timing)
     peak, peak_src = measured_peak()
@@ -497,6 +497,7 @@ def run_single_gpu(args):
         lctx = model = r = None
         try:
             rq = measure_decode(llama, lib, synth.LLAMA_7B, True, max(1024, PROMPT_LEN + 2 * W + K + 1), K, W, ClockSampler(0))
+            outputs["q8_7b_ctx1024_logits"] = rq["logits"]
             configs["q8_7b_ctx1024"] = sub_record(rq, peak, "BASELINE config 3: LLaMA-7B INT8 block-quant (Q8_0) decode, context 1024, %d-token prompt" % PROMPT_LEN, K, W,
                                                   {"dtype": "q8_0 weights x f32 activations"})
             release(rq["lctx"], rq["model"])
@@ -505,6 +506,7 @@ def run_single_gpu(args):
             configs["q8_7b_ctx1024"] = {"error": str(e)}
         try:
             rp = measure_pods(llama, lib, synth.LLAMA_7B, 8, max(CTX, PROMPT_LEN + 2 * W + 2 * K + 2), K, W, ClockSampler(0))
+            outputs["pods8_logits"] = rp["logits"]
             configs["pods8"] = pods_record(rp, peak, peak_src, "LLaMA-7B FP32, 8 pods (independent sequences, server.go:84-106) batched per weight pass, "
                                            "context 512, %d-token prompts" % PROMPT_LEN, K, W)
             rp = None
@@ -513,6 +515,7 @@ def run_single_gpu(args):
             configs["pods8"] = {"error": str(e)}
         try:
             r13 = measure_decode(llama, lib, synth.LLAMA_13B, False, max(CTX, PROMPT_LEN + 2 * W + K + 1), K, W, ClockSampler(0))
+            outputs["llama13b_1gpu_logits"] = r13["logits"]
             configs["llama13b_1gpu"] = sub_record(r13, peak, "LLaMA-13B FP32 single-sequence decode on 1 GPU, context 512 (BASELINE config 4's model, unsharded)", K, W,
                                                   {"dtype": "f32"})
             release(r13["lctx"], r13["model"])
@@ -531,7 +534,7 @@ def run_single_gpu(args):
     wbytes = bytes_per_token - (2 * hp.layers * (PROMPT_LEN + W + K / 2.0) * hp.dim * 4 + 2 * hp.layers * hp.dim * 4 + 4 * hp.vocab)
     line = {
         "metric": metric_name(args.model) if not q8 else "LLaMA-%s INT8 block-quant (Q8_0) decode tokens/sec" % args.model.upper(), "value": value, "unit": UNIT,
-        "n_gpus": 1, "steps": K, "warmup": W, "repeats": repeats, "repeat_ms": repeat_ms,
+        "n_gpus": 1, "steps": K, "warmup": W,
         "ms_per_step": ms / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32" if not q8 else "q8_0 weights x f32 activations", "data": "synthetic",
         "config": {"workload": "LLaMA-%s %s single-sequence decode, context %d, %d-token prompt prefilled, past %d..%d"
@@ -539,7 +542,7 @@ def run_single_gpu(args):
                    "weights": "random-init (device RNG, seed 0) %.1f GB" % (wbytes / 1e9), "kv_cache": "fp32 in HBM",
                    "sequences_in_flight": 1, "parallelism": "single GPU", "l2": "inputs>L2 (%.1f GB weights per step)" % (wbytes / 1e9),
                    "decode_path": DECODE_PATHS.get(path, path) + ", CUDA-graph replay",
-                   "timed_regions": "%d regions of exactly %d steps each (CUDA events), mean reported" % (repeats, K),
+                   "timed_regions": "1 region of exactly %d steps (CUDA events)" % K,
                    "setup_s": round(t_setup, 1)},
         "clocks": clocks,
         "e2e": {"value": e2e, "unit": UNIT, "h2d_bytes_per_step": 4 + 8, "d2h_bytes_per_step": 4 * hp.vocab,
@@ -566,6 +569,8 @@ def run_single_gpu(args):
         "reference_stream": ref_stream,
         "configs": configs,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
 
 
@@ -583,13 +588,15 @@ def run_pods(args):
     rec = pods_record(r, peak, peak_src, "LLaMA-%s FP32, %d independent sequences (pods), one token each per step, context %d, %d-token prompts"
                       % (args.model.upper(), B, ctx_size, PROMPT_LEN), K, W)
     line = {"metric": "LLaMA-%s FP32 decode tokens/sec, aggregate over %d pods batched per weight pass" % (args.model.upper(), B),
-            "value": rec["value"], "unit": UNIT, "n_gpus": 1, "steps": K, "warmup": W, "repeats": rec["repeats"], "ms_per_step": rec["ms_per_step"],
+            "value": rec["value"], "unit": UNIT, "n_gpus": 1, "steps": K, "warmup": W, "ms_per_step": rec["ms_per_step"],
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": rec["workload"], "sequences_in_flight": B, "l2": "inputs>L2", "decode_path": rec["decode_path"]},
             "clocks": rec["clocks"],
             "e2e": {"value": rec["e2e"], "unit": UNIT, "h2d_bytes_per_step": 8 * B + 8, "d2h_bytes_per_step": 4 * hp.vocab * B,
                     "api": "lb_batch_eval (host buffers, synchronous)"},
             "gpu_launches": rec["gpu_launches"], "roofline": dict(rec["roofline"], traffic=None), "cpu_baseline": None}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": r["logits"]})
     print(json.dumps(line), flush=True)
 
 
@@ -605,11 +612,16 @@ def main():
     ap.add_argument("--model", default="7b", choices=sorted(MODELS), help="default 7b = the headline metric; 13b/65b = BASELINE configs 4-5")
     ap.add_argument("--context", type=int, default=0, help="override the context size (BASELINE config 5 uses 2048)")
     ap.add_argument("--pods", type=int, default=1, help="extra measurement: B pods (1..8) batched per weight pass on one GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the logits of the last timed step of each measured path to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    rank, world, _ = rank_world()
+    if args.dump_outputs and (args.impl == "reference" or world > 1 or args.gpus > 1):
+        ap.error("--dump-outputs is available for the single-GPU arms of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
-    rank, world, _ = rank_world()
     if world > 1 or args.gpus > 1:
         from bench_pipeline import run_pipeline   # layer-sharded multi-GPU arm
         return run_pipeline(args)

@@ -10,8 +10,10 @@ Runs ONLY in the build container (needs /root/reference via oracle/_ref):
      (prompt eval + decode steps, scalar dot order), the golden vectors the GPU path is
      compared against on the GPU box (where /root/reference does not exist).
 
-Usage: python tools/gen_golden.py
+Usage: python tools/gen_golden.py [case ...]            # refbin_<case>.json, logits_<case>.npz
+       python tools/gen_golden.py swap|threads2|vdot    # refbin_swap.json, refbin_threads2.json, vdot_ref.npz
 """
+import hashlib
 import json
 import os
 import sys
@@ -92,7 +94,7 @@ def main():
     print("done")
 
 
-if __name__ == "__main__" and "swap" not in sys.argv[1:]:
+if __name__ == "__main__" and not {"swap", "threads2", "vdot"} & set(sys.argv[1:]):
     main()
 
 
@@ -125,3 +127,56 @@ def gen_swap():
 
 if __name__ == "__main__" and "swap" in sys.argv[1:]:
     gen_swap()
+
+
+def gen_threads2():
+    """refbin_threads2.json — the reference binary (--avx, 2 threads) on the ggjt files synth.write_ggjt makes for the tiny
+    and hd128 cases: the file's SHA-256, the printed stream and the number of evals it timed.  Pins the ggjt writer and
+    the oracle's --avx stream to a third thread count."""
+    O.build()
+    out = {}
+    for name in ("tiny", "hd128"):
+        with open(os.path.join(ROOT, "tests", "golden", f"refbin_{name}.json")) as f:
+            rec = json.load(f)
+        hp = synth.HParams(*rec["hparams"])
+        vocab = synth.byte_vocab(hp.vocab)
+        with tempfile.TemporaryDirectory() as td:
+            path = os.path.join(td, "m.bin")
+            synth.write_ggjt(path, hp, synth.synth_model(rec["seed"], hp), vocab)
+            with open(path, "rb") as f:
+                sha = hashlib.sha256(f.read()).hexdigest()
+            r = refbin.run(path, rec["prompt"], rec["predict"], rec["context"], 2, True, port=18181)
+        exp = refbin.expected_text(vocab, rec["prompt_ids"], rec["oracle_tokens"])
+        assert refbin.same_stream(r["text"], exp), name
+        out[name] = {"threads": 2, "avx": True, "ggjt_sha256": sha, "text_hex": r["text"].hex(), "evals": len(r["eval_ms"])}
+        print(f"[{name}/threads2] binary text len {len(r['text'])}, {len(r['eval_ms'])} evals")
+    with open(os.path.join(ROOT, "tests", "golden", "refbin_threads2.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
+def gen_vdot():
+    """vdot_ref.npz — _mm256_dot of the reference's utils/floats_avx.c, compiled as-is (oracle/_ref/libvdot_ref.so), on
+    seeded vectors of the lengths that exercise its 8-lane body and scalar tail.  Pins the oracle's --avx dot order."""
+    import ctypes as C
+    O.build()
+    L = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libvdot_ref.so"))
+    fp = C.POINTER(C.c_float)
+    L._mm256_dot.argtypes = [fp, fp, C.c_int64, fp]
+    rng = np.random.default_rng(0)
+    ns = [8, 9, 15, 16, 128, 131, 4096, 11008]
+    a = rng.standard_normal(sum(ns)).astype(np.float32)
+    b = rng.standard_normal(sum(ns)).astype(np.float32)
+    dots, off = [], 0
+    for n in ns:
+        ret = C.c_float(0)
+        L._mm256_dot(a[off:].ctypes.data_as(fp), b[off:].ctypes.data_as(fp), n, C.byref(ret))
+        dots.append(ret.value)
+        off += n
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "vdot_ref.npz"), n=np.asarray(ns, np.int64), a=a, b=b,
+                        dot=np.asarray(dots, np.float32))
+
+
+if __name__ == "__main__" and "threads2" in sys.argv[1:]:
+    gen_threads2()
+if __name__ == "__main__" and "vdot" in sys.argv[1:]:
+    gen_vdot()
