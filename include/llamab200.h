@@ -57,7 +57,9 @@ LB_API uint64_t    lb_kernel_launches(void);       /* kernels launched by this l
 /* ---- model = llama.Model + LoadModel's tensor map (llama.go:712-976) ------------------ */
 /* Layers [layer_begin, layer_end) live on `device`; the stage with layer_begin == 0 also owns
  * tok_embeddings, the stage with layer_end == layers also owns norm + output (SURVEY §8e).
- * weight_type: LB_TYPE_F32, or LB_TYPE_Q8_0 to hold the 2-D matrices block-quantised. */
+ * weight_type: LB_TYPE_F32; LB_TYPE_F16 to hold every 2-D MulMat matrix (wq|wk|wv, wo, w1, w2, w3, output) as
+ * IEEE binary16 — half the bytes, the same arithmetic on the widened values (needs dim and ff multiples of 32);
+ * or LB_TYPE_Q8_0 to hold them block-quantised.  Norm vectors and tok_embeddings always stay FP32. */
 LB_API lb_model *lb_model_create(const lb_hparams *hp, int device, uint32_t layer_begin,
                                  uint32_t layer_end, int weight_type);
 LB_API void      lb_model_free(lb_model *m);
@@ -67,9 +69,12 @@ LB_API void      lb_model_free(lb_model *m);
 LB_API lb_model *lb_model_load_ggjt(const char *path, int device, uint32_t layer_begin, uint32_t layer_end,
                                     int weight_type, lb_hparams *hp_out);
 /* name = ggjt tensor name (llama.go:826-861); dtype LB_TYPE_F32 or LB_TYPE_F16 (widened to FP32
- * like llama.go:938-941); tensors of layers this stage does not own are accepted and ignored. */
+ * like llama.go:938-941); tensors of layers this stage does not own are accepted and ignored.
+ * Into an LB_TYPE_F16 model's matrices F16 data is stored byte for byte and F32 data is rounded to nearest
+ * even (as numpy's astype(float16)); a finite value beyond +-65504 is an error.  The same holds for
+ * lb_model_load_ggjt and lb_model_init_random. */
 LB_API int       lb_model_set_tensor(lb_model *m, const char *name, int dtype, const void *host, size_t nbytes);
-LB_API int       lb_model_get_tensor(lb_model *m, const char *name, float *host, size_t nelem); /* dequantised */
+LB_API int       lb_model_get_tensor(lb_model *m, const char *name, float *host, size_t nelem); /* dequantised / widened to FP32 */
 /* Synthetic weights generated on the device; bit-identical to llama.go_b200/synth.py. */
 LB_API int       lb_model_init_random(lb_model *m, uint64_t seed);
 LB_API uint64_t  lb_model_weight_bytes(const lb_model *m);   /* bytes one decoded token streams */
@@ -83,7 +88,7 @@ LB_API int       lb_synth_fill_host(float *dst, uint64_t count, uint64_t seed, u
  * 5 attention at `past`, 6 rmsnorm, 7 prefill GEMM w1 x min(512, ctx) tokens — bytes_out then holds its
  * FLOPs) `iters` times back to back on the context's stream, cycling
  * through the layers so the weights never sit in L2; ms_out = CUDA-event time of all launches,
- * bytes_out = algorithmic bytes of ONE launch. */
+ * bytes_out = algorithmic bytes of ONE launch.  F32 and Q8_0 models only (an F16 model is refused). */
 LB_API int       lb_bench_kernel(lb_context *c, int which, uint32_t iters, uint32_t past, float *ms_out,
                                  uint64_t *bytes_out);
 
@@ -96,7 +101,8 @@ LB_API int lb_eval(lb_context *c, const uint32_t *tokens, uint32_t n, uint32_t p
 /* Same, but every row of logits ([n][vocab]) as the reference computes them (llama.go:384). */
 LB_API int lb_eval_all_logits(lb_context *c, const uint32_t *tokens, uint32_t n, uint32_t past, float *logits_out);
 /* The same forward pass built node for node with the op API below, exactly as llama.go:211-426
- * builds it, and run by lb_graph_compute (slow path; exists to prove the op API is a drop-in). */
+ * builds it, and run by lb_graph_compute (slow path; exists to prove the op API is a drop-in).
+ * The op API is FP32 like the reference's: Q8_0 and F16 models are refused. */
 LB_API int lb_eval_graph(lb_context *c, const uint32_t *tokens, uint32_t n, uint32_t past, float *logits_out);
 /* Device-resident decode: enqueue `steps` single-token evals starting at `past` with the given
  * tokens (teacher forcing), no host copies; used by bench.py for the kernel-only number.
@@ -139,8 +145,9 @@ LB_API int lb_eval_stage(lb_context *c, const uint32_t *tokens, uint32_t n, uint
                          const float *hidden_in_dev, float *hidden_out_dev, float *logits_out);
 LB_API float *lb_context_hidden_buffer(lb_context *c);   /* device [max_batch][dim] scratch for hand-offs */
 LB_API void  *lb_context_stream(lb_context *c);          /* cudaStream_t */
-/* which kernels a single-token Eval of this context runs: "ring" (TMA-ring megakernel), "mega" (register-fed megakernel),
-   "ring_q8" (Q8_0 ring megakernel) or "perop" (one kernel per op) — measurement aid, no reference counterpart */
+/* which kernels a single-token Eval of this context runs: "ring" (TMA-ring megakernel), "ring_f16" (the same with F16 weights),
+   "mega" (register-fed megakernel), "ring_q8" (Q8_0 ring megakernel) or "perop" (one kernel per op) — measurement aid,
+   no reference counterpart */
 LB_API const char *lb_context_decode_path(lb_context *c);
 /* work split / data layout of the ring megakernels, evaluated on the HOST by the same functions the kernels use (test aid, no
    GPU needed, no reference counterpart).  kind 0: FP32 ring, K = a -> out {chunks per row, floats per chunk};
@@ -187,7 +194,7 @@ LB_API int  lb_nccl_version(void);
  * a barrier over all stages after import and after every lb_pipeline_prefill, before any stage calls lb_pipeline_decode —
  * prefill is outside the hand-off's flag protocol (llama.go_b200/pipeline.py does both barriers). */
 LB_API int lb_pipeline_p2p_export(lb_context **ctxs, uint32_t n, void *handles_out);
-LB_API int lb_pipeline_p2p_import(lb_context **ctxs, uint32_t n, const void *downstream_handles, const void *upstream_handles);
+LB_API int lb_pipeline_p2p_import(lb_context **ctxs, uint32_t n, const void *downstream_handles, const void *upstream_handles);   /* FP32 stages only: F16 is refused */
 LB_API int lb_pipeline_p2p_disable(lb_context **ctxs, uint32_t n);   /* back to NCCL (e.g. another rank's import failed) */
 /* Pipelined steady-state decode of `n_seq` in-flight sequences ("pods", server.go:84-106) for `steps`
  * tokens each, starting at position `past`: per (step, sequence) this rank receives the residual

@@ -213,7 +213,8 @@ const char *lb_context_decode_path(lb_context *c) {
     if (!c) return "";
     if (c->c->use_ring_q8) return "ring_q8";
     if (!c->c->use_mega) return "perop";
-    return c->c->use_ring ? "ring" : "mega";
+    if (c->c->use_ring) return c->c->model->f16() ? "ring_f16" : "ring";
+    return "mega";
 }
 
 // ---- pod batching ----

@@ -44,6 +44,8 @@ void rope(float *x, uint32_t ne0, uint32_t ne1, uint32_t ne2, uint32_t past, uin
 void mul_mat_generic(const TView &a, const TView &b, const TView &dst, cudaStream_t st);
 void init_random(float *dst, uint64_t count, uint64_t seed, uint64_t tid, float mean, float sigma_scale, cudaStream_t st);
 void f16_to_f32(const uint16_t *src, float *dst, size_t n, cudaStream_t st);
+// binary16 round to nearest even (numpy's astype(float16)); *overflow = 1 if a finite value rounds to +-inf
+void f32_to_f16(const float *src, uint16_t *dst, size_t n, unsigned *overflow, cudaStream_t st);
 
 // ---- fused hot-path kernels (llama::Eval) ----
 enum Epilogue { EPI_NONE = 0, EPI_ADD_RESIDUAL = 1 };
@@ -53,6 +55,12 @@ void gemv_f32(const float *W, uint32_t M, uint32_t K, const float *x, uint32_t l
               float *y, uint32_t ldy, const float *residual, cudaStream_t st);
 // act[n][m] = silu(W1[m]·x[n]) * (W3[m]·x[n])   (llama.go:354-361)
 void gemv_f32_swiglu(const float *W1, const float *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
+                     uint32_t N, float *act, uint32_t ldy, cudaStream_t st);
+// the same two with IEEE binary16 weights, widened in registers: each lane reads the elements it reads in the F32
+// kernels and issues the same FMAs in the same order, so the results equal the F32 kernels' on the widened weights
+void gemv_f16(const uint16_t *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, uint32_t N,
+              float *y, uint32_t ldy, const float *residual, cudaStream_t st);
+void gemv_f16_swiglu(const uint16_t *W1, const uint16_t *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
                      uint32_t N, float *act, uint32_t ldy, cudaStream_t st);
 // prefill GEMM, any N: Y[n][m] = sum_k W[m][k] X[n][k] (+ residual)
 void gemm_f32(const float *W, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
@@ -66,6 +74,10 @@ void gemm_tf32x3(const float *W, uint32_t M, uint32_t K, const float *X, uint32_
 // dispatcher for N > 8: tensor-core path when the shape allows (and LB_NO_TC is unset), else gemm_f32
 void gemm_auto(const float *W, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
                float *Y, uint32_t ldy, const float *residual, cudaStream_t st);
+// the same tcgen05 GEMM with a row-major binary16 weight operand (K % 32 == 0), widened in the shared-memory stage;
+// binary16 is exact in TF32, so the weight has no lo part and each K step issues two MMAs (W*X_hi + W*X_lo)
+void gemm_f16_tc(const uint16_t *W, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
+                 float *Y, uint32_t ldy, const float *residual, cudaStream_t st);
 // q (rows ldq apart, [N][dim]) rotated in place at positions past+n; k rotated and stored to
 // Kc[(past+n)][dim]; v stored to Vc[(past+n)][dim]   (llama.go:274-297 — K is cached rotated)
 // `past_dev` is a DEVICE pointer to the position of the first new token, so that a captured CUDA
@@ -112,6 +124,7 @@ struct MegaLayerHost {  // one per layer, array lives in device memory
     float *Kc, *Vc;
     const int8_t *q_wqkv, *q_wo, *q_w1, *q_w3, *q_w2;  // Q8_0 planes (nullptr for F32 models)
     const float *d_wqkv, *d_wo, *d_w1, *d_w3, *d_w2;
+    const uint16_t *h_wqkv, *h_wo, *h_w1, *h_w3, *h_w2;  // binary16 matrices (F16 models, TMA-ring kernel only)
 };
 struct MegaParamsHost {
     const MegaLayerHost *layers_dev;
@@ -122,6 +135,8 @@ struct MegaParamsHost {
     const int8_t *q_output = nullptr; // Q8_0 lm_head planes (experiment: Q8 megakernel)
     const float *d_output = nullptr;
     bool q8 = false;
+    bool f16 = false;                 // F16 weights: the layers' h_* matrices and h_output (decode_ring only)
+    const uint16_t *h_output = nullptr;
     float *x, *y, *qkv, *attn, *act, *logits;
     float *part_o, *part_ml;
     unsigned *tickets, *barrier;

@@ -503,5 +503,23 @@ void f16_to_f32(const uint16_t *src, float *dst, size_t n, cudaStream_t st) {
     LB_LAUNCH_CHECK();
 }
 
+// __float2half_rn rounds to nearest even with gradual underflow, exactly like numpy's float32 -> float16 cast
+__global__ void f32_to_f16_kernel(const float *__restrict__ src, __half *__restrict__ dst, size_t n, unsigned *overflow) {
+    size_t stride = (size_t)gridDim.x * blockDim.x;
+    bool over = false;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float v = src[i];
+        const __half h = __float2half_rn(v);
+        over |= isfinite(v) && __hisinf(h);
+        dst[i] = h;
+    }
+    if (over) atomicExch(overflow, 1u);
+}
+void f32_to_f16(const float *src, uint16_t *dst, size_t n, unsigned *overflow, cudaStream_t st) {
+    if (!n) return;
+    f32_to_f16_kernel<<<blocks_for(n, 256), 256, 0, st>>>(src, reinterpret_cast<__half *>(dst), n, overflow);
+    LB_LAUNCH_CHECK();
+}
+
 }  // namespace k
 }  // namespace lb

@@ -324,6 +324,7 @@ struct MegaLayer {
     float *Kc, *Vc;
     const int8_t *q_wqkv, *q_wo, *q_w1, *q_w3, *q_w2;  // Q8_0 planes (Q8 megakernel)
     const float *d_wqkv, *d_wo, *d_w1, *d_w3, *d_w2;
+    const uint16_t *h_wqkv, *h_wo, *h_w1, *h_w3, *h_w2;  // F16 matrices (read by the TMA-ring kernel only)
 };
 struct MegaParams {
     const MegaLayer *layers;

@@ -1,16 +1,28 @@
 // kernels_mulmat.cu — MulMat family (ComputeForwardMulMatFP32, pkg/ml/ml.go:1976-2098).
 //   gemv_f32 / gemv_f32_swiglu : decode (N = 1..8 activation columns), HBM-bound weight streaming
+//   gemv_f16 / gemv_f16_swiglu : the same kernels reading binary16 weights (widened in registers)
 //   gemm_f32                   : prefill (any N), shared-memory tiled FP32
 //   mul_mat_generic            : arbitrary strided operands (the permuted K·Q / V^T·P products
 //                                of the op-level API)
 // dst[n][m] = sum_k W[m][k] * x[n][k], FP32 multiply-add (the GPU fuses mul+add into FMA; the
 // reference's scalar loop and AVX1 vdot do not — a <=1e-6 relative difference, far inside the
 // 1e-3 logits budget; summation order likewise differs).
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 #include "kernels.cuh"
 
 namespace lb {
 namespace k {
+
+// 4 consecutive weights -> float4: FP32 (one streaming 128-bit load) or binary16 (one streaming 64-bit load, widened exactly)
+__device__ __forceinline__ float4 ld_w4(const float *p) { return ld_stream_f4(p); }
+__device__ __forceinline__ float4 ld_w4(const __half *p) {
+    uint32_t a, b;
+    asm volatile("ld.global.nc.L1::no_allocate.v2.b32 {%0,%1}, [%2];" : "=r"(a), "=r"(b) : "l"(p));
+    const float2 lo = __half22float2(*reinterpret_cast<const __half2 *>(&a)), hi = __half22float2(*reinterpret_cast<const __half2 *>(&b));
+    return make_float4(lo.x, lo.y, hi.x, hi.y);
+}
 
 // ------------------------------------------------------------------------------------------
 // Decode GEMV.  One warp owns RPW consecutive weight rows; the 32 lanes stride the row in
@@ -20,9 +32,9 @@ namespace k {
 constexpr int GEMV_WARPS = 8;   // swiglu kernel
 constexpr int GEMV_UNROLL = 4;
 
-template <int NC, int RPW, int WARPS, int UNROLL>
+template <typename WT, int NC, int RPW, int WARPS, int UNROLL>
 __global__ void __launch_bounds__(WARPS * 32)
-gemv_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const float *__restrict__ x, uint32_t ldx,
+gemv_kernel(const WT *__restrict__ W, uint32_t M, uint32_t K, const float *__restrict__ x, uint32_t ldx,
             float *__restrict__ y, uint32_t ldy, const float *__restrict__ res) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t row0 = (blockIdx.x * WARPS + warp) * RPW;
@@ -32,7 +44,7 @@ gemv_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const float *__
     for (int r = 0; r < RPW; r++)
 #pragma unroll
         for (int c = 0; c < NC; c++) acc[r][c] = 0.f;
-    const float *wr[RPW];
+    const WT *wr[RPW];
 #pragma unroll
     for (int r = 0; r < RPW; r++) wr[r] = W + (size_t)min(row0 + r, M - 1) * K;
 
@@ -45,7 +57,7 @@ gemv_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const float *__
             uint32_t kq = kk + u * 128;
 #pragma unroll
             for (int r = 0; r < RPW; r++)
-                w[u][r] = (kq < K) ? ld_stream_f4(wr[r] + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
+                w[u][r] = (kq < K) ? ld_w4(wr[r] + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
     };
     pdl_launch_dependents();
@@ -96,9 +108,9 @@ gemv_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const float *__
     }
 }
 
-template <int NC>
+template <typename WT, int NC>
 __global__ void __launch_bounds__(GEMV_WARPS * 32)
-gemv_swiglu_kernel(const float *__restrict__ W1, const float *__restrict__ W3, uint32_t M, uint32_t K,
+gemv_swiglu_kernel(const WT *__restrict__ W1, const WT *__restrict__ W3, uint32_t M, uint32_t K,
                    const float *__restrict__ x, uint32_t ldx, float *__restrict__ act, uint32_t ldy) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t row = blockIdx.x * GEMV_WARPS + warp;
@@ -106,14 +118,14 @@ gemv_swiglu_kernel(const float *__restrict__ W1, const float *__restrict__ W3, u
     float a1[NC], a3[NC];
 #pragma unroll
     for (int c = 0; c < NC; c++) a1[c] = a3[c] = 0.f;
-    const float *w1 = W1 + (size_t)row * K, *w3 = W3 + (size_t)row * K;
+    const WT *w1 = W1 + (size_t)row * K, *w3 = W3 + (size_t)row * K;
     float4 p[GEMV_UNROLL], q[GEMV_UNROLL];
     auto load_batch = [&](uint32_t kk) {
 #pragma unroll
         for (int u = 0; u < GEMV_UNROLL; u++) {
             uint32_t kq = kk + u * 128;
-            p[u] = (kq < K) ? ld_stream_f4(w1 + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
-            q[u] = (kq < K) ? ld_stream_f4(w3 + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
+            p[u] = (kq < K) ? ld_w4(w1 + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
+            q[u] = (kq < K) ? ld_w4(w3 + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
     };
     pdl_launch_dependents();
@@ -148,9 +160,9 @@ gemv_swiglu_kernel(const float *__restrict__ W1, const float *__restrict__ W3, u
 // Multi-column (pod batch, NC >= 3) variant: a warp owns 4 weight rows so every activation float4 it
 // pulls through L1 is used by 4 rows — with one row per warp the 8 activation columns would need
 // ~190 B/clk of L1 bandwidth per SM to keep up with the weight stream (the L1 limit is 128).
-template <int NC>
+template <typename WT, int NC>
 __global__ void __launch_bounds__(128)
-gemv_cols_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const float *__restrict__ x, uint32_t ldx,
+gemv_cols_kernel(const WT *__restrict__ W, uint32_t M, uint32_t K, const float *__restrict__ x, uint32_t ldx,
                  float *__restrict__ y, uint32_t ldy, const float *__restrict__ res) {
     constexpr int RPW = 4, U = 2;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -161,7 +173,7 @@ gemv_cols_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const floa
     for (int r = 0; r < RPW; r++)
 #pragma unroll
         for (int c = 0; c < NC; c++) acc[r][c] = 0.f;
-    const float *wr[RPW];
+    const WT *wr[RPW];
 #pragma unroll
     for (int r = 0; r < RPW; r++) wr[r] = W + (size_t)min(row0 + r, M - 1) * K;
     float4 w[U][RPW];
@@ -170,7 +182,7 @@ gemv_cols_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const floa
         for (int u = 0; u < U; u++) {
             const uint32_t kq = kk + u * 128;
 #pragma unroll
-            for (int r = 0; r < RPW; r++) w[u][r] = (kq < K) ? ld_stream_f4(wr[r] + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
+            for (int r = 0; r < RPW; r++) w[u][r] = (kq < K) ? ld_w4(wr[r] + kq) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
     };
     pdl_launch_dependents();
@@ -215,60 +227,78 @@ gemv_cols_kernel(const float *__restrict__ W, uint32_t M, uint32_t K, const floa
     }
 }
 
-template <int NC>
-static void gemv_launch(const float *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, float *y, uint32_t ldy,
+template <typename WT, int NC>
+static void gemv_launch(const WT *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, float *y, uint32_t ldy,
                         const float *res, cudaStream_t st) {
     // Large M (qkv, lm_head): 2 rows per warp, 8 warps.  Small M (wo, w2: M = dim): one row per warp
     // and 4-warp blocks so that the grid is >= 6 blocks per SM and every SM holds the same number of
     // warps (256 blocks of 16 rows left 1.7 blocks per SM: measured 51-63 % of HBM peak).
     constexpr bool two = (NC <= 2);
     if (NC >= 3) {
-        launch_pdl(gemv_cols_kernel<NC>, dim3((M + 15) / 16), dim3(128), 0, st, W, M, K, x, ldx, y, ldy, res);
+        launch_pdl(gemv_cols_kernel<WT, NC>, dim3((M + 15) / 16), dim3(128), 0, st, W, M, K, x, ldx, y, ldy, res);
     } else if (two && M >= 8192) {
         unsigned grid = (M + 15) / 16;
-        launch_pdl(gemv_kernel<NC, 2, 8, 4>, dim3(grid), dim3(256), 0, st, W, M, K, x, ldx, y, ldy, res);
+        launch_pdl(gemv_kernel<WT, NC, 2, 8, 4>, dim3(grid), dim3(256), 0, st, W, M, K, x, ldx, y, ldy, res);
     } else {
         unsigned grid = (M + 3) / 4;
-        launch_pdl(gemv_kernel<NC, 1, 4, (NC <= 4 ? 8 : 4)>, dim3(grid), dim3(128), 0, st, W, M, K, x, ldx, y, ldy, res);
+        launch_pdl(gemv_kernel<WT, NC, 1, 4, (NC <= 4 ? 8 : 4)>, dim3(grid), dim3(128), 0, st, W, M, K, x, ldx, y, ldy, res);
     }
 }
 
+template <typename WT>
+static void gemv_any(const char *what, const WT *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, uint32_t N, float *y,
+                     uint32_t ldy, const float *residual, cudaStream_t st) {
+    LB_CHECK(N >= 1 && N <= 8, std::string(what) + ": N must be 1..8");
+    LB_CHECK((K & 3) == 0 && (ldx & 3) == 0, std::string(what) + ": K and ldx must be multiples of 4");
+    switch (N) {
+        case 1: gemv_launch<WT, 1>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 2: gemv_launch<WT, 2>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 3: gemv_launch<WT, 3>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 4: gemv_launch<WT, 4>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 5: gemv_launch<WT, 5>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 6: gemv_launch<WT, 6>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        case 7: gemv_launch<WT, 7>(W, M, K, x, ldx, y, ldy, residual, st); break;
+        default: gemv_launch<WT, 8>(W, M, K, x, ldx, y, ldy, residual, st); break;
+    }
+}
 void gemv_f32(const float *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, uint32_t N, float *y,
               uint32_t ldy, const float *residual, cudaStream_t st) {
-    LB_CHECK(N >= 1 && N <= 8, "gemv_f32: N must be 1..8");
-    LB_CHECK((K & 3) == 0 && (ldx & 3) == 0, "gemv_f32: K and ldx must be multiples of 4");
-    switch (N) {
-        case 1: gemv_launch<1>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 2: gemv_launch<2>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 3: gemv_launch<3>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 4: gemv_launch<4>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 5: gemv_launch<5>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 6: gemv_launch<6>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        case 7: gemv_launch<7>(W, M, K, x, ldx, y, ldy, residual, st); break;
-        default: gemv_launch<8>(W, M, K, x, ldx, y, ldy, residual, st); break;
-    }
+    gemv_any("gemv_f32", W, M, K, x, ldx, N, y, ldy, residual, st);
+}
+void gemv_f16(const uint16_t *W, uint32_t M, uint32_t K, const float *x, uint32_t ldx, uint32_t N, float *y,
+              uint32_t ldy, const float *residual, cudaStream_t st) {
+    gemv_any("gemv_f16", reinterpret_cast<const __half *>(W), M, K, x, ldx, N, y, ldy, residual, st);
 }
 
-template <int NC>
-static void swiglu_launch(const float *W1, const float *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
+template <typename WT, int NC>
+static void swiglu_launch(const WT *W1, const WT *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
                           float *act, uint32_t ldy, cudaStream_t st) {
     unsigned grid = (M + GEMV_WARPS - 1) / GEMV_WARPS;
-    launch_pdl(gemv_swiglu_kernel<NC>, dim3(grid), dim3(GEMV_WARPS * 32), 0, st, W1, W3, M, K, x, ldx, act, ldy);
+    launch_pdl(gemv_swiglu_kernel<WT, NC>, dim3(grid), dim3(GEMV_WARPS * 32), 0, st, W1, W3, M, K, x, ldx, act, ldy);
+}
+template <typename WT>
+static void swiglu_any(const char *what, const WT *W1, const WT *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
+                       uint32_t N, float *act, uint32_t ldy, cudaStream_t st) {
+    LB_CHECK(N >= 1 && N <= 8, std::string(what) + ": N must be 1..8");
+    LB_CHECK((K & 3) == 0 && (ldx & 3) == 0, std::string(what) + ": K and ldx must be multiples of 4");
+    switch (N) {
+        case 1: swiglu_launch<WT, 1>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 2: swiglu_launch<WT, 2>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 3: swiglu_launch<WT, 3>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 4: swiglu_launch<WT, 4>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 5: swiglu_launch<WT, 5>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 6: swiglu_launch<WT, 6>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        case 7: swiglu_launch<WT, 7>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+        default: swiglu_launch<WT, 8>(W1, W3, M, K, x, ldx, act, ldy, st); break;
+    }
 }
 void gemv_f32_swiglu(const float *W1, const float *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
                      uint32_t N, float *act, uint32_t ldy, cudaStream_t st) {
-    LB_CHECK(N >= 1 && N <= 8, "gemv_f32_swiglu: N must be 1..8");
-    LB_CHECK((K & 3) == 0 && (ldx & 3) == 0, "gemv_f32_swiglu: K and ldx must be multiples of 4");
-    switch (N) {
-        case 1: swiglu_launch<1>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 2: swiglu_launch<2>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 3: swiglu_launch<3>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 4: swiglu_launch<4>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 5: swiglu_launch<5>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 6: swiglu_launch<6>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        case 7: swiglu_launch<7>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-        default: swiglu_launch<8>(W1, W3, M, K, x, ldx, act, ldy, st); break;
-    }
+    swiglu_any("gemv_f32_swiglu", W1, W3, M, K, x, ldx, N, act, ldy, st);
+}
+void gemv_f16_swiglu(const uint16_t *W1, const uint16_t *W3, uint32_t M, uint32_t K, const float *x, uint32_t ldx,
+                     uint32_t N, float *act, uint32_t ldy, cudaStream_t st) {
+    swiglu_any("gemv_f16_swiglu", reinterpret_cast<const __half *>(W1), reinterpret_cast<const __half *>(W3), M, K, x, ldx, N, act, ldy, st);
 }
 
 // ------------------------------------------------------------------------------------------

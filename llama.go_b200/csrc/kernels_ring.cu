@@ -26,7 +26,13 @@
 // Slot q lives in ring entry q % n; full[] (expect_tx + the copy's complete_tx) / empty[] (the 16 warps' arrivals).
 // Numerics are those of kernels_mega.cu (f64 RMSNorm sums, f64 RoPE, f64 exp softmax terms, K-slice partial sums combined
 // in warp order); only the chunking of K > 4096 rows differs in the association order of the FP32 dot products.
+//
+// F16 weights (WT = __half): the same kernel streams the binary16 matrices.  The K chunking stays 4096 ELEMENTS per slot
+// (8 KB, so twice as many slots fit in the ring), and each lane reads the same elements as in the FP32 ring — two LDS.64
+// instead of two LDS.128 — widens them exactly and issues the same FMAs in the same order: every product and partial sum
+// equals the FP32 ring's on the widened weights, so the logits are bit-identical to an FP32 model holding those weights.
 #include <cooperative_groups.h>
+#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -40,9 +46,9 @@ constexpr int RG_CWARPS = 16;                      // consumer warps
 constexpr int RG_CTHREADS = RG_CWARPS * 32;        // 512
 constexpr int RG_THREADS = RG_CTHREADS + 32;       // + the producer warp
 constexpr int RG_HALF = RG_CTHREADS / 2;
-constexpr uint32_t RG_SLOT_FLOATS = 4096;          // one slot = one row (or a K chunk of a longer row): ONE bulk copy of <= 16 KB
-constexpr uint32_t RG_SLOT = RG_SLOT_FLOATS * 4;
-constexpr int RG_MAX_SLOTS = 13;
+constexpr uint32_t RG_SLOT_FLOATS = 4096;          // one slot = one row (or a K chunk of a longer row) of <= 4096 weights: ONE bulk copy
+template <typename WT> constexpr uint32_t RG_SLOT = RG_SLOT_FLOATS * sizeof(WT);   // 16 KB (FP32) / 8 KB (F16)
+template <typename WT> constexpr int RG_MAX_SLOTS = sizeof(WT) == 4 ? 13 : 26;
 constexpr int RG_GROUP = 32;                       // rows whose K-slice partials are combined per CTA barrier
 constexpr int RG_MAX_PHASES = 4 * 160 + 1;        // MulMat phases of a launch: 4 per layer + lm_head
 constexpr int RG_MAX_ITEMS = 2 * kNumSMs;
@@ -56,6 +62,24 @@ __device__ __forceinline__ float4 lds4(uint32_t addr) {
     float4 r;
     asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr));
     return r;
+}
+// 4 consecutive ring weights -> float4: FP32 (LDS.128) or binary16 (LDS.64, widened exactly)
+template <typename WT>
+__device__ __forceinline__ float4 lds_w4(uint32_t addr) {
+    if constexpr (sizeof(WT) == 4) {
+        return lds4(addr);
+    } else {
+        uint32_t a, b;
+        asm volatile("ld.shared.v2.b32 {%0,%1}, [%2];" : "=r"(a), "=r"(b) : "r"(addr));
+        const float2 lo = __half22float2(*reinterpret_cast<const __half2 *>(&a)), hi = __half22float2(*reinterpret_cast<const __half2 *>(&b));
+        return make_float4(lo.x, lo.y, hi.x, hi.y);
+    }
+}
+// a layer matrix of the element type the kernel streams
+template <typename WT>
+__device__ __forceinline__ const WT *wsel(const float *f32, const uint16_t *f16) {
+    if constexpr (sizeof(WT) == 4) return f32;
+    else return reinterpret_cast<const WT *>(f16);
 }
 __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
     unsigned v;
@@ -112,6 +136,7 @@ struct RingParams {
     const uint32_t *tokens;
     const uint32_t *state;        // {past, step}
     const float *final_norm, *output;  // nullptr: no lm_head on this stage
+    const uint16_t *output_h;          // binary16 lm_head (F16 weights)
     float *x, *y, *qkv, *attn, *act, *logits;
     float *part_o, *part_ml;
     unsigned *barrier;
@@ -125,9 +150,10 @@ struct RingParams {
     uint32_t *p2p_flag_out, *p2p_ack_out;
 };
 
+template <int NS>
 struct RingShared {
-    unsigned long long full[RG_MAX_SLOTS], empty[RG_MAX_SLOTS];
-    unsigned jobrow[RG_MAX_SLOTS];  // the output row the slot's bytes belong to
+    unsigned long long full[NS], empty[NS];
+    unsigned jobrow[NS];  // the output row the slot's bytes belong to
     unsigned short done_jobs[RG_MAX_PHASES];   // jobs of MulMat phase i of this launch (0xFFFF: the producer has not finished it)
     float part[2][2][RG_GROUP][RG_CWARPS];     // [buffer][matrix (w1|w3)][row of the group][warp]
     unsigned grow[2][RG_GROUP];                // output rows of the group
@@ -195,8 +221,8 @@ __host__ __device__ __forceinline__ uint32_t ring_chunk(uint32_t K, uint32_t nch
 constexpr unsigned RG_STATIC_NUM = 4, RG_STATIC_DEN = 5;
 // rows per ticket: ~64 KB of stream (1.4 us of an SM's share; r02q: 4-row tickets of the w1|w3 pair = 128 KB left the CTAs up to
 // 4.6 us apart at the barrier), at most 2 rows when a CTA has fewer than 48 rows in the phase
-__device__ __forceinline__ uint32_t ticket_rows(uint32_t M, uint32_t K, uint32_t NM) {
-    uint32_t t = 65536u / (K * 4u * NM);
+__device__ __forceinline__ uint32_t ticket_rows(uint32_t M, uint32_t K, uint32_t NM, uint32_t esz) {
+    uint32_t t = 65536u / (K * esz * NM);
     t = t < 1u ? 1u : (t > 4u ? 4u : t);
     return (M / gridDim.x < 48u && t > 2u) ? 2u : t;
 }
@@ -204,13 +230,13 @@ __device__ __forceinline__ uint32_t ticket_rows(uint32_t M, uint32_t K, uint32_t
 // ---------------------------------------------------------------------------------------------------------
 // producer (one thread)
 // ---------------------------------------------------------------------------------------------------------
-template <int NM>
-__device__ __forceinline__ void produce(const float *W, const float *W3, uint32_t K, uint32_t M, RingPos &q, uint32_t phidx, unsigned *ticket,
-                                        uint32_t ring_base, RingShared &sh, uint32_t n_slots, unsigned long long *pstat = nullptr) {
+template <typename WT, int NM, typename SH>
+__device__ __forceinline__ void produce(const WT *W, const WT *W3, uint32_t K, uint32_t M, RingPos &q, uint32_t phidx, unsigned *ticket,
+                                        uint32_t ring_base, SH &sh, uint32_t n_slots, unsigned long long *pstat = nullptr) {
     unsigned long long stall = 0;   // profiling aid (pstat != nullptr): ns this producer spent waiting for a free ring entry
     const uint32_t nch = ring_nch(K), CH = ring_chunk(K, nch);
     const uint32_t Q = (uint32_t)(((uint64_t)M * RG_STATIC_NUM) / (RG_STATIC_DEN * gridDim.x));   // static rows per CTA
-    const uint32_t pool0 = Q * gridDim.x, TR = ticket_rows(M, K, NM);
+    const uint32_t pool0 = Q * gridDim.x, TR = ticket_rows(M, K, NM, sizeof(WT));
     uint32_t njobs = 0;
     auto job = [&](uint32_t row) {
         for (uint32_t c = 0; c < nch; c++) {
@@ -230,8 +256,8 @@ __device__ __forceinline__ void produce(const float *W, const float *W3, uint32_
                 }
                 *reinterpret_cast<volatile unsigned *>(&sh.jobrow[slot]) = row;
                 __threadfence_block();
-                mbar_expect_tx(fb, len * 4);
-                bulk_g2s(ring_base + slot * RG_SLOT, (m == 0 ? W : W3) + (size_t)row * K + k0, len * 4, fb);
+                mbar_expect_tx(fb, len * (uint32_t)sizeof(WT));
+                bulk_g2s(ring_base + slot * RG_SLOT<WT>, (m == 0 ? W : W3) + (size_t)row * K + k0, len * (uint32_t)sizeof(WT), fb);
                 q.next(n_slots);
             }
         }
@@ -268,9 +294,9 @@ __device__ __forceinline__ void produce(const float *W, const float *W3, uint32_
 // (xs[c][v] = float4 (v * 32 + lane) of the warp's slice of chunk c).  EPI: 0 none, 1 + res[row];
 // NM == 2: out[row] = silu(W1[row].x) * (W3[row].x)
 // ---------------------------------------------------------------------------------------------------------
-template <int NM, int EPI, int NCH>
+template <typename WT, int NM, int EPI, int NCH, typename SH>
 __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], float *out, const float *res, RingPos &q, uint32_t phidx,
-                                        uint32_t ring_base, RingShared &sh, uint32_t n_slots, uint32_t spin_ns, bool peer_out = false) {
+                                        uint32_t ring_base, SH &sh, uint32_t n_slots, uint32_t spin_ns, bool peer_out = false) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t CH = ring_chunk(K, NCH);
     int buf = 0;
@@ -326,9 +352,9 @@ __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], 
             for (int m = 0; m < NM; m++) {
                 const uint32_t slot = q.slot;
                 if (c | m) mbar_wait(smem_u32(&sh.full[slot]), q.par, spin_ns);
-                const uint32_t base = ring_base + slot * RG_SLOT + ((uint32_t)warp * sl16 + (uint32_t)lane * 4) * 4u;
-                const float4 wa = v0 ? lds4(base) : make_float4(0.f, 0.f, 0.f, 0.f);
-                const float4 wb = v1 ? lds4(base + 512) : make_float4(0.f, 0.f, 0.f, 0.f);
+                const uint32_t base = ring_base + slot * RG_SLOT<WT> + ((uint32_t)warp * sl16 + (uint32_t)lane * 4) * (uint32_t)sizeof(WT);
+                const float4 wa = v0 ? lds_w4<WT>(base) : make_float4(0.f, 0.f, 0.f, 0.f);
+                const float4 wb = v1 ? lds_w4<WT>(base + 128 * (uint32_t)sizeof(WT)) : make_float4(0.f, 0.f, 0.f, 0.f);
                 float s = acc[m];
                 s = fmaf(wa.x, xs[c][0].x, s); s = fmaf(wa.y, xs[c][0].y, s); s = fmaf(wa.z, xs[c][0].z, s); s = fmaf(wa.w, xs[c][0].w, s);
                 s = fmaf(wb.x, xs[c][1].x, s); s = fmaf(wb.y, xs[c][1].y, s); s = fmaf(wb.z, xs[c][1].z, s); s = fmaf(wb.w, xs[c][1].w, s);
@@ -361,8 +387,8 @@ __device__ __forceinline__ uint32_t slice_index(uint32_t K, uint32_t CH, int c, 
 }
 // y = w * (x * f32(1/sqrt(mean_f64(x^2) + 1e-5)))   (ComputeForwardRMSNormFP32 + Mul, ml.go:1753-1812; llama.go:255-259)
 // The 16 warps' slices tile x exactly once, so the slice a thread keeps is also its share of the sum of squares: one L2 round trip.
-template <int NCH>
-__device__ __forceinline__ void fill_norm(float4 (&xs)[NCH][2], const float *x, const float *w, uint32_t K, RingShared &sh) {
+template <int NCH, typename SH>
+__device__ __forceinline__ void fill_norm(float4 (&xs)[NCH][2], const float *x, const float *w, uint32_t K, SH &sh) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t CH = ring_chunk(K, NCH);
     float4 ww[NCH][2];
@@ -413,8 +439,8 @@ __device__ __forceinline__ void fill_plain(float4 (&xs)[NCH][2], const float *x,
         }
 }
 // merge of the attention splits (see kernels_mega.cu::merged_attention_slice): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s)
-template <int HD, int NCH>
-__device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParams &p, RingShared &sh) {
+template <int HD, int NCH, typename SH>
+__device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParams &p, SH &sh) {
     const uint32_t S = p.splits, items = p.heads * S, K = p.dim, CH = ring_chunk(K, NCH);
     for (uint32_t i = threadIdx.x; i < items; i += RG_CTHREADS) {
         const float2 ml = __ldcg(reinterpret_cast<const float2 *>(p.part_ml) + i);
@@ -469,8 +495,8 @@ __device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParam
 }
 
 // ---- attention phase: identical to kernels_mega.cu::attention_phase (items (head, split), two per CTA at a time)
-template <int HD>
-__device__ __forceinline__ void attention_phase(const RingParams &p, const MegaLayerHost &L, uint32_t past, RingShared &sh, float *scores_all) {
+template <int HD, typename SH>
+__device__ __forceinline__ void attention_phase(const RingParams &p, const MegaLayerHost &L, uint32_t past, SH &sh, float *scores_all) {
     constexpr int LANES = HD / 4;
     constexpr int HW = RG_CWARPS / 2;
     constexpr int KG = RG_HALF / LANES;
@@ -593,13 +619,13 @@ __device__ __forceinline__ void attention_phase(const RingParams &p, const MegaL
 }
 
 // dynamic shared memory: [ring: n_slots x RG_SLOT][scores: 2 x chunk_cap floats][RingShared]
-template <int HD, int ND, int NF>
+template <typename WT, int HD, int ND, int NF>
 __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingParams p) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     const uint32_t dim = p.dim, ff = p.ff, n_slots = p.n_slots;
     uint8_t *ring = smem_raw;
-    float *scores = reinterpret_cast<float *>(smem_raw + (size_t)n_slots * RG_SLOT);
-    RingShared &sh = *reinterpret_cast<RingShared *>(scores + 2 * (size_t)((p.chunk_cap + 3) & ~3u));
+    float *scores = reinterpret_cast<float *>(smem_raw + (size_t)n_slots * RG_SLOT<WT>);
+    RingShared<RG_MAX_SLOTS<WT>> &sh = *reinterpret_cast<RingShared<RG_MAX_SLOTS<WT>> *>(scores + 2 * (size_t)((p.chunk_cap + 3) & ~3u));
     const bool producer = threadIdx.x >= RG_CTHREADS;
 
     if (threadIdx.x == 0) {
@@ -631,12 +657,12 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             const MegaLayerHost L = p.layers[li];
             // profiling aid: layer 5's producer wait time and job count per CTA and phase (after the 13 stamps per layer and the 5 x grid arrival stamps)
             unsigned long long *ps = (p.trace && li == 5 && p.n_layers > 6) ? p.trace + (size_t)p.n_layers * 13 + 5 * (size_t)gridDim.x : nullptr;
-            produce<1>(L.wqkv, nullptr, dim, 3 * dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps); phidx++;
-            produce<1>(L.wo, nullptr, dim, dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + gridDim.x : nullptr); phidx++;
-            produce<2>(L.w1, L.w3, dim, ff, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + 2 * gridDim.x : nullptr); phidx++;
-            produce<1>(L.w2, nullptr, ff, dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + 3 * gridDim.x : nullptr); phidx++;
+            produce<WT, 1>(wsel<WT>(L.wqkv, L.h_wqkv), (const WT *)nullptr, dim, 3 * dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps); phidx++;
+            produce<WT, 1>(wsel<WT>(L.wo, L.h_wo), (const WT *)nullptr, dim, dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + gridDim.x : nullptr); phidx++;
+            produce<WT, 2>(wsel<WT>(L.w1, L.h_w1), wsel<WT>(L.w3, L.h_w3), dim, ff, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + 2 * gridDim.x : nullptr); phidx++;
+            produce<WT, 1>(wsel<WT>(L.w2, L.h_w2), (const WT *)nullptr, ff, dim, pos, phidx, tk + phidx, ring_base, sh, n_slots, ps ? ps + 3 * gridDim.x : nullptr); phidx++;
         }
-        if (p.final_norm) produce<1>(p.output, nullptr, dim, p.vocab, pos, phidx, tk + phidx, ring_base, sh, n_slots);
+        if (p.final_norm) produce<WT, 1>(wsel<WT>(p.output, p.output_h), (const WT *)nullptr, dim, p.vocab, pos, phidx, tk + phidx, ring_base, sh, n_slots);
         return;
     }
     // ================= consumers =================
@@ -675,7 +701,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             float4 xs[ND][2];
             fill_norm<ND>(xs, xin, L.attention_norm, dim, sh);
             stamp(li, 1);
-            consume<1, 0, ND>(dim, xs, p.qkv, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
+            consume<WT, 1, 0, ND>(dim, xs, p.qkv, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 2);
         grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 0));
@@ -688,7 +714,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
         {   // ---- P3: merge the attention splits, wo + residual (llama.go:336-340)
             float4 xs[ND][2];
             fill_merge<HD, ND>(xs, p, sh);
-            consume<1, 1, ND>(dim, xs, p.y, xin, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
+            consume<WT, 1, 1, ND>(dim, xs, p.y, xin, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 6);
         grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 2));
@@ -697,7 +723,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             float4 xs[ND][2];
             fill_norm<ND>(xs, p.y, L.ffn_norm, dim, sh);
             stamp(li, 8);
-            consume<2, 0, ND>(dim, xs, p.act, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
+            consume<WT, 2, 0, ND>(dim, xs, p.act, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 9);
         grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 3));
@@ -706,7 +732,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             float4 xf[NF][2];
             fill_plain<NF>(xf, p.act, ff);
             const bool to_peer = p.p2p_x_out != nullptr && li + 1 == p.n_layers;
-            consume<1, 1, NF>(ff, xf, to_peer ? p.p2p_x_out : p.x, p.y, pos, phidx++, ring_base, sh, n_slots, p.spin_ns, to_peer);
+            consume<WT, 1, 1, NF>(ff, xf, to_peer ? p.p2p_x_out : p.x, p.y, pos, phidx++, ring_base, sh, n_slots, p.spin_ns, to_peer);
         }
         stamp(li, 11);
         grid_barrier(p.barrier, target, gridDim.x, p.p2p_x_out != nullptr && li + 1 == p.n_layers, arr(li, 4));
@@ -716,7 +742,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
     if (p.final_norm) {  // final norm + lm_head (llama.go:374-384)
         float4 xs[ND][2];
         fill_norm<ND>(xs, xin, p.final_norm, dim, sh);
-        consume<1, 0, ND>(dim, xs, p.logits, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
+        consume<WT, 1, 0, ND>(dim, xs, p.logits, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
     }
     if (p.p2p_flags && blockIdx.x == 0 && threadIdx.x == 0) {
         // every CTA passed the last grid barrier (system-scope fences below) after storing its rows of the residual
@@ -726,14 +752,14 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
     }
 }
 
-template <int HD, int ND, int NF>
+template <typename WT, int HD, int ND, int NF>
 static cudaError_t launch(const RingParams &p, size_t smem, cudaStream_t st) {
     static size_t attr[64] = {};  // function attributes are per device
     int dev = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     if (dev < 0 || dev >= 64 || attr[dev] < smem) {
-        e = cudaFuncSetAttribute(decode_ring_kernel<HD, ND, NF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        e = cudaFuncSetAttribute(decode_ring_kernel<WT, HD, ND, NF>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) attr[dev] = 227 * 1024;
     }
@@ -743,7 +769,7 @@ static cudaError_t launch(const RingParams &p, size_t smem, cudaStream_t st) {
     at[0].id = cudaLaunchAttributeCooperative;
     at[0].val.cooperative = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, decode_ring_kernel<HD, ND, NF>, p);
+    return cudaLaunchKernelEx(&cfg, decode_ring_kernel<WT, HD, ND, NF>, p);
 }
 // instantiated (chunks of dim, chunks of ff): (1,1) (1,2) test models — every head dim; (1,3) 7B, (2,4) 13B, (2,5) 30B, (2,6) 65B — head dim 128
 static bool ring_variant(uint32_t dim, uint32_t ff, uint32_t hd) {
@@ -752,9 +778,17 @@ static bool ring_variant(uint32_t dim, uint32_t ff, uint32_t hd) {
     if (hd != 128) return false;
     return (nd == 1 && nf == 3) || (nd == 2 && (nf == 4 || nf == 5 || nf == 6));
 }
-template <int HD>
+template <typename WT, int HD>
 static cudaError_t launch_small(const RingParams &p, uint32_t nf, size_t smem, cudaStream_t st) {
-    return nf == 1 ? launch<HD, 1, 1>(p, smem, st) : launch<HD, 1, 2>(p, smem, st);
+    return nf == 1 ? launch<WT, HD, 1, 1>(p, smem, st) : launch<WT, HD, 1, 2>(p, smem, st);
+}
+template <typename WT>
+static cudaError_t launch_shape(const RingParams &p, uint32_t hd, uint32_t nd, uint32_t nf, size_t smem, cudaStream_t st) {
+    if (nd == 1 && nf <= 2) return hd == 128 ? launch_small<WT, 128>(p, nf, smem, st) : hd == 64 ? launch_small<WT, 64>(p, nf, smem, st) : launch_small<WT, 32>(p, nf, smem, st);
+    if (nd == 1) return launch<WT, 128, 1, 3>(p, smem, st);
+    if (nf == 4) return launch<WT, 128, 2, 4>(p, smem, st);
+    if (nf == 5) return launch<WT, 128, 2, 5>(p, smem, st);
+    return launch<WT, 128, 2, 6>(p, smem, st);
 }
 
 static uint32_t ring_splits(uint32_t heads) {
@@ -762,14 +796,15 @@ static uint32_t ring_splits(uint32_t heads) {
     return s < 1 ? 1 : (s > 32 ? 32 : s);
 }
 // shared-memory plan: returns the number of ring slots (0 = does not fit)
+template <typename WT>
 static uint32_t ring_plan(uint32_t heads, uint32_t ctx, size_t *smem_out) {
     const uint32_t S = ring_splits(heads), chunk_cap = (ctx + S - 1) / S;
-    const size_t fixed = 2 * (size_t)((chunk_cap + 3) & ~3u) * 4 + sizeof(RingShared) + 128;
+    const size_t fixed = 2 * (size_t)((chunk_cap + 3) & ~3u) * 4 + sizeof(RingShared<RG_MAX_SLOTS<WT>>) + 128;
     const size_t cap = 227 * 1024;
-    if (fixed + 4 * (size_t)RG_SLOT > cap) return 0;
-    uint32_t n = (uint32_t)((cap - fixed) / RG_SLOT);
-    if (n > RG_MAX_SLOTS) n = RG_MAX_SLOTS;
-    if (smem_out) *smem_out = fixed - 128 + (size_t)n * RG_SLOT;
+    if (fixed + 4 * (size_t)RG_SLOT<WT> > cap) return 0;
+    uint32_t n = (uint32_t)((cap - fixed) / RG_SLOT<WT>);
+    if (n > (uint32_t)RG_MAX_SLOTS<WT>) n = RG_MAX_SLOTS<WT>;
+    if (smem_out) *smem_out = fixed - 128 + (size_t)n * RG_SLOT<WT>;
     return n;
 }
 
@@ -788,7 +823,7 @@ bool decode_ring_supported(uint32_t dim, uint32_t ff, uint32_t heads, uint32_t v
     if (hd != 128 && hd != 64 && hd != 32) return false;
     if (dim % 64 || ff % 64) return false;             // every warp's 1/16 slice of a chunk is whole float4s; 16-byte bulk copies
     if (!ring_variant(dim, ff, hd)) return false;
-    return ring_plan(heads, ctx, nullptr) >= 4;
+    return ring_plan<float>(heads, ctx, nullptr) >= 4;   // (an F16 ring has slots of half the size: it fits wherever this does)
 }
 
 void decode_ring(const MegaParamsHost &h, cudaStream_t st) {
@@ -797,17 +832,17 @@ void decode_ring(const MegaParamsHost &h, cudaStream_t st) {
     p.layers = h.layers_dev;
     p.n_layers = h.n_layers;
     p.tok_embeddings = h.tok_embeddings; p.tokens = h.tokens; p.state = h.state;
-    p.final_norm = h.final_norm; p.output = h.output;
+    p.final_norm = h.final_norm; p.output = h.output; p.output_h = h.h_output;
     p.x = h.x; p.y = h.y; p.qkv = h.qkv; p.attn = h.attn; p.act = h.act; p.logits = h.logits;
     p.part_o = h.part_o; p.part_ml = h.part_ml; p.barrier = h.barrier;
     p.dim = h.dim; p.ff = h.ff; p.heads = h.heads; p.vocab = h.vocab; p.ctx = h.ctx;
     p.splits = ring_splits(h.heads);
     p.chunk_cap = (h.ctx + p.splits - 1) / p.splits;
     size_t smem = 0;
-    p.n_slots = ring_plan(h.heads, h.ctx, &smem);
+    p.n_slots = h.f16 ? ring_plan<__half>(h.heads, h.ctx, &smem) : ring_plan<float>(h.heads, h.ctx, &smem);
     if (const char *e = getenv("LB_RING_SLOTS")) {   // profiling aid: a shallower ring
         const uint32_t n = (uint32_t)atoi(e);
-        if (n >= 2 && n < p.n_slots) { smem -= (size_t)(p.n_slots - n) * RG_SLOT; p.n_slots = n; }
+        if (n >= 2 && n < p.n_slots) { smem -= (size_t)(p.n_slots - n) * (h.f16 ? RG_SLOT<__half> : RG_SLOT<float>); p.n_slots = n; }
     }
     p.trace = reinterpret_cast<unsigned long long *>(h.trace);
     static const uint32_t spin_ns = getenv("LB_RING_SPIN_NS") ? (uint32_t)atoi(getenv("LB_RING_SPIN_NS")) : 50u;   // no effect on an un-capped box (r02q); fewer polls = less power under the 1 kW cap
@@ -816,13 +851,7 @@ void decode_ring(const MegaParamsHost &h, cudaStream_t st) {
     p.p2p_x_out = h.p2p_x_out; p.p2p_flag_out = h.p2p_flag_out; p.p2p_ack_out = h.p2p_ack_out;
     LB_CUDA(cudaMemsetAsync(h.barrier, 0, sizeof(unsigned) * (3 + 4 * (size_t)h.n_layers), st));   // grid barrier + per-phase row tickets
     const uint32_t hd = h.dim / h.heads, nd = ring_nch(h.dim), nf = ring_nch(h.ff);
-    cudaError_t e;
-    if (nd == 1 && nf <= 2) e = hd == 128 ? launch_small<128>(p, nf, smem, st) : hd == 64 ? launch_small<64>(p, nf, smem, st) : launch_small<32>(p, nf, smem, st);
-    else if (nd == 1) e = launch<128, 1, 3>(p, smem, st);
-    else if (nf == 4) e = launch<128, 2, 4>(p, smem, st);
-    else if (nf == 5) e = launch<128, 2, 5>(p, smem, st);
-    else e = launch<128, 2, 6>(p, smem, st);
-    LB_CUDA(e);
+    LB_CUDA(h.f16 ? launch_shape<__half>(p, hd, nd, nf, smem, st) : launch_shape<float>(p, hd, nd, nf, smem, st));
     count_launch();
 }
 

@@ -16,10 +16,15 @@
 // (K = 256), then an accumulate warp-group adds that partial tile into FP32 registers (round to
 // nearest) while the MMA warp fills the other TMEM buffer.
 //
-// Q8_0 weights (template Q8 = true): the weight operand arrives as the int8 tile (4 KB) + its block
+// Q8_0 weights (WK_Q8): the weight operand arrives as the int8 tile (4 KB) + its block
 // scales (512 B) by TMA from the 4-row-interleaved planes of kernels_q8.cu, and the transform warp-group
 // DEQUANTISES IN THE SHARED-MEMORY STAGE: v = f32(d*q) is written as the hi operand and v - trunc(v)
 // as the lo operand, both at the 128-byte-swizzled K-major positions the MMA descriptors expect.
+//
+// F16 weights (WK_F16): the weight operand arrives as the row-major binary16 tile (128 rows x 64 B, 8 KB) by TMA into
+// the stage's a_lo buffer, and the transform warp-group widens it to FP32 into a_raw at the swizzled K-major positions.
+// Every binary16 value (subnormals included) is exact in TF32, so the weight's lo part is zero: each K step issues
+// two MMAs, a*b_lo + a*b_hi, with the same two-level accumulation.
 //
 // Warp roles (320 threads, 1 CTA per SM, one 128x128 output tile per CTA):
 //   warp 0      : TMA producer (one elected lane)
@@ -31,6 +36,7 @@
 //            tmem_empty[b] (accumulate -> MMA).
 // Every wait has a clock-based timeout that traps instead of hanging the GPU.
 #include <cuda.h>
+#include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
@@ -50,6 +56,8 @@ constexpr uint32_t TC_A_BYTES = TC_BM * TC_BK * 4;  // 16 KB
 constexpr uint32_t TC_B_BYTES = TC_BN * TC_BK * 4;  // 16 KB
 constexpr uint32_t TC_Q_BYTES = TC_BM * TC_BK;              // int8 weight tile (Q8 mode): 32 row groups x 128 B
 constexpr uint32_t TC_D_BYTES = (TC_BM / 4) * 16;           // its scales: one float4 per row group
+constexpr uint32_t TC_H_BYTES = TC_BM * TC_BK * 2;          // binary16 weight tile (F16 mode), staged in the a_lo buffer
+enum WeightKind { WK_F32 = 0, WK_Q8 = 1, WK_F16 = 2 };
 constexpr uint32_t TC_STAGE_BYTES = 2 * TC_A_BYTES + 2 * TC_B_BYTES + TC_Q_BYTES + 1024;  // raw + lo for A and B, q tile, scales (padded)
 constexpr uint32_t TC_SMEM_BYTES = TC_STAGES * TC_STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
 
@@ -147,7 +155,7 @@ __device__ __forceinline__ void tc_unpack4(uint32_t w, float f[4]) {
     f[3] = __uint_as_float(__byte_perm(u, 0x4B000000u, 0x7653)) - 8388736.0f;
 }
 
-template <bool Q8>
+template <int WK>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmD,
                    const __grid_constant__ CUtensorMap tmX, float *__restrict__ Y,
@@ -199,10 +207,13 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
                 const int s = kb % TC_STAGES;
                 const uint32_t ph = (kb / TC_STAGES) & 1;
                 mbar_wait(empty(s), ph ^ 1);
-                if (Q8) {
+                if (WK == WK_Q8) {
                     mbar_expect_tx(full_raw(s), TC_Q_BYTES + TC_D_BYTES + TC_B_BYTES);
                     tma_load_2d(q_tile(s), &tmW, full_raw(s), (int)(kb * TC_BK * 4), (int)(m0 / 4));  // 128 B per row group
                     tma_load_2d(d_tile(s), &tmD, full_raw(s), (int)(kb * 4), (int)(m0 / 4));           // one float4 per row group
+                } else if (WK == WK_F16) {
+                    mbar_expect_tx(full_raw(s), TC_H_BYTES + TC_B_BYTES);
+                    tma_load_2d(a_lo(s), &tmW, full_raw(s), (int)(kb * TC_BK), (int)m0);             // 64 B per row, unswizzled
                 } else {
                     mbar_expect_tx(full_raw(s), TC_A_BYTES + TC_B_BYTES);
                     tma_load_2d(a_raw(s), &tmW, full_raw(s), (int)(kb * TC_BK), (int)m0);
@@ -232,9 +243,14 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
                     const uint32_t koff = kk * TC_UK * 4;  // 32 bytes per K step inside the swizzled row
                     const uint64_t dA = make_smem_desc(a_raw(s) + koff), dAl = make_smem_desc(a_lo(s) + koff);
                     const uint64_t dB = make_smem_desc(b_raw(s) + koff), dBl = make_smem_desc(b_lo(s) + koff);
-                    tc_mma_tf32(tmem_d, dAl, dB, idesc, (first_of_chunk && kk == 0) ? 0u : 1u);  // a_lo * b_hi
-                    tc_mma_tf32(tmem_d, dA, dBl, idesc, 1u);                                     // a_hi * b_lo
-                    tc_mma_tf32(tmem_d, dA, dB, idesc, 1u);                                      // a_hi * b_hi
+                    if (WK == WK_F16) {   // a is exact in TF32: no a_lo term
+                        tc_mma_tf32(tmem_d, dA, dBl, idesc, (first_of_chunk && kk == 0) ? 0u : 1u);  // a * b_lo
+                        tc_mma_tf32(tmem_d, dA, dB, idesc, 1u);                                      // a * b_hi
+                    } else {
+                        tc_mma_tf32(tmem_d, dAl, dB, idesc, (first_of_chunk && kk == 0) ? 0u : 1u);  // a_lo * b_hi
+                        tc_mma_tf32(tmem_d, dA, dBl, idesc, 1u);                                     // a_hi * b_lo
+                        tc_mma_tf32(tmem_d, dA, dB, idesc, 1u);                                      // a_hi * b_hi
+                    }
                 }
                 tc_commit(empty(s));  // frees the stage once these MMAs have read it
                 if ((kb % TC_CHUNK_KB) == TC_CHUNK_KB - 1 || kb == num_kb - 1) tc_commit(tmem_full(buf));
@@ -252,7 +268,7 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
             const float4 *br = reinterpret_cast<const float4 *>(base_ptr + s * TC_STAGE_BYTES + 2 * TC_A_BYTES);
             float4 *bl = reinterpret_cast<float4 *>(base_ptr + s * TC_STAGE_BYTES + 2 * TC_A_BYTES + TC_B_BYTES);
             auto lo = [](float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); };
-            if (Q8) {
+            if (WK == WK_Q8) {
                 // dequantise in the shared-memory stage: 256 vectors (row group g, k4) of 4 rows x 4 int8
                 const uint4 *qt = reinterpret_cast<const uint4 *>(base_ptr + s * TC_STAGE_BYTES + 2 * TC_A_BYTES + 2 * TC_B_BYTES);
                 const float4 *dt = reinterpret_cast<const float4 *>(base_ptr + s * TC_STAGE_BYTES + 2 * TC_A_BYTES + 2 * TC_B_BYTES + TC_Q_BYTES);
@@ -274,6 +290,23 @@ gemm_tf32x3_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constan
                         ah[off] = v;
                         al[off] = make_float4(lo(v.x), lo(v.y), lo(v.z), lo(v.w));
                     }
+                }
+            } else if (WK == WK_F16) {
+                // widen in the shared-memory stage: 512 vectors (row, 8 halves) of the unswizzled tile in the a_lo buffer
+                const uint4 *ht = reinterpret_cast<const uint4 *>(al);
+                float4 *ah = reinterpret_cast<float4 *>(base_ptr + s * TC_STAGE_BYTES);
+                uint4 hv[TC_H_BYTES / 16 / 128];
+#pragma unroll
+                for (int i = 0; i < (int)(TC_H_BYTES / 16 / 128); i++) hv[i] = ht[t + i * 128];
+#pragma unroll
+                for (int i = 0; i < (int)(TC_H_BYTES / 16 / 128); i++) {
+                    const int vec = t + i * 128, row = vec >> 2, k8 = vec & 3;
+                    const float2 f0 = __half22float2(*reinterpret_cast<const __half2 *>(&hv[i].x));
+                    const float2 f1 = __half22float2(*reinterpret_cast<const __half2 *>(&hv[i].y));
+                    const float2 f2 = __half22float2(*reinterpret_cast<const __half2 *>(&hv[i].z));
+                    const float2 f3 = __half22float2(*reinterpret_cast<const __half2 *>(&hv[i].w));
+                    ah[row * 8 + ((2 * k8) ^ (row & 7))] = make_float4(f0.x, f0.y, f1.x, f1.y);       // float4 index inside the swizzled tile
+                    ah[row * 8 + ((2 * k8 + 1) ^ (row & 7))] = make_float4(f2.x, f2.y, f3.x, f3.y);
                 }
             } else {
 #pragma unroll
@@ -380,14 +413,14 @@ bool gemm_tf32x3_supported(uint32_t M, uint32_t K, uint32_t ldx, const float *W,
     return K >= TC_BK && (K % TC_BK) == 0 && (ldx % 4) == 0 && ((uintptr_t)W % 16) == 0 && ((uintptr_t)X % 16) == 0;
 }
 
-template <bool Q8>
+template <int WK>
 static void set_attr_once() {
     // function attributes are per device: the C-ABI lets one process hold models on several GPUs
     static bool attr[64] = {};
     int dev = 0;
     LB_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || !attr[dev]) {
-        LB_CUDA(cudaFuncSetAttribute(gemm_tf32x3_kernel<Q8>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
+        LB_CUDA(cudaFuncSetAttribute(gemm_tf32x3_kernel<WK>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_BYTES));
         if (dev >= 0 && dev < 64) attr[dev] = true;
     }
 }
@@ -396,11 +429,11 @@ void gemm_tf32x3(const float *W, uint32_t M, uint32_t K, const float *X, uint32_
                  const float *residual, cudaStream_t st) {
     LB_CHECK(gemm_tf32x3_supported(M, K, ldx, W, X), "gemm_tf32x3: unsupported shape (K must be a multiple of 32)");
     if (!M || !N) return;
-    set_attr_once<false>();
+    set_attr_once<WK_F32>();
     CUtensorMap tmW = make_map(W, M, K, K, TC_BM);
     CUtensorMap tmX = make_map(X, N, K, ldx, TC_BN);
     dim3 grid((M + TC_BM - 1) / TC_BM, (N + TC_BN - 1) / TC_BN);
-    gemm_tf32x3_kernel<false><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmW, tmW, tmX, Y, ldy, residual, M, N, K);
+    gemm_tf32x3_kernel<WK_F32><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmW, tmW, tmX, Y, ldy, residual, M, N, K);
     LB_LAUNCH_CHECK();
 }
 
@@ -411,14 +444,28 @@ void gemm_q8_tc(const int8_t *Q, const float *D, uint32_t M, uint32_t K, const f
     LB_CHECK(K >= TC_BK && K % TC_BK == 0 && M % 4 == 0 && ldx % 4 == 0 && (uintptr_t)Q % 16 == 0 && (uintptr_t)D % 16 == 0 &&
                  (uintptr_t)X % 16 == 0, "gemm_q8_tc: unsupported shape");
     if (!M || !N) return;
-    set_attr_once<true>();
+    set_attr_once<WK_Q8>();
     CUtensorMap tmQ = make_map_raw(Q, CU_TENSOR_MAP_DATA_TYPE_UINT8, M / 4, (uint64_t)K * 4, (uint64_t)K * 4, TC_BK * 4, TC_BM / 4,
                                    CU_TENSOR_MAP_SWIZZLE_NONE);
     CUtensorMap tmD = make_map_raw(D, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, M / 4, (uint64_t)(K / 32) * 4, (uint64_t)(K / 32) * 16, 4, TC_BM / 4,
                                    CU_TENSOR_MAP_SWIZZLE_NONE);
     CUtensorMap tmX = make_map(X, N, K, ldx, TC_BN);
     dim3 grid((M + TC_BM - 1) / TC_BM, (N + TC_BN - 1) / TC_BN);
-    gemm_tf32x3_kernel<true><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmQ, tmD, tmX, Y, ldy, residual, M, N, K);
+    gemm_tf32x3_kernel<WK_Q8><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmQ, tmD, tmX, Y, ldy, residual, M, N, K);
+    LB_LAUNCH_CHECK();
+}
+
+// F16 weights: row-major [M][K] binary16 plane; box = 32 halves (64 B) x 128 rows, unswizzled (widened by the transform warps)
+void gemm_f16_tc(const uint16_t *W, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N, float *Y, uint32_t ldy,
+                 const float *residual, cudaStream_t st) {
+    LB_CHECK(K >= TC_BK && K % TC_BK == 0 && ldx % 4 == 0 && (uintptr_t)W % 16 == 0 && (uintptr_t)X % 16 == 0,
+             "gemm_f16_tc: unsupported shape (K must be a multiple of 32)");
+    if (!M || !N) return;
+    set_attr_once<WK_F16>();
+    CUtensorMap tmW = make_map_raw(W, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, M, K, (uint64_t)K * 2, TC_BK, TC_BM, CU_TENSOR_MAP_SWIZZLE_NONE);
+    CUtensorMap tmX = make_map(X, N, K, ldx, TC_BN);
+    dim3 grid((M + TC_BM - 1) / TC_BM, (N + TC_BN - 1) / TC_BN);
+    gemm_tf32x3_kernel<WK_F16><<<grid, TC_THREADS, TC_SMEM_BYTES, st>>>(tmW, tmW, tmX, Y, ldy, residual, M, N, K);
     LB_LAUNCH_CHECK();
 }
 

@@ -33,23 +33,26 @@ Model::Model(const HParams &h, int dev, uint32_t lb_, uint32_t le_, int wt) : hp
     LB_CHECK(hp.dim % hp.heads == 0, "model: dim must be divisible by heads");
     LB_CHECK(hp.dim % 4 == 0, "model: dim must be a multiple of 4");
     LB_CHECK(layer_begin < layer_end && layer_end <= hp.layers, "model: bad layer range");
-    LB_CHECK(wt == 0 || wt == 16, "model: weight type must be LB_TYPE_F32 or LB_TYPE_Q8_0");
+    LB_CHECK(wt == 0 || wt == 1 || wt == 16, "model: weight type must be LB_TYPE_F32, LB_TYPE_F16 or LB_TYPE_Q8_0");
     if (q8()) LB_CHECK(hp.dim % 32 == 0 && hp.ff() % 32 == 0 && hp.vocab % 4 == 0, "model: Q8_0 needs dim and ff to be multiples of 32 and vocab of 4");
+    // F16: the tcgen05 prefill GEMM always applies (K % 32) and every row is a whole number of 64-byte bulk-copy units
+    if (f16()) LB_CHECK(hp.dim % 32 == 0 && hp.ff() % 32 == 0, "model: F16 needs dim and ff to be multiples of 32");
     LB_CUDA(cudaSetDevice(device));
     const size_t d = hp.dim, ff = hp.ff(), V = hp.vocab;
     const size_t A = 64;  // floats: 256-byte alignment of every tensor
-    size_t total = 0, qtotal = 0, dtotal = 0;
+    size_t total = 0, qtotal = 0, dtotal = 0, htotal = 0;
     auto reserve = [&](size_t n) { size_t off = total; total += align_up(n, A); return off; };
-    // a MulMat matrix: float slab (F32) or q/d planes (Q8_0); returns {float off, q off, d off}
-    struct MOff { size_t f, q, d; };
+    // a MulMat matrix: float slab (F32), q/d planes (Q8_0) or half slab (F16); returns {float off, q off, d off, half off}
+    struct MOff { size_t f, q, d, h; };
     auto reserve_mat = [&](size_t n) {
-        MOff o{0, 0, 0};
+        MOff o{0, 0, 0, 0};
         if (q8()) { o.q = qtotal; qtotal += align_up(n, 512); o.d = dtotal; dtotal += align_up(n / 32, A); }   // 512 = one 16 x 32 tile block (tile-major plane offsets)
+        else if (f16()) { o.h = htotal; htotal += align_up(n, 2 * A); }   // 256-byte alignment
         else o.f = reserve(n);
         return o;
     };
     size_t o_emb = 0, o_norm = 0;
-    MOff o_out{0, 0, 0};
+    MOff o_out{0, 0, 0, 0};
     if (has_embedding()) o_emb = reserve(V * d);
     if (has_head()) { o_norm = reserve(d); o_out = reserve_mat(V * d); }
     struct LOff { size_t an, fn; MOff qkv, wo, w1, w2, w3; };
@@ -66,7 +69,12 @@ Model::Model(const HParams &h, int dev, uint32_t lb_, uint32_t le_, int wt) : hp
         dslab = mem.dmalloc<float>(dtotal);
         tmslab = mem.dmalloc<uint8_t>(qtotal / 512 * 576 + 256);   // every matrix: (rows / 16) x (K / 32) records of 576 bytes
     }
-    auto fptr = [&](const MOff &o) { return q8() ? nullptr : slab + o.f; };
+    if (f16()) {
+        hslab = mem.dmalloc<uint16_t>(htotal);
+        f16_overflow = mem.dmalloc<unsigned>(1);
+    }
+    auto fptr = [&](const MOff &o) { return f32() ? slab + o.f : nullptr; };
+    auto hptr = [&](const MOff &o) { return f16() ? hslab + o.h : nullptr; };
     // (matrix offsets o.q are multiples of 512 elements; the decode plane holds 36 bytes per 32 elements, k::q8_tile_major_bytes)
     auto qmat = [&](const MOff &o, size_t rows_total, size_t cols, size_t row_off = 0) {
         Q8Mat m;
@@ -83,9 +91,9 @@ Model::Model(const HParams &h, int dev, uint32_t lb_, uint32_t le_, int wt) : hp
         tensors["tok_embeddings.weight"] = {tok_embeddings, V * d, 1, 0.f, 1.f, Q8Mat()};
     }
     if (has_head()) {
-        norm = slab + o_norm; output = fptr(o_out); output8 = qmat(o_out, V, d);
+        norm = slab + o_norm; output = fptr(o_out); output8 = qmat(o_out, V, d); outputh = hptr(o_out);
         tensors["norm.weight"] = {norm, d, 2, 1.f, 0.1f, Q8Mat()};
-        tensors["output.weight"] = {output, V * d, 3, 0.f, sdd, output8, (uint32_t)d};
+        tensors["output.weight"] = {output, V * d, 3, 0.f, sdd, output8, (uint32_t)d, outputh};
     }
     layers.resize(lo.size());
     for (size_t i = 0; i < lo.size(); i++) {
@@ -93,19 +101,21 @@ Model::Model(const HParams &h, int dev, uint32_t lb_, uint32_t le_, int wt) : hp
         L.attention_norm = slab + lo[i].an; L.ffn_norm = slab + lo[i].fn;
         L.wqkv = fptr(lo[i].qkv); L.wo = fptr(lo[i].wo); L.w1 = fptr(lo[i].w1); L.w3 = fptr(lo[i].w3); L.w2 = fptr(lo[i].w2);
         L.wqkv8 = qmat(lo[i].qkv, 3 * d, d); L.wo8 = qmat(lo[i].wo, d, d); L.w18 = qmat(lo[i].w1, ff, d); L.w38 = qmat(lo[i].w3, ff, d); L.w28 = qmat(lo[i].w2, d, ff);
+        L.wqkvh = hptr(lo[i].qkv); L.woh = hptr(lo[i].wo); L.w1h = hptr(lo[i].w1); L.w3h = hptr(lo[i].w3); L.w2h = hptr(lo[i].w2);
         uint32_t il = layer_begin + (uint32_t)i;
         std::string p = "layers." + std::to_string(il) + ".";
         uint64_t base = 16ull * (il + 1);
-        auto fq = [&](size_t rows_off) { return q8() ? nullptr : L.wqkv + rows_off; };
+        auto fq = [&](size_t rows_off) { return f32() ? L.wqkv + rows_off : nullptr; };
+        auto hq = [&](size_t rows_off) { return f16() ? L.wqkvh + rows_off : nullptr; };
         tensors[p + "attention_norm.weight"] = {L.attention_norm, d, base + 0, 1.f, 0.1f, Q8Mat()};
-        tensors[p + "attention.wq.weight"] = {fq(0), d * d, base + 1, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, 0), (uint32_t)d};
-        tensors[p + "attention.wk.weight"] = {fq(d * d), d * d, base + 2, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, d), (uint32_t)d};
-        tensors[p + "attention.wv.weight"] = {fq(2 * d * d), d * d, base + 3, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, 2 * d), (uint32_t)d};
-        tensors[p + "attention.wo.weight"] = {L.wo, d * d, base + 4, 0.f, sdd, L.wo8, (uint32_t)d};
+        tensors[p + "attention.wq.weight"] = {fq(0), d * d, base + 1, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, 0), (uint32_t)d, hq(0)};
+        tensors[p + "attention.wk.weight"] = {fq(d * d), d * d, base + 2, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, d), (uint32_t)d, hq(d * d)};
+        tensors[p + "attention.wv.weight"] = {fq(2 * d * d), d * d, base + 3, 0.f, sdd, qmat(lo[i].qkv, 3 * d, d, 2 * d), (uint32_t)d, hq(2 * d * d)};
+        tensors[p + "attention.wo.weight"] = {L.wo, d * d, base + 4, 0.f, sdd, L.wo8, (uint32_t)d, L.woh};
         tensors[p + "ffn_norm.weight"] = {L.ffn_norm, d, base + 5, 1.f, 0.1f, Q8Mat()};
-        tensors[p + "feed_forward.w1.weight"] = {L.w1, ff * d, base + 6, 0.f, sdd, L.w18, (uint32_t)d};
-        tensors[p + "feed_forward.w2.weight"] = {L.w2, d * ff, base + 7, 0.f, sf, L.w28, (uint32_t)ff};
-        tensors[p + "feed_forward.w3.weight"] = {L.w3, ff * d, base + 8, 0.f, sdd, L.w38, (uint32_t)d};
+        tensors[p + "feed_forward.w1.weight"] = {L.w1, ff * d, base + 6, 0.f, sdd, L.w18, (uint32_t)d, L.w1h};
+        tensors[p + "feed_forward.w2.weight"] = {L.w2, d * ff, base + 7, 0.f, sf, L.w28, (uint32_t)ff, L.w2h};
+        tensors[p + "feed_forward.w3.weight"] = {L.w3, ff * d, base + 8, 0.f, sdd, L.w38, (uint32_t)d, L.w3h};
     }
 }
 
@@ -114,7 +124,8 @@ Model::~Model() {}  // `mem` releases the slabs
 void Model::set_tensor(const std::string &name, int dtype, const void *host, size_t nbytes) {
     // LoadModel's tensor loop, llama.go:889-959: unknown names abort (:906-910); only F32 and F16
     // are accepted (:937-959), F16 is widened to FP32.  With Q8_0 weights the MulMat matrices are
-    // block-quantised on the device as they arrive.
+    // block-quantised on the device as they arrive; with F16 weights they keep F16 input byte for
+    // byte and round F32 input to nearest even.
     LB_CHECK(known_name(hp, name), "Unknown tensor '" + name + "' in model file");
     auto it = tensors.find(name);
     if (it == tensors.end()) return;  // belongs to another pipeline stage
@@ -123,6 +134,20 @@ void Model::set_tensor(const std::string &name, int dtype, const void *host, siz
     const size_t esz = dtype == 0 ? 4 : 2;
     LB_CHECK(nbytes == e.nelem * esz, "tensor '" + name + "' has the wrong size");
     LB_CUDA(cudaSetDevice(device));
+    if (e.h) {
+        if (dtype == 1) {
+            LB_CUDA(cudaMemcpy(e.h, host, nbytes, cudaMemcpyHostToDevice));
+        } else {
+            void *tmp = nullptr;
+            LB_CUDA(cudaMalloc(&tmp, nbytes));
+            try {
+                LB_CUDA(cudaMemcpy(tmp, host, nbytes, cudaMemcpyHostToDevice));
+                round_to_f16(static_cast<const float *>(tmp), e.h, e.nelem, name, 0);
+            } catch (...) { cudaFree(tmp); throw; }
+            cudaFree(tmp);
+        }
+        return;
+    }
     const bool quant = e.q8.q != nullptr;
     float *dst = e.ptr;
     void *tmp16 = nullptr, *tmp32 = nullptr;
@@ -143,13 +168,29 @@ void Model::set_tensor(const std::string &name, int dtype, const void *host, siz
     if (tmp32) cudaFree(tmp32);
 }
 
+void Model::round_to_f16(const float *src, uint16_t *dst, size_t n, const std::string &name, cudaStream_t st) {
+    unsigned over = 0;
+    LB_CUDA(cudaMemsetAsync(f16_overflow, 0, sizeof(unsigned), st));
+    k::f32_to_f16(src, dst, n, f16_overflow, st);
+    LB_CUDA(cudaMemcpyAsync(&over, f16_overflow, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
+    LB_CUDA(cudaStreamSynchronize(st));
+    LB_CHECK(over == 0, "tensor '" + name + "' holds a finite value outside the F16 range (|x| > 65504)");
+}
+
 void Model::get_tensor(const std::string &name, float *host, size_t nelem) {
     auto it = tensors.find(name);
     LB_CHECK(it != tensors.end(), "tensor '" + name + "' is not held by this stage");
     const Entry &e = it->second;
     LB_CHECK(nelem == e.nelem, "tensor '" + name + "' has the wrong size");
     LB_CUDA(cudaSetDevice(device));
-    if (e.q8.q) {
+    if (e.h) {
+        void *tmp = nullptr;
+        LB_CUDA(cudaMalloc(&tmp, nelem * sizeof(float)));
+        k::f16_to_f32(e.h, static_cast<float *>(tmp), nelem, 0);
+        const cudaError_t err = cudaMemcpy(host, tmp, nelem * sizeof(float), cudaMemcpyDeviceToHost);
+        cudaFree(tmp);
+        LB_CUDA(err);
+    } else if (e.q8.q) {
         void *tmp = nullptr;
         LB_CUDA(cudaMalloc(&tmp, nelem * sizeof(float)));
         k::dequantize_q8(e.q8.q, e.q8.d, static_cast<float *>(tmp), (uint32_t)(nelem / e.cols), e.cols, 0);
@@ -165,7 +206,7 @@ void Model::init_random(uint64_t seed) {
     void *tmp = nullptr;
     size_t tmp_elems = 0;
     for (auto &kv : tensors)
-        if (kv.second.q8.q && kv.second.nelem > tmp_elems) tmp_elems = kv.second.nelem;
+        if ((kv.second.q8.q || kv.second.h) && kv.second.nelem > tmp_elems) tmp_elems = kv.second.nelem;
     if (tmp_elems) LB_CUDA(cudaMalloc(&tmp, tmp_elems * sizeof(float)));
     for (auto &kv : tensors) {
         const Entry &e = kv.second;
@@ -175,6 +216,9 @@ void Model::init_random(uint64_t seed) {
             k::init_random(static_cast<float *>(tmp), e.nelem, seed, e.tid, e.mean, sscale, 0);
             k::quantize_q8(static_cast<float *>(tmp), e.q8.q, e.q8.d, (uint32_t)(e.nelem / e.cols), e.cols, 0);
             k::q8_to_tile_major(e.q8.q, e.q8.d, e.q8.tm, e.q8.tm_rows, e.q8.tm_row0, (uint32_t)(e.nelem / e.cols), e.cols, 0);
+        } else if (e.h) {
+            k::init_random(static_cast<float *>(tmp), e.nelem, seed, e.tid, e.mean, sscale, 0);
+            round_to_f16(static_cast<const float *>(tmp), e.h, e.nelem, kv.first, 0);
         } else {
             k::init_random(e.ptr, e.nelem, seed, e.tid, e.mean, sscale, 0);
         }
@@ -186,11 +230,11 @@ void Model::init_random(uint64_t seed) {
 uint64_t Model::weight_bytes_per_token() const {
     // SURVEY §8(d): every layer matrix + both norms, lm_head, final norm, one embedding row
     const uint64_t d = hp.dim, ff = hp.ff(), V = hp.vocab;
-    // matrices cost 4 B/weight (F32) or 36 B per 32 weights (Q8_0); vectors are always F32
+    // matrices cost 4 B/weight (F32), 2 B/weight (F16) or 36 B per 32 weights (Q8_0); vectors are always F32
     const uint64_t nl = layer_end - layer_begin;
     uint64_t mat = nl * (4 * d * d + 3 * d * ff) + (has_head() ? V * d : 0);
     uint64_t vec = nl * 2 * d + (has_head() ? d : 0) + (has_embedding() ? d : 0);
-    return (q8() ? mat / 32 * 36 : mat * 4) + vec * 4;
+    return (q8() ? mat / 32 * 36 : f16() ? mat * 2 : mat * 4) + vec * 4;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -224,7 +268,8 @@ Context::Context(Model *m, uint32_t cs) : model(m), ctx_size(cs) {
     //  slower — 173 vs 240 tok/s on 7B, too few bytes in flight per warp with 1-byte weights)
     const bool mega_ok = k::decode_mega_supported(hp.dim, hp.ff(), hp.heads);
     const bool ring_ok = getenv("LB_NO_RING") == nullptr && k::decode_ring_supported(hp.dim, hp.ff(), hp.heads, hp.vocab, cs);
-    use_mega = getenv("LB_NO_MEGA") == nullptr && !m->q8() && (mega_ok || ring_ok);
+    // (F16 models: only the TMA-ring megakernel has an F16 weight stream; the register-fed one never runs them)
+    use_mega = getenv("LB_NO_MEGA") == nullptr && ((m->f32() && (mega_ok || ring_ok)) || (m->f16() && ring_ok));
     // TMA-ring megakernel (kernels_ring.cu, version 3): 234 vs 221 tok/s on an un-capped box, 224 vs 216 under the power cap
     // (profiles/README.md r02o/r02p) — the default; LB_NO_RING=1 keeps the register-fed megakernel (kernels_mega.cu)
     use_ring = use_mega && ring_ok;
@@ -238,7 +283,8 @@ Context::Context(Model *m, uint32_t cs) : model(m), ctx_size(cs) {
             const Layer &L = m->layers[i];
             ml[i] = {L.attention_norm, L.wqkv, L.wo, L.ffn_norm, L.w1, L.w3, L.w2,
                      kv_k + i * (size_t)cs * d, kv_v + i * (size_t)cs * d,
-                     L.wqkv8.q, L.wo8.q, L.w18.q, L.w38.q, L.w28.q, L.wqkv8.d, L.wo8.d, L.w18.d, L.w38.d, L.w28.d};
+                     L.wqkv8.q, L.wo8.q, L.w18.q, L.w38.q, L.w28.q, L.wqkv8.d, L.wo8.d, L.w18.d, L.w38.d, L.w28.d,
+                     L.wqkvh, L.woh, L.w1h, L.w3h, L.w2h};
         }
         mega_layers_dev = mem.dmalloc<k::MegaLayerHost>(nl, false);
         LB_CUDA(cudaMemcpy(mega_layers_dev, ml.data(), nl * sizeof(k::MegaLayerHost), cudaMemcpyHostToDevice));
@@ -267,12 +313,15 @@ Context::~Context() {
     // buffers, events and the stream are released by `mem`
 }
 
-// MulMat of a weight matrix: F32 or Q8_0 planes, GEMV (N <= 8) or GEMM
-static void matmul(const float *W, const Q8Mat &W8, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
+// MulMat of a weight matrix: F32, Q8_0 planes or F16, GEMV (N <= 8) or GEMM
+static void matmul(const float *W, const Q8Mat &W8, const uint16_t *Wh, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
                    float *Y, uint32_t ldy, const float *res, cudaStream_t st) {
     if (W8.q) {
         if (N <= 8) k::gemv_q8(W8.q, W8.d, M, K, X, ldx, N, Y, ldy, res, st);
         else k::gemm_q8_auto(W8.q, W8.d, M, K, X, ldx, N, Y, ldy, res, st);
+    } else if (Wh) {
+        if (N <= 8) k::gemv_f16(Wh, M, K, X, ldx, N, Y, ldy, res, st);
+        else k::gemm_f16_tc(Wh, M, K, X, ldx, N, Y, ldy, res, st);
     } else {
         if (N <= 8) k::gemv_f32(W, M, K, X, ldx, N, Y, ldy, res, st);
         else k::gemm_auto(W, M, K, X, ldx, N, Y, ldy, res, st);
@@ -309,6 +358,8 @@ void Context::forward(uint32_t n, bool tokens_indirect, bool all_rows, const flo
         mp.q_output = model->has_head() ? model->output8.q : nullptr;
         mp.d_output = model->has_head() ? model->output8.d : nullptr;
         mp.q8 = model->q8();
+        mp.f16 = model->f16();
+        mp.h_output = model->has_head() ? model->outputh : nullptr;
         mp.x = x; mp.y = y; mp.qkv = qkv; mp.attn = attn; mp.act = act; mp.logits = logits;
         const uint32_t hd = hp.head_dim();
         mp.part_o = attn_scratch;
@@ -340,21 +391,22 @@ void Context::forward(uint32_t n, bool tokens_indirect, bool all_rows, const flo
         const Layer &L = model->layers[li];
         float *Kc = kv_k + li * (size_t)ctx_size * d, *Vc = kv_v + li * (size_t)ctx_size * d;
         k::rms_norm(x, L.attention_norm, cur, d, n, st);
-        matmul(L.wqkv, L.wqkv8, 3 * d, d, cur, d, n, qkv, 3 * d, nullptr, st);
+        matmul(L.wqkv, L.wqkv8, L.wqkvh, 3 * d, d, cur, d, n, qkv, 3 * d, nullptr, st);
         k::rope_qk_store(qkv, qkv + d, qkv + 2 * d, 3 * d, Kc, Vc, n, past_dev, d, H, st);
         if (n == 1) k::attention_decode(qkv, Kc, Vc, attn, past_dev, ctx_size, d, H, attn_scratch, st);
         else k::attention(qkv, 3 * d, Kc, Vc, attn, n, past_dev, ctx_size, d, H, st);
-        matmul(L.wo, L.wo8, d, d, attn, d, n, y, d, x, st);
+        matmul(L.wo, L.wo8, L.woh, d, d, attn, d, n, y, d, x, st);
         k::rms_norm(y, L.ffn_norm, cur, d, n, st);
         if (n <= 8) {
             if (model->q8()) k::gemv_q8_swiglu(L.w18.q, L.w18.d, L.w38.q, L.w38.d, ff, d, cur, d, n, act, ff, st);
+            else if (model->f16()) k::gemv_f16_swiglu(L.w1h, L.w3h, ff, d, cur, d, n, act, ff, st);
             else k::gemv_f32_swiglu(L.w1, L.w3, ff, d, cur, d, n, act, ff, st);
         } else {
-            matmul(L.w3, L.w38, ff, d, cur, d, n, up, ff, nullptr, st);
-            matmul(L.w1, L.w18, ff, d, cur, d, n, act, ff, nullptr, st);
+            matmul(L.w3, L.w38, L.w3h, ff, d, cur, d, n, up, ff, nullptr, st);
+            matmul(L.w1, L.w18, L.w1h, ff, d, cur, d, n, act, ff, nullptr, st);
             k::swiglu(act, up, act, (size_t)n * ff, st);
         }
-        matmul(L.w2, L.w28, d, ff, act, ff, n, x, d, y, st);
+        matmul(L.w2, L.w28, L.w2h, d, ff, act, ff, n, x, d, y, st);
     }
     if (hidden_out && hidden_out != x)
         LB_CUDA(cudaMemcpyAsync(hidden_out, x, (size_t)n * d * sizeof(float), cudaMemcpyDeviceToDevice, st));
@@ -362,11 +414,11 @@ void Context::forward(uint32_t n, bool tokens_indirect, bool all_rows, const flo
         if (all_rows) {
             if (!all_logits) all_logits = mem.dmalloc<float>((size_t)max_batch * V, false);
             k::rms_norm(x, model->norm, cur, d, n, st);
-            matmul(model->output, model->output8, V, d, cur, d, n, all_logits, V, nullptr, st);
+            matmul(model->output, model->output8, model->outputh, V, d, cur, d, n, all_logits, V, nullptr, st);
         } else {
             // only row n-1 is ever read (llama.go:394-401); the reference computes all n (:384)
             k::rms_norm(x + (size_t)(n - 1) * d, model->norm, cur, d, 1, st);
-            matmul(model->output, model->output8, V, d, cur, d, 1, logits, V, nullptr, st);
+            matmul(model->output, model->output8, model->outputh, V, d, cur, d, 1, logits, V, nullptr, st);
         }
     }
 }
@@ -656,6 +708,7 @@ float Context::bench_kernel(int which, uint32_t iters, uint32_t past, uint64_t *
     const uint32_t d = hp.dim, ff = hp.ff(), V = hp.vocab, H = hp.heads;
     const size_t nl = model->layers.size();
     LB_CHECK(iters >= 1 && nl >= 1, "bench_kernel : nothing to run");
+    LB_CHECK(model->f32() || model->q8(), "bench_kernel : F32 and Q8_0 weights only");
     LB_CHECK(past < ctx_size, "bench_kernel : past exceeds the context");
     LB_CUDA(cudaSetDevice(model->device));
     state_host[0] = past; state_host[1] = 0;
@@ -665,17 +718,17 @@ float Context::bench_kernel(int which, uint32_t iters, uint32_t past, uint64_t *
         const Layer &L = model->layers[i % nl];
         float *Kc = kv_k + (i % nl) * (size_t)ctx_size * d, *Vc = kv_v + (i % nl) * (size_t)ctx_size * d;
         switch (which) {
-            case 0: matmul(L.wqkv, L.wqkv8, 3 * d, d, cur, d, 1, qkv, 3 * d, nullptr, stream); break;
-            case 1: matmul(L.wo, L.wo8, d, d, attn, d, 1, y, d, x, stream); break;
+            case 0: matmul(L.wqkv, L.wqkv8, nullptr, 3 * d, d, cur, d, 1, qkv, 3 * d, nullptr, stream); break;
+            case 1: matmul(L.wo, L.wo8, nullptr, d, d, attn, d, 1, y, d, x, stream); break;
             case 2: if (model->q8()) k::gemv_q8_swiglu(L.w18.q, L.w18.d, L.w38.q, L.w38.d, ff, d, cur, d, 1, act, ff, stream);
                     else k::gemv_f32_swiglu(L.w1, L.w3, ff, d, cur, d, 1, act, ff, stream);
                     break;
-            case 3: matmul(L.w2, L.w28, d, ff, act, ff, 1, up, d, y, stream); break;
+            case 3: matmul(L.w2, L.w28, nullptr, d, ff, act, ff, 1, up, d, y, stream); break;
             case 4: LB_CHECK(model->has_head(), "no lm_head on this stage");
-                    matmul(model->output, model->output8, V, d, cur, d, 1, logits, V, nullptr, stream); break;
+                    matmul(model->output, model->output8, nullptr, V, d, cur, d, 1, logits, V, nullptr, stream); break;
             case 5: k::attention_decode(qkv, Kc, Vc, attn, state_dev, ctx_size, d, H, attn_scratch, stream); break;
             case 6: k::rms_norm(x, L.attention_norm, cur, d, 1, stream); break;
-            case 7: matmul(L.w1, L.w18, ff, d, cur, d, pf_n, act, ff, nullptr, stream); break;  // prefill GEMM
+            case 7: matmul(L.w1, L.w18, nullptr, ff, d, cur, d, pf_n, act, ff, nullptr, stream); break;  // prefill GEMM
             default: LB_CHECK(false, "bench_kernel : unknown kernel id");
         }
     };
@@ -740,7 +793,7 @@ void Context::eval_graph(const uint32_t *tokens, uint32_t N, uint32_t pastCount,
     using namespace ml;
     const HParams &hp = model->hp;
     LB_CHECK(model->has_embedding() && model->has_head(), "eval_graph : needs a single-stage model");
-    LB_CHECK(!model->q8(), "eval_graph : the pkg/ml op API is FP32 only (like the reference)");
+    LB_CHECK(model->f32(), "eval_graph : the pkg/ml op API is FP32 only (like the reference)");
     LB_CHECK(N >= 1 && (uint64_t)pastCount + N <= ctx_size, "Eval : pastCount + N exceeds the context size");
     LB_CUDA(cudaSetDevice(model->device));
     const uint32_t embdSize = hp.dim, layersCount = hp.layers, ctxSize = ctx_size, headsCount = hp.heads;

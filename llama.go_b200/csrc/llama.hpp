@@ -35,6 +35,7 @@ struct Layer {  // llama.go:128-146; wq|wk|wv are stored as one [3*dim][dim] mat
     float *ffn_norm = nullptr;
     float *w1 = nullptr, *w2 = nullptr, *w3 = nullptr;
     Q8Mat wqkv8, wo8, w18, w28, w38;  // used instead of the float matrices when weight_type == Q8_0
+    uint16_t *wqkvh = nullptr, *woh = nullptr, *w1h = nullptr, *w2h = nullptr, *w3h = nullptr;  // IEEE binary16 (weight_type == F16)
 };
 
 // llama.Model (llama.go:181-193) for one pipeline stage: layers [layer_begin, layer_end).
@@ -54,10 +55,15 @@ struct Model {
     int8_t *qslab = nullptr;  // Q8_0: int8 plane of every MulMat matrix of the stage
     float *dslab = nullptr;   //       and the per-block scales
     uint8_t *tmslab = nullptr;   // the same matrices as tile-major decode planes (ring megakernel)
+    uint16_t *hslab = nullptr;   // F16: every MulMat matrix of the stage as IEEE binary16, row-major
+    uint16_t *outputh = nullptr;
+    unsigned *f16_overflow = nullptr;  // F16: set by the device rounding when a finite value rounds to +-inf
     std::vector<Layer> layers;  // index = global layer - layer_begin
+    bool f32() const { return weight_type == 0; }
+    bool f16() const { return weight_type == 1; }
     bool q8() const { return weight_type == 16; }
 
-    struct Entry { float *ptr; size_t nelem; uint64_t tid; float mean, sigma; Q8Mat q8; uint32_t cols = 0; };
+    struct Entry { float *ptr; size_t nelem; uint64_t tid; float mean, sigma; Q8Mat q8; uint32_t cols = 0; uint16_t *h = nullptr; };
     std::map<std::string, Entry> tensors;  // ggjt names (llama.go:826-861) owned by this stage
 
     Model(const HParams &hp, int device, uint32_t lb, uint32_t le, int weight_type);
@@ -68,6 +74,8 @@ struct Model {
     void get_tensor(const std::string &name, float *host, size_t nelem);
     void init_random(uint64_t seed);
     uint64_t weight_bytes_per_token() const;
+    // n FP32 values on the device -> binary16 at dst, round to nearest even; a finite value that rounds to +-inf is an error
+    void round_to_f16(const float *src, uint16_t *dst, size_t n, const std::string &name, cudaStream_t st);
 };
 
 // llama.Context (llama.go:83-113): FP32 KV cache in HBM + activations + stream + decode graph.

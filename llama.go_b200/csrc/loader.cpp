@@ -7,7 +7,8 @@
 // names abort (llama.go:906-910).  Differences in mechanism, not in result: the file is memory-mapped
 // and every tensor goes host -> HBM through two pinned staging buffers on a copy stream (the
 // reference reads F16 tensors with one 2-byte Read per element); with LB_TYPE_Q8_0 the MulMat
-// matrices are block-quantised on the device as they arrive.
+// matrices are block-quantised on the device as they arrive; with LB_TYPE_F16 they keep F16 data byte
+// for byte (streamed straight into place) and F32 data is rounded to nearest even on the device.
 #include <fcntl.h>
 #include <string.h>
 #include <sys/mman.h>
@@ -127,13 +128,14 @@ LoadedModel load_ggjt(const std::string &path, int device, uint32_t layer_begin,
             if (it == m.tensors.end()) continue;  // another pipeline stage's tensor
             const Model::Entry &e = it->second;
             LB_CHECK(e.nelem == nelem, "tensor '" + name + "' has the wrong size");
-            const bool direct = dtype == 0 && !e.q8.q;  // FP32 tensor stored as FP32: stream straight into place
+            // stored as it is in the file (FP32 into FP32, F16 into an F16 matrix): stream straight into place
+            const bool direct = e.h ? dtype == 1 : (dtype == 0 && !e.q8.q);
             if (!direct && dev_tmp_bytes < nbytes + nelem * 4) {
                 if (dev_tmp) { LB_CUDA(cudaStreamSynchronize(cs)); cudaFree(dev_tmp); dev_tmp = nullptr; }
                 dev_tmp_bytes = nbytes + nelem * 4;
                 LB_CUDA(cudaMalloc(&dev_tmp, dev_tmp_bytes));
             }
-            uint8_t *raw_dst = direct ? reinterpret_cast<uint8_t *>(e.ptr) : static_cast<uint8_t *>(dev_tmp);
+            uint8_t *raw_dst = !direct ? static_cast<uint8_t *>(dev_tmp) : e.h ? reinterpret_cast<uint8_t *>(e.h) : reinterpret_cast<uint8_t *>(e.ptr);
             for (size_t o = 0; o < nbytes; o += CHUNK) {
                 const size_t c = nbytes - o < CHUNK ? nbytes - o : CHUNK;
                 LB_CUDA(cudaEventSynchronize(ev[slot]));  // staging buffer free again
@@ -142,7 +144,9 @@ LoadedModel load_ggjt(const std::string &path, int device, uint32_t layer_begin,
                 LB_CUDA(cudaEventRecord(ev[slot], cs));
                 slot ^= 1;
             }
-            if (!direct) {
+            if (!direct && e.h) {
+                m.round_to_f16(static_cast<const float *>(dev_tmp), e.h, nelem, name, cs);   // synchronises cs: dev_tmp is reused
+            } else if (!direct) {
                 float *f32 = e.q8.q ? reinterpret_cast<float *>(static_cast<uint8_t *>(dev_tmp) + nbytes) : e.ptr;
                 const float *quant_src = f32;
                 if (dtype == 1) k::f16_to_f32(static_cast<const uint16_t *>(dev_tmp), f32, nelem, cs);

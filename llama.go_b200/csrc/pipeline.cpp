@@ -124,6 +124,7 @@ void p2p_import(llama::Context **ctxs, uint32_t n_seq, const void *down, const v
     LB_CHECK(ctxs && n_seq >= 1, "p2p_import: nil argument");
     for (uint32_t s = 0; s < n_seq; s++) {
         llama::Context *c = ctxs[s];
+        LB_CHECK(!c->model->f16(), "p2p_import: the fused hand-off does not carry F16 weights (FP32 only)");
         LB_CHECK(c->p2p_flags != nullptr, "p2p_import: call p2p_export first");
         LB_CHECK(c->use_mega && !c->use_ring_q8, "p2p_import: the fused hand-off needs the FP32 decode megakernel (unsupported shape, Q8 weights or LB_NO_MEGA)");
         LB_CHECK(!c->stage_graph, "p2p_import: the stage graph is already captured");

@@ -49,9 +49,10 @@ PodBatch::PodBatch(const std::vector<Context *> &cs) : ctxs(cs) {
     // one persistent megakernel per step (kernels_mega_pods.cu) for FP32 weights and supported shapes;
     // LB_NO_MEGA_PODS=1 keeps the per-op B-column kernels
     // (TMA-ring variant kernels_ring_pods.cu when the shape allows, LB_NO_RING_PODS=1: the register-fed kernels_mega_pods.cu)
-    use_ring = getenv("LB_NO_MEGA_PODS") == nullptr && getenv("LB_NO_RING_PODS") == nullptr && !model->q8() &&
+    // (Q8_0 and F16 models keep the per-op B-column kernels)
+    use_ring = getenv("LB_NO_MEGA_PODS") == nullptr && getenv("LB_NO_RING_PODS") == nullptr && model->f32() &&
                k::decode_ring_pods_supported(hp.dim, hp.ff(), hp.heads, hp.vocab, ctx_size);
-    use_mega = use_ring || (getenv("LB_NO_MEGA_PODS") == nullptr && !model->q8() &&
+    use_mega = use_ring || (getenv("LB_NO_MEGA_PODS") == nullptr && model->f32() &&
                             k::decode_mega_pods_supported(hp.dim, hp.ff(), hp.heads, hp.vocab, ctx_size));
     if (use_mega) {
         const size_t nl = model->layers.size();
@@ -82,9 +83,10 @@ PodBatch::~PodBatch() {
     // buffers, events and the stream are released by `mem`
 }
 
-static void mm(const float *W, const Q8Mat &W8, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N, float *Y,
-               uint32_t ldy, const float *res, cudaStream_t st) {
+static void mm(const float *W, const Q8Mat &W8, const uint16_t *Wh, uint32_t M, uint32_t K, const float *X, uint32_t ldx, uint32_t N,
+               float *Y, uint32_t ldy, const float *res, cudaStream_t st) {
     if (W8.q) k::gemv_q8(W8.q, W8.d, M, K, X, ldx, N, Y, ldy, res, st);
+    else if (Wh) k::gemv_f16(Wh, M, K, X, ldx, N, Y, ldy, res, st);
     else k::gemv_f32(W, M, K, X, ldx, N, Y, ldy, res, st);
 }
 
@@ -119,17 +121,18 @@ void PodBatch::forward() {
         const Layer &L = model->layers[li];
         pp.layer_off = li * (size_t)ctx_size * d;
         k::rms_norm(x, L.attention_norm, cur, d, B, st);
-        mm(L.wqkv, L.wqkv8, 3 * d, d, cur, d, B, qkv, 3 * d, nullptr, st);
+        mm(L.wqkv, L.wqkv8, L.wqkvh, 3 * d, d, cur, d, B, qkv, 3 * d, nullptr, st);
         k::rope_qk_store_pods(qkv, qkv + d, qkv + 2 * d, 3 * d, B, pp, d, H, st);
         k::attention_decode_pods(qkv, attn, B, pp, ctx_size, d, H, attn_scratch, st);
-        mm(L.wo, L.wo8, d, d, attn, d, B, y, d, x, st);
+        mm(L.wo, L.wo8, L.woh, d, d, attn, d, B, y, d, x, st);
         k::rms_norm(y, L.ffn_norm, cur, d, B, st);
         if (model->q8()) k::gemv_q8_swiglu(L.w18.q, L.w18.d, L.w38.q, L.w38.d, ff, d, cur, d, B, act, ff, st);
+        else if (model->f16()) k::gemv_f16_swiglu(L.w1h, L.w3h, ff, d, cur, d, B, act, ff, st);
         else k::gemv_f32_swiglu(L.w1, L.w3, ff, d, cur, d, B, act, ff, st);
-        mm(L.w2, L.w28, d, ff, act, ff, B, x, d, y, st);
+        mm(L.w2, L.w28, L.w2h, d, ff, act, ff, B, x, d, y, st);
     }
     k::rms_norm(x, model->norm, cur, d, B, st);
-    mm(model->output, model->output8, V, d, cur, d, B, logits, V, nullptr, st);
+    mm(model->output, model->output8, model->outputh, V, d, cur, d, B, logits, V, nullptr, st);
     k::advance_pods(pasts_dev, state_dev, B, st);
 }
 

@@ -15,7 +15,7 @@ from ._capi import HParamsC, LlamaB200Error, check, check_ptr, lib  # noqa: F401
 
 _f32p = C.POINTER(C.c_float)
 _u32p = C.POINTER(C.c_uint32)
-LB_TYPE_F32, LB_TYPE_Q8_0 = 0, 16  # include/llamab200.h
+LB_TYPE_F32, LB_TYPE_F16, LB_TYPE_Q8_0 = 0, 1, 16  # include/llamab200.h
 
 
 class Model:

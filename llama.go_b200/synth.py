@@ -183,6 +183,19 @@ def is_q8_matrix(name: str) -> bool:
     return name.endswith(Q8_MATRICES)
 
 
+# --------------------------------------------------------------------------- F16 weights
+def round_f16(w: np.ndarray) -> np.ndarray:
+    """What an LB_TYPE_F16 model holds for an FP32 matrix, widened back: binary16 round-to-nearest-even."""
+    return np.asarray(w, np.float32).astype(np.float16).astype(np.float32)
+
+
+def synth_model_f16(seed: int, hp: HParams):
+    """synth_model() as an LB_TYPE_F16 model holds it: the MulMat matrices (is_q8_matrix) rounded to binary16 and
+    widened back, norm vectors and the embedding table untouched.  The oracle's input for F16 models."""
+    for name, arr in synth_model(seed, hp):
+        yield name, round_f16(arr) if is_q8_matrix(name) else arr
+
+
 # --------------------------------------------------------------------------- vocab
 def byte_vocab(vocab_size: int):
     """Synthetic vocab under which the reference tokenizer (pkg/ml/ml.go:2761-2848) maps every

@@ -12,6 +12,11 @@ Runs ONLY in the build container (needs /root/reference via oracle/_ref):
 
 Usage: python tools/gen_golden.py [case ...]            # refbin_<case>.json, logits_<case>.npz
        python tools/gen_golden.py swap|threads2|vdot    # refbin_swap.json, refbin_threads2.json, vdot_ref.npz
+       python tools/gen_golden.py f16                   # refbin_f16.json
+
+refbin_f16.json pins F16 input (the format LLaMA ggjt checkpoints most often come in): the reference binary's scalar and
+--avx greedy streams on the tiny and hd128 models written with F16 matrices, the SHA-256 of those files, and the oracle's
+tokens on the widened weights.  LB_TYPE_F16 models (the MulMat matrices held as binary16) are checked against it on the GPU.
 """
 import hashlib
 import json
@@ -94,7 +99,7 @@ def main():
     print("done")
 
 
-if __name__ == "__main__" and not {"swap", "threads2", "vdot"} & set(sys.argv[1:]):
+if __name__ == "__main__" and not {"swap", "threads2", "vdot", "f16"} & set(sys.argv[1:]):
     main()
 
 
@@ -180,3 +185,58 @@ if __name__ == "__main__" and "threads2" in sys.argv[1:]:
     gen_threads2()
 if __name__ == "__main__" and "vdot" in sys.argv[1:]:
     gen_vdot()
+
+
+def gen_f16():
+    """refbin_f16.json — the reference binary (scalar, and --avx at 4 threads) on the ggjt files synth.write_ggjt(f16=True) makes for
+    the tiny and hd128 cases (every 2-D tensor stored as F16, which the reference widens at load): the files' SHA-256, the printed
+    streams, and the oracle's stream on the widened weights.  The F16 rounding must move the logits measurably against the FP32
+    fixtures (logits_<case>.npz), or the pin could not tell F16 input apart from FP32."""
+    O.build()
+    out = {}
+    for name in ("tiny", "hd128"):
+        with open(os.path.join(ROOT, "tests", "golden", f"refbin_{name}.json")) as f:
+            base = json.load(f)
+        g = np.load(os.path.join(ROOT, "tests", "golden", f"logits_{name}.npz"))
+        hp = synth.HParams(*base["hparams"])
+        vocab = synth.byte_vocab(hp.vocab)
+        ids = base["prompt_ids"]
+        rec = {k: base[k] for k in ("hparams", "seed", "prompt", "prompt_ids", "context", "predict")}
+        rec["runs"] = {}
+        with tempfile.TemporaryDirectory() as td:
+            path = os.path.join(td, "m.bin")
+            synth.write_ggjt(path, hp, synth.synth_model(base["seed"], hp), vocab, f16=True)
+            with open(path, "rb") as f:
+                rec["ggjt_sha256"] = hashlib.sha256(f.read()).hexdigest()
+            for mode, threads, avx in (("scalar", 1, False), ("avx", 4, True)):
+                r = refbin.run(path, base["prompt"], base["predict"], base["context"], threads, avx, port=18183)
+                rec["runs"][mode] = {"threads": threads, "text_hex": r["text"].hex(), "evals": len(r["eval_ms"])}
+            _, _, widened = synth.read_ggjt(path)
+        tensors = [(n, widened[n]) for n, *_ in synth.tensor_table(hp)]
+        for mode in ("scalar", "avx"):
+            O.set_dot_mode(mode == "avx")
+            try:
+                c = O.OracleContext(O.OracleModel(hp).load(tensors), base["context"])
+                toks, logits, margins = O.greedy_stream(c, ids, base["predict"], base["context"], return_logits=True)
+            finally:
+                O.set_dot_mode(False)
+            exp = refbin.expected_text(vocab, ids, toks)
+            assert refbin.same_stream(bytes.fromhex(rec["runs"][mode]["text_hex"]), exp), (name, mode)
+            if mode == "scalar":
+                rec["oracle_tokens"] = toks
+                rec["min_margin"] = min(margins)
+                shift = float(np.abs(logits[0] - g["step_logits"][0]).max() / np.abs(g["step_logits"][0]).max())
+            else:
+                assert toks == rec["oracle_tokens"], name
+        # a pin that cannot tell F16 from FP32 pins nothing: the rounding must move the prompt logits far beyond summation noise
+        assert shift > 1e-4, (name, shift)
+        rec["prompt_logit_shift_vs_f32"] = shift
+        rec["differs_from_f32_stream"] = rec["oracle_tokens"] != base["oracle_tokens"]
+        out[name] = rec
+        print(f"[{name}/f16] streams pinned, prompt logits moved {shift:.3e} (relative) by the F16 rounding")
+    with open(os.path.join(ROOT, "tests", "golden", "refbin_f16.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
+if __name__ == "__main__" and "f16" in sys.argv[1:]:
+    gen_f16()
