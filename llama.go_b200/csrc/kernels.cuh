@@ -122,7 +122,9 @@ void advance_state(uint32_t *state, uint32_t dp, uint32_t ds, cudaStream_t st, u
 struct MegaLayerHost {  // one per layer, array lives in device memory
     const float *attention_norm, *wqkv, *wo, *ffn_norm, *w1, *w3, *w2;
     float *Kc, *Vc;
-    const int8_t *q_wqkv, *q_wo, *q_w1, *q_w3, *q_w2;  // Q8_0 planes (nullptr for F32 models)
+    // Q8_0 planes (nullptr for F32 models).  No kernel reads them (kernels_ring_q8.cu streams RingQ8Layer); they keep the
+    // layout of this table, which the decode kernels' register allocation depends on.
+    const int8_t *q_wqkv, *q_wo, *q_w1, *q_w3, *q_w2;
     const float *d_wqkv, *d_wo, *d_w1, *d_w3, *d_w2;
     const uint16_t *h_wqkv, *h_wo, *h_w1, *h_w3, *h_w2;  // binary16 matrices (F16 models, TMA-ring kernel only)
 };
@@ -132,9 +134,6 @@ struct MegaParamsHost {
     const float *tok_embeddings;      // nullptr: residual comes in through x (pipeline stage > 0)
     const uint32_t *tokens, *state;   // device: token ids, {past, step}
     const float *final_norm, *output; // final_norm == nullptr: no lm_head on this stage
-    const int8_t *q_output = nullptr; // Q8_0 lm_head planes (experiment: Q8 megakernel)
-    const float *d_output = nullptr;
-    bool q8 = false;
     bool f16 = false;                 // F16 weights: the layers' h_* matrices and h_output (decode_ring only)
     const uint16_t *h_output = nullptr;
     float *x, *y, *qkv, *attn, *act, *logits;
@@ -153,7 +152,6 @@ struct MegaParamsHost {
     uint32_t *p2p_ack_out = nullptr;  // peer-mapped flags of the upstream context (its ack is [1])
 };
 bool decode_mega_supported(uint32_t dim, uint32_t ff, uint32_t heads);
-bool decode_mega_q8_supported(uint32_t dim, uint32_t ff, uint32_t heads, uint32_t vocab);
 uint32_t decode_mega_splits(uint32_t heads);
 void decode_mega(const MegaParamsHost &p, cudaStream_t st);
 

@@ -25,12 +25,14 @@
 // K > 5632 (w2: K = ff) does not fit the 176 KB activation stage: its K axis is walked in passes with the
 // next pass's columns arriving by cp.async behind the current pass's MMAs.
 // Numerics of everything else (RMSNorm f64 sums, f64 RoPE, f64 exp softmax terms, FP32 sequential-order
-// independent sums) are those of kernels_mega.cu / kernels_attn.cu.
+// independent sums) are those of kernels_mega.cu / kernels_attn.cu.  The attention phase (attention_pods), merge
+// statistics, grid barrier and PTX wrappers are shared with the other decode kernels (megakernel.cuh).
 #include <cooperative_groups.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "megakernel.cuh"
 
 namespace lb {
 namespace k {
@@ -38,7 +40,6 @@ namespace {
 
 constexpr int PM_WARPS = 12;   // 384 threads -> 168 registers per thread: room for a 10-chunk weight ring per warp
 constexpr int PM_THREADS = PM_WARPS * 32;
-constexpr int PM_HALF = PM_THREADS / 2;
 constexpr int PM_MAXB = 8;
 #ifndef PM_U1
 #define PM_U1 10  // ring depth (chunks in flight per warp) of the one-matrix phases
@@ -52,44 +53,10 @@ constexpr uint32_t PM_PASS_CHUNKS = PM_XS_CHUNKS / 2;  // streamed phases: two b
 constexpr int PM_MAX_ITEMS = 2 * kNumSMs + 64;         // (pod, head, split) items whose statistics are merged
 constexpr int PM_MAX_TILES = 8;                        // 16-row tiles of a CTA in a streamed (multi-pass) phase
 
-__device__ __forceinline__ void csync() { asm volatile("bar.sync 1, %0;" ::"n"(PM_THREADS) : "memory"); }
-__device__ __forceinline__ void hsync(int half) { asm volatile("bar.sync %0, %1;" ::"r"(2 + half), "n"(PM_HALF) : "memory"); }
-__device__ __forceinline__ float4 ldcg4(const float *p) { return __ldcg(reinterpret_cast<const float4 *>(p)); }
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned &target, unsigned nctas) {
-    target += nctas;
-    csync();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(bar, 1u);
-        const long long t0 = clock64();
-        while (ld_acquire_u32(bar) < target) {
-            if (clock64() - t0 > 4000000000LL) __trap();  // never hang the GPU on a scheduling bug
-        }
-        __threadfence();
-    }
-    csync();
-}
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gsrc) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
-
-// D(16x8, f32) += A(16x8, tf32, row) * B(8x8, tf32, col)
-__device__ __forceinline__ void mma_tf32(float (&d)[4], float a0, float a1, float a2, float a3, float b0, float b1) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(__float_as_uint(a0)), "r"(__float_as_uint(a1)), "r"(__float_as_uint(a2)), "r"(__float_as_uint(a3)),
-          "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
-// v - trunc_tf32(v): exact in FP32 (the tensor core reads only the upper 19 bits of an operand register)
-__device__ __forceinline__ float tf32_lo(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
-__device__ __forceinline__ float4 tf32_lo4(float4 v) { return make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)); }
 
 using PodsLayer = MegaLayerHost;  // Kc/Vc unused here: every pod has its own cache (PodsParams::Kb/Vb + layer_off)
 struct PodsParams {
@@ -148,14 +115,14 @@ __device__ __forceinline__ void fill_norm(float4 *xs, const float *w, uint32_t K
     acc += __shfl_xor_sync(0xffffffffu, acc, 1);
     acc += __shfl_xor_sync(0xffffffffu, acc, 2);
     if (t == 0) sh.red[warp][pod] = acc;
-    csync();
+    csync<PM_THREADS>();
     if (threadIdx.x < PM_MAXB) {
         double s = 0.0;
 #pragma unroll
         for (int i = 0; i < PM_WARPS; i++) s += sh.red[i][threadIdx.x];
         sh.scale[threadIdx.x] = (float)(1.0 / sqrt(s / (double)K + 1e-5));
     }
-    csync();
+    csync<PM_THREADS>();
     const float sc = sh.scale[pod];
     for (uint32_t f = threadIdx.x; f < nf4; f += PM_THREADS) {
         const uint32_t kk = (f >> 5) * 16 + t * 4;
@@ -164,7 +131,7 @@ __device__ __forceinline__ void fill_norm(float4 *xs, const float *w, uint32_t K
         xs[f] = make_float4(__fmul_rn(ww.x, __fmul_rn(v.x, sc)), __fmul_rn(ww.y, __fmul_rn(v.y, sc)),
                             __fmul_rn(ww.z, __fmul_rn(v.z, sc)), __fmul_rn(ww.w, __fmul_rn(v.w, sc)));
     }
-    csync();
+    csync<PM_THREADS>();
 }
 
 // plain rows X[pod] = src + pod * ld (written earlier in this launch by other CTAs -> L2 loads)
@@ -175,36 +142,15 @@ __device__ __forceinline__ void fill_rows(float4 *xs, const float *src, uint32_t
         const uint32_t kk = (f >> 5) * 16 + t * 4;
         xs[f] = pod < (int)B ? ldcg4(src + (size_t)pod * ld + kk) : make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    csync();
+    csync<PM_THREADS>();
 }
 
 // merge of the attention splits straight into the stage (S > 1): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s),
 // w_s = expf(m_s - max_s m_s) — the same reassociation of the single-pass softmax as kernels_mega.cu.
 template <int HD>
 __device__ __forceinline__ void fill_merge(float4 *xs, const PodsParams &p, PodsShared &sh) {
-    const uint32_t S = p.splits, BH = p.B * p.heads, items = BH * S;
-    for (uint32_t i = threadIdx.x; i < items; i += PM_THREADS) {
-        const float2 ml = __ldcg(reinterpret_cast<const float2 *>(p.part_ml) + i);
-        sh.mrg_m[i] = ml.x;
-        sh.mrg_l[i] = ml.y;
-    }
-    csync();
-    for (uint32_t bh = threadIdx.x; bh < BH; bh += PM_THREADS) {
-        float M = -INFINITY;
-        for (uint32_t s = 0; s < S; s++) M = fmaxf(M, sh.mrg_m[bh * S + s]);
-        float Lsum = 0.f;
-        for (uint32_t s = 0; s < S; s++) {
-            const float l = sh.mrg_l[bh * S + s];
-            float wgt = 0.f;
-            if (l > 0.f) {
-                wgt = expf(__fsub_rn(sh.mrg_m[bh * S + s], M));
-                Lsum = fmaf(l, wgt, Lsum);
-            }
-            sh.mrg_w[bh * S + s] = wgt;
-        }
-        sh.mrg_inv[bh] = __fdiv_rn(1.0f, Lsum);
-    }
-    csync();
+    const uint32_t S = p.splits;
+    merge_stats<PM_THREADS>(p, p.B * p.heads, sh);
     const int lane = threadIdx.x & 31, pod = lane >> 2, t = lane & 3;
     const uint32_t nf4 = p.dim * 2;
     for (uint32_t f = threadIdx.x; f < nf4; f += PM_THREADS) {
@@ -226,7 +172,7 @@ __device__ __forceinline__ void fill_merge(float4 *xs, const PodsParams &p, Pods
         }
         xs[f] = o;
     }
-    csync();
+    csync<PM_THREADS>();
 }
 
 // one K pass of a streamed phase: chunks [c0, c1) of src rows -> buffer `dst` by cp.async (16 B per slot)
@@ -260,13 +206,13 @@ __device__ __forceinline__ void gemv_pods(const float *__restrict__ W1, const fl
     if (npass > 1) {  // first two passes on their way before anything else
         stream_pass(xs, xsrc, ldx, pass_c0(0), pass_c0(1), B);
         cp_async_wait_all();
-        csync();
+        csync<PM_THREADS>();
         stream_pass(xs + PM_XS_F4 / 2, xsrc, ldx, pass_c0(1), pass_c0(2), B);
     }
     if (NT == 0) {  // (cannot happen for M >= gridDim.x; keeps the barrier counts consistent if it does)
         for (uint32_t p = 0; p + 1 < npass; p++) {
             cp_async_wait_all();
-            csync();
+            csync<PM_THREADS>();
             if (p + 2 < npass) stream_pass(xs + (p & 1) * (PM_XS_F4 / 2), xsrc, ldx, pass_c0(p + 2), pass_c0(p + 3), B);
         }
         return;
@@ -367,7 +313,7 @@ __device__ __forceinline__ void gemv_pods(const float *__restrict__ W1, const fl
                         for (int i = 0; i < 4; i++) hh[m][i] = lh[m][i] = hl[m][i] = 0.f;
                     }
                     if (npass > 1 && last_tile_of_pass && !last_pass) cp_async_wait_all();  // next pass's columns (this thread's share)
-                    csync();
+                    csync<PM_THREADS>();
                     if (threadIdx.x < 128) {
                         const uint32_t row = r_begin + tj * 16 + (threadIdx.x >> 3), pod = threadIdx.x & 7;
                         float s1 = 0.f, s3 = 0.f;
@@ -388,7 +334,7 @@ __device__ __forceinline__ void gemv_pods(const float *__restrict__ W1, const fl
                             out[(size_t)pod * ldo + row] = v;
                         }
                     }
-                    if (NM == 2) csync();   // single-buffered partials in the two-matrix phase
+                    if (NM == 2) csync<PM_THREADS>();   // single-buffered partials in the two-matrix phase
                     else buf ^= 1;
                     if (npass > 1 && last_tile_of_pass && tp + 2 < npass)  // buffer (tp & 1) is free now: stream pass tp + 2 into it
                         stream_pass(xs + (tp & 1) * (PM_XS_F4 / 2), xsrc, ldx, pass_c0(tp + 2), pass_c0(tp + 3), B);
@@ -402,140 +348,6 @@ __device__ __forceinline__ void gemv_pods(const float *__restrict__ W1, const fl
                 }
             }
         }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// attention phase: items (pod, head, split); two items run concurrently per CTA (one per half, 8 warps each).
-// Same numerics as kernels_mega.cu::attention_phase.  With S == 1 the normalised output goes straight to
-// p.attn[pod][h*HD..]; with S > 1 the split partials are merged by fill_merge in the wo phase.
-// ---------------------------------------------------------------------------------------------------------
-template <int HD>
-__device__ __forceinline__ void attention_pods(const PodsParams &p, size_t layer_off, PodsShared &sh, float *scores_all) {
-    constexpr int LANES = HD / 4;
-    constexpr int HW = PM_WARPS / 2;
-    constexpr int KG = PM_HALF / LANES;
-    constexpr int AU = 8;
-    const int half = threadIdx.x / PM_HALF, ht = threadIdx.x % PM_HALF;
-    const int hwarp = ht >> 5, lane = threadIdx.x & 31;
-    const uint32_t dim = p.dim, S = p.splits;
-    const float scale = (float)(1.0 / sqrt((double)HD));  // f32(1/sqrt(dim/heads)), llama.go:306
-    const uint32_t items = p.B * p.heads * S;
-    float *scores = scores_all + (size_t)half * p.chunk_cap;
-    float4 *pv = sh.pv + half * PM_HALF;
-    const uint32_t kg = ht / LANES, dl = ht % LANES;
-    for (uint32_t item = blockIdx.x * 2 + half; item < items; item += gridDim.x * 2) {
-        const uint32_t sp = item % S, bh = item / S, h = bh % p.heads, b = bh / p.heads;
-        const uint32_t past = p.pasts[b], Tn = past + 1;
-        const uint32_t chunk = min((Tn + S - 1) / S, p.chunk_cap);
-        const uint32_t t0 = min(sp * chunk, Tn), t1 = min(t0 + chunk, Tn), nk = t1 - t0;
-        float *Kh = p.Kb[b] + layer_off + (size_t)h * HD;
-        float *Vh = p.Vb[b] + layer_off + (size_t)h * HD;
-        const float *qkv = p.qkv + (size_t)b * 3 * dim;
-        float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (lane < LANES) {
-            const float4 qr = ldcg4(qkv + (size_t)h * HD + lane * 4);
-            const double c0 = sh.rope_cs[b][lane * 2][0], s0 = sh.rope_cs[b][lane * 2][1];
-            const double c1 = sh.rope_cs[b][lane * 2 + 1][0], s1 = sh.rope_cs[b][lane * 2 + 1][1];
-            qv.x = (float)(__dsub_rn(__dmul_rn((double)qr.x, c0), __dmul_rn((double)qr.y, s0)));
-            qv.y = (float)(__dadd_rn(__dmul_rn((double)qr.x, s0), __dmul_rn((double)qr.y, c0)));
-            qv.z = (float)(__dsub_rn(__dmul_rn((double)qr.z, c1), __dmul_rn((double)qr.w, s1)));
-            qv.w = (float)(__dadd_rn(__dmul_rn((double)qr.z, s1), __dmul_rn((double)qr.w, c1)));
-            if (hwarp == 0 && past >= t0 && past < t1) {  // the item that owns position `past` stores the new K (rotated) and V rows
-                const float4 kr = ldcg4(qkv + dim + (size_t)h * HD + lane * 4);
-                float4 ko;
-                ko.x = (float)(__dsub_rn(__dmul_rn((double)kr.x, c0), __dmul_rn((double)kr.y, s0)));
-                ko.y = (float)(__dadd_rn(__dmul_rn((double)kr.x, s0), __dmul_rn((double)kr.y, c0)));
-                ko.z = (float)(__dsub_rn(__dmul_rn((double)kr.z, c1), __dmul_rn((double)kr.w, s1)));
-                ko.w = (float)(__dadd_rn(__dmul_rn((double)kr.z, s1), __dmul_rn((double)kr.w, c1)));
-                *reinterpret_cast<float4 *>(Kh + (size_t)past * dim + lane * 4) = ko;
-                *reinterpret_cast<float4 *>(Vh + (size_t)past * dim + lane * 4) = ldcg4(qkv + 2 * dim + (size_t)h * HD + lane * 4);
-            }
-        }
-        hsync(half);
-        for (uint32_t i = hwarp; i < nk; i += HW * AU) {
-            float4 kk[AU];
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                kk[u] = (ii < nk && lane < LANES) ? ldcg4(Kh + (size_t)(t0 + ii) * dim + lane * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                float dd = kk[u].x * qv.x;
-                dd = fmaf(kk[u].y, qv.y, dd); dd = fmaf(kk[u].z, qv.z, dd); dd = fmaf(kk[u].w, qv.w, dd);
-                dd = warp_sum(dd);
-                if (lane == 0 && ii < nk) scores[ii] = __fmul_rn(dd, scale);
-            }
-        }
-        float4 vf[AU];
-#pragma unroll
-        for (int u = 0; u < AU; u++) {
-            const uint32_t key = kg + u * KG;
-            vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        hsync(half);
-        float m = -INFINITY;
-        for (uint32_t i = ht; i < nk; i += PM_HALF) m = fmaxf(m, scores[i]);
-        m = warp_max(m);
-        if (lane == 0) sh.fred[half][hwarp] = m;
-        hsync(half);
-        if (ht == 0) {
-            float tt = sh.fred[half][0];
-            for (int i = 1; i < HW; i++) tt = fmaxf(tt, sh.fred[half][i]);
-            sh.hbcast[half] = tt;
-        }
-        hsync(half);
-        m = sh.hbcast[half];
-        float l = 0.f;
-        for (uint32_t i = ht; i < nk; i += PM_HALF) {
-            float e = (float)exp((double)__fsub_rn(scores[i], m));
-            scores[i] = e;
-            l += e;
-        }
-        l = warp_sum(l);
-        hsync(half);
-        if (lane == 0) sh.fred[half][hwarp] = l;
-        hsync(half);
-        if (ht == 0) {
-            float tt = 0.f;
-            for (int i = 0; i < HW; i++) tt += sh.fred[half][i];
-            sh.hbcast[half] = tt;
-            if (S > 1) {
-                p.part_ml[((size_t)bh * S + sp) * 2 + 0] = m;
-                p.part_ml[((size_t)bh * S + sp) * 2 + 1] = tt;
-            }
-        }
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (uint32_t base = 0; base < nk; base += KG * AU) {
-            if (base) {
-#pragma unroll
-                for (int u = 0; u < AU; u++) {
-                    const uint32_t key = base + kg + u * KG;
-                    vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t key = base + kg + u * KG;
-                if (key < nk) {
-                    const float sc = scores[key];
-                    acc.x = fmaf(vf[u].x, sc, acc.x); acc.y = fmaf(vf[u].y, sc, acc.y);
-                    acc.z = fmaf(vf[u].z, sc, acc.z); acc.w = fmaf(vf[u].w, sc, acc.w);
-                }
-            }
-        }
-        pv[ht] = acc;
-        hsync(half);  // also publishes hbcast = l
-        if (ht < HD) {
-            const float *pvf = reinterpret_cast<const float *>(pv);
-            float r = 0.f;
-            for (int i = 0; i < KG; i++) r += pvf[i * HD + ht];
-            if (S > 1) p.part_o[((size_t)bh * S + sp) * HD + ht] = r;
-            else p.attn[(size_t)b * dim + (size_t)h * HD + ht] = __fmul_rn(r, __fdiv_rn(1.0f, sh.hbcast[half]));  // p = e * f32(1/sum), ml.go:2493-2499
-        }
-        hsync(half);
     }
 }
 
@@ -565,7 +377,7 @@ __global__ void __launch_bounds__(PM_THREADS, 1) decode_mega_pods_kernel(const P
     if (threadIdx.x < PM_MAXB)
         sh.xrow[threadIdx.x] = threadIdx.x < B ? p.tok_embeddings + (size_t)p.tokens[(size_t)threadIdx.x * p.tok_stride + p.state[1]] * dim
                                                  : nullptr;  // GetRows, llama.go:244
-    csync();
+    csync<PM_THREADS>();
     const uint32_t np_ff = (ff / 16 + PM_PASS_CHUNKS - 1) / PM_PASS_CHUNKS;  // K passes of the w2 phase
     uint32_t r0, r1;
     for (uint32_t li = 0; li < p.n_layers; li++) {
@@ -575,23 +387,23 @@ __global__ void __launch_bounds__(PM_THREADS, 1) decode_mega_pods_kernel(const P
         fill_norm(xs, L.attention_norm, dim, B, sh);
         cta_rows(3 * dim, r0, r1);
         gemv_pods<1, PM_U1, 0>(L.wqkv, nullptr, dim, r0, r1, 1, nullptr, 0, p.qkv, 3 * dim, nullptr, 0, B, xs, sh);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<PM_THREADS>(p.barrier, target, gridDim.x);
         // ---- P2: RoPE, KV store, attention (llama.go:274-333)
-        attention_pods<HD>(p, layer_off, sh, scores);
-        grid_barrier(p.barrier, target, gridDim.x);
+        attention_pods<HD, PM_THREADS>(p, layer_off, sh, scores);
+        grid_barrier<PM_THREADS>(p.barrier, target, gridDim.x);
         // ---- P3: wo + residual (llama.go:336-340)
         if (p.splits > 1) fill_merge<HD>(xs, p, sh);
         else fill_rows(xs, p.attn, dim, dim, B);
         cta_rows(dim, r0, r1);
         gemv_pods<1, PM_U1, 1>(L.wo, nullptr, dim, r0, r1, 1, nullptr, 0, p.y, dim, nullptr, 0, B, xs, sh);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<PM_THREADS>(p.barrier, target, gridDim.x);
         // ---- P4: rmsnorm * ffn_norm, silu(w1·)·(w3·) (llama.go:346-361)
         if (threadIdx.x < PM_MAXB) sh.xrow[threadIdx.x] = threadIdx.x < B ? p.y + (size_t)threadIdx.x * dim : nullptr;
-        csync();
+        csync<PM_THREADS>();
         fill_norm(xs, L.ffn_norm, dim, B, sh);
         cta_rows(ff, r0, r1);
         gemv_pods<2, PM_U2, 0>(L.w1, L.w3, dim, r0, r1, 1, nullptr, 0, p.act, ff, nullptr, 0, B, xs, sh);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<PM_THREADS>(p.barrier, target, gridDim.x);
         // ---- P5: w2 + residual (llama.go:363-366)
         cta_rows(dim, r0, r1);
         if (np_ff > 1) {
@@ -600,9 +412,9 @@ __global__ void __launch_bounds__(PM_THREADS, 1) decode_mega_pods_kernel(const P
             fill_rows(xs, p.act, ff, ff, B);
             gemv_pods<1, PM_U1, 1>(L.w2, nullptr, ff, r0, r1, 1, nullptr, 0, p.x, dim, p.y, dim, B, xs, sh);
         }
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<PM_THREADS>(p.barrier, target, gridDim.x);
         if (threadIdx.x < PM_MAXB) sh.xrow[threadIdx.x] = threadIdx.x < B ? p.x + (size_t)threadIdx.x * dim : nullptr;
-        csync();
+        csync<PM_THREADS>();
     }
     if (p.final_norm) {  // final norm + lm_head (llama.go:374-384)
         fill_norm(xs, p.final_norm, dim, B, sh);

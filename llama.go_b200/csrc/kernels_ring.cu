@@ -31,12 +31,14 @@
 // (8 KB, so twice as many slots fit in the ring), and each lane reads the same elements as in the FP32 ring — two LDS.64
 // instead of two LDS.128 — widens them exactly and issues the same FMAs in the same order: every product and partial sum
 // equals the FP32 ring's on the widened weights, so the logits are bit-identical to an FP32 model holding those weights.
+// The attention phase, grid barrier and PTX wrappers are shared with the other decode kernels (megakernel.cuh).
 #include <cooperative_groups.h>
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "megakernel.cuh"
 
 namespace lb {
 namespace k {
@@ -45,7 +47,6 @@ namespace {
 constexpr int RG_CWARPS = 16;                      // consumer warps
 constexpr int RG_CTHREADS = RG_CWARPS * 32;        // 512
 constexpr int RG_THREADS = RG_CTHREADS + 32;       // + the producer warp
-constexpr int RG_HALF = RG_CTHREADS / 2;
 constexpr uint32_t RG_SLOT_FLOATS = 4096;          // one slot = one row (or a K chunk of a longer row) of <= 4096 weights: ONE bulk copy
 template <typename WT> constexpr uint32_t RG_SLOT = RG_SLOT_FLOATS * sizeof(WT);   // 16 KB (FP32) / 8 KB (F16)
 template <typename WT> constexpr int RG_MAX_SLOTS = sizeof(WT) == 4 ? 13 : 26;
@@ -53,21 +54,15 @@ constexpr int RG_GROUP = 32;                       // rows whose K-slice partial
 constexpr int RG_MAX_PHASES = 4 * 160 + 1;        // MulMat phases of a launch: 4 per layer + lm_head
 constexpr int RG_MAX_ITEMS = 2 * kNumSMs;
 constexpr int RG_MAX_HEADS = 256;
+// failed mbarrier polls before a trap: ~8 s at ~60 ns per poll, longer than any legitimate wait for a peer stage (p2p_wait
+// traps after ~10 s)
+constexpr uint32_t RG_MAX_SPINS = 1u << 27;
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ccsync() { asm volatile("bar.sync 1, %0;" ::"n"(RG_CTHREADS) : "memory"); }   // consumers only
-__device__ __forceinline__ void hsync(int half) { asm volatile("bar.sync %0, %1;" ::"r"(2 + half), "n"(RG_HALF) : "memory"); }
-__device__ __forceinline__ float4 ldcg4(const float *p) { return __ldcg(reinterpret_cast<const float4 *>(p)); }
-__device__ __forceinline__ float4 lds4(uint32_t addr) {
-    float4 r;
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(addr));
-    return r;
-}
 // 4 consecutive ring weights -> float4: FP32 (LDS.128) or binary16 (LDS.64, widened exactly)
 template <typename WT>
 __device__ __forceinline__ float4 lds_w4(uint32_t addr) {
     if constexpr (sizeof(WT) == 4) {
-        return lds4(addr);
+        return lds_f4(addr);
     } else {
         uint32_t a, b;
         asm volatile("ld.shared.v2.b32 {%0,%1}, [%2];" : "=r"(a), "=r"(b) : "r"(addr));
@@ -80,53 +75,6 @@ template <typename WT>
 __device__ __forceinline__ const WT *wsel(const float *f32, const uint16_t *f16) {
     if constexpr (sizeof(WT) == 4) return f32;
     else return reinterpret_cast<const WT *>(f16);
-}
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return done != 0;
-}
-// (try_wait suspends the thread in hardware for a bounded time; the spin counter only exists so that a pipeline bug traps
-//  after a few seconds instead of hanging the box — no clock read per iteration: ncu r02n counted 6.5 % CS2R instructions)
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, uint32_t backoff_ns = 0) {
-    if (mbar_try(bar, parity)) return;
-    uint32_t spins = 0;
-    while (!mbar_try(bar, parity)) {
-        if (backoff_ns) __nanosleep(backoff_ns);   // (consumers) polling burns issue slots and power: the decode step runs into the 1 kW cap
-        if (++spins > (1u << 27)) __trap();   // ~8 s at ~60 ns per failed poll: longer than any legitimate wait for a peer stage (p2p_wait traps after ~10 s)
-    }
-}
-struct RingPos {   // ring entry and mbarrier phase parity of the next slot (no division on the hot path: ncu r02n)
-    uint32_t slot, par;
-    __device__ __forceinline__ void next(uint32_t n_slots) {
-        if (++slot == n_slots) { slot = 0; par ^= 1u; }
-    }
-};
-// 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (TMA engine, no tensor map)
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
 }
 
 struct RingParams {
@@ -164,44 +112,6 @@ struct RingShared {
     float4 pv[RG_CTHREADS];
     float mrg_m[RG_MAX_ITEMS], mrg_l[RG_MAX_ITEMS], mrg_w[RG_MAX_ITEMS], mrg_inv[RG_MAX_HEADS];
 };
-
-__device__ __forceinline__ unsigned ld_acquire_sys_u32(const unsigned *p) {
-    unsigned v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_sys_u32(unsigned *p, unsigned v) {
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-// spin (one thread) until *flag >= want; traps after ~10 s instead of hanging the GPU if the peer stage died
-__device__ __forceinline__ void p2p_wait(const unsigned *flag, unsigned want) {
-    const long long t0 = clock64();
-    while (ld_acquire_sys_u32(flag) < want) {
-        if (clock64() - t0 > 20000000000LL) __trap();
-    }
-}
-
-// ---- grid barrier among the consumer threads of all CTAs (the producer warps never take part)
-__device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned &target, unsigned nctas, bool sys = false, unsigned long long *arrive = nullptr) {
-    target += nctas;
-    ccsync();
-    if (threadIdx.x == 0) {
-        if (arrive) {
-            unsigned long long t;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-            arrive[blockIdx.x] = t;
-        }
-        if (sys) __threadfence_system();   // this CTA's stores to the peer GPU are ordered before the hand-off flag
-        else __threadfence();
-        atomicAdd(bar, 1u);
-        const long long t0 = clock64();
-        while (ld_acquire_u32(bar) < target) {
-            if (clock64() - t0 > 4000000000LL) __trap();
-        }
-        __threadfence();
-    }
-    ccsync();
-}
 
 // A row of K floats is streamed as NCH = ceil(K / 4096) chunks of CH floats (a multiple of 64: every warp's 1/16 slice of
 // a chunk is whole float4s); the last chunk may be shorter.  Inside chunk c warp w owns floats [w * len_c / 16, (w + 1) * len_c / 16),
@@ -243,16 +153,16 @@ __device__ __forceinline__ void produce(const WT *W, const WT *W3, uint32_t K, u
             const uint32_t k0 = c * CH, len = min(CH, K - k0);
 #pragma unroll
             for (int m = 0; m < NM; m++) {
-                const uint32_t slot = q.slot, ph = q.par;
+                const uint32_t slot = q.slot, ph = q.phase;
                 const uint32_t fb = smem_u32(&sh.full[slot]);
                 if (pstat) {
                     unsigned long long ta, tb;
                     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ta));
-                    mbar_wait(smem_u32(&sh.empty[slot]), ph ^ 1);
+                    mbar_wait<RG_MAX_SPINS, true>(smem_u32(&sh.empty[slot]), ph ^ 1);
                     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(tb));
                     stall += tb - ta;
                 } else {
-                    mbar_wait(smem_u32(&sh.empty[slot]), ph ^ 1);   // all 16 warps have read slot q - n_slots
+                    mbar_wait<RG_MAX_SPINS, true>(smem_u32(&sh.empty[slot]), ph ^ 1);   // all 16 warps have read slot q - n_slots
                 }
                 *reinterpret_cast<volatile unsigned *>(&sh.jobrow[slot]) = row;
                 __threadfence_block();
@@ -302,7 +212,7 @@ __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], 
     int buf = 0;
     uint32_t ingroup = 0, j = 0;
     auto combine = [&](uint32_t n) {
-        ccsync();
+        csync<RG_CTHREADS>();
         if (threadIdx.x < n) {
             float s1 = 0.f, s3 = 0.f;
 #pragma unroll
@@ -321,7 +231,7 @@ __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], 
             //  r02r, logits 6e-3 off with the fence in the grid barrier only)
             if (peer_out) __threadfence_system();
         }
-        buf ^= 1;   // the other buffer is written next; this one is reused only after the next ccsync
+        buf ^= 1;   // the other buffer is written next; this one is reused only after the next csync
     };
     while (true) {
         // job j's first slot — or the end of the phase (the producer publishes the job count before it installs anything
@@ -331,12 +241,12 @@ __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], 
             uint32_t spins = 0;
             bool over = false;
             while (true) {
-                const bool got = mbar_try(fb, q.par);
+                const bool got = mbar_try(fb, q.phase);
                 const unsigned dj = *reinterpret_cast<volatile unsigned short *>(&sh.done_jobs[phidx]);
                 if (dj != 0xFFFFu && j >= dj) { over = true; break; }
                 if (got) break;
                 if (spin_ns) __nanosleep(spin_ns);
-                if (++spins > (1u << 27)) __trap();   // ~8 s at ~60 ns per failed poll: longer than any legitimate wait for a peer stage (p2p_wait traps after ~10 s)
+                if (++spins > RG_MAX_SPINS) __trap();
             }
             if (over) break;
         }
@@ -351,7 +261,7 @@ __device__ __forceinline__ void consume(uint32_t K, const float4 (&xs)[NCH][2], 
 #pragma unroll
             for (int m = 0; m < NM; m++) {
                 const uint32_t slot = q.slot;
-                if (c | m) mbar_wait(smem_u32(&sh.full[slot]), q.par, spin_ns);
+                if (c | m) mbar_wait<RG_MAX_SPINS, true>(smem_u32(&sh.full[slot]), q.phase, spin_ns);
                 const uint32_t base = ring_base + slot * RG_SLOT<WT> + ((uint32_t)warp * sl16 + (uint32_t)lane * 4) * (uint32_t)sizeof(WT);
                 const float4 wa = v0 ? lds_w4<WT>(base) : make_float4(0.f, 0.f, 0.f, 0.f);
                 const float4 wb = v1 ? lds_w4<WT>(base + 128 * (uint32_t)sizeof(WT)) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -414,7 +324,7 @@ __device__ __forceinline__ void fill_norm(float4 (&xs)[NCH][2], const float *x, 
         }
     acc = warp_sum(acc);
     if (lane == 0) sh.red[warp] = acc;
-    ccsync();
+    csync<RG_CTHREADS>();
     double t = 0.0;
 #pragma unroll
     for (int i = 0; i < RG_CWARPS; i++) t += sh.red[i];
@@ -425,7 +335,7 @@ __device__ __forceinline__ void fill_norm(float4 (&xs)[NCH][2], const float *x, 
         for (int v = 0; v < 2; v++)
             xs[c][v] = make_float4(__fmul_rn(ww[c][v].x, __fmul_rn(xs[c][v].x, sc)), __fmul_rn(ww[c][v].y, __fmul_rn(xs[c][v].y, sc)),
                                    __fmul_rn(ww[c][v].z, __fmul_rn(xs[c][v].z, sc)), __fmul_rn(ww[c][v].w, __fmul_rn(xs[c][v].w, sc)));
-    ccsync();   // sh.red may be rewritten
+    csync<RG_CTHREADS>();   // sh.red may be rewritten
 }
 template <int NCH>
 __device__ __forceinline__ void fill_plain(float4 (&xs)[NCH][2], const float *x, uint32_t K) {
@@ -438,7 +348,9 @@ __device__ __forceinline__ void fill_plain(float4 (&xs)[NCH][2], const float *x,
             xs[c][v] = e != 0xFFFFFFFFu ? ldcg4(x + e) : make_float4(0.f, 0.f, 0.f, 0.f);
         }
 }
-// merge of the attention splits (see kernels_mega.cu::merged_attention_slice): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s)
+// merge of the attention splits (see merge_stats, megakernel.cuh): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s).
+// The statistics are computed in line here, like the RoPE table in the kernel: through the shared functions this kernel's
+// machine code changes (register allocation), while the other decode kernels compile to the same code either way.
 template <int HD, int NCH, typename SH>
 __device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParams &p, SH &sh) {
     const uint32_t S = p.splits, items = p.heads * S, K = p.dim, CH = ring_chunk(K, NCH);
@@ -447,7 +359,7 @@ __device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParam
         sh.mrg_m[i] = ml.x;
         sh.mrg_l[i] = ml.y;
     }
-    ccsync();
+    csync<RG_CTHREADS>();
     for (uint32_t h = threadIdx.x; h < p.heads; h += RG_CTHREADS) {
         float M = -INFINITY;
         for (uint32_t s = 0; s < S; s++) M = fmaxf(M, sh.mrg_m[h * S + s]);
@@ -463,7 +375,7 @@ __device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParam
         }
         sh.mrg_inv[h] = __fdiv_rn(1.0f, Lsum);
     }
-    ccsync();
+    csync<RG_CTHREADS>();
     constexpr int MB = 12;   // splits per batch of loads (a per-split loop of L2 reads costs one round trip per split)
 #pragma unroll
     for (int c = 0; c < NCH; c++)
@@ -494,130 +406,6 @@ __device__ __forceinline__ void fill_merge(float4 (&xs)[NCH][2], const RingParam
         }
 }
 
-// ---- attention phase: identical to kernels_mega.cu::attention_phase (items (head, split), two per CTA at a time)
-template <int HD, typename SH>
-__device__ __forceinline__ void attention_phase(const RingParams &p, const MegaLayerHost &L, uint32_t past, SH &sh, float *scores_all) {
-    constexpr int LANES = HD / 4;
-    constexpr int HW = RG_CWARPS / 2;
-    constexpr int KG = RG_HALF / LANES;
-    constexpr int AU = 8;
-    const int half = threadIdx.x / RG_HALF, ht = threadIdx.x % RG_HALF;
-    const int hwarp = ht >> 5, lane = threadIdx.x & 31;
-    const uint32_t dim = p.dim, S = p.splits, Tn = past + 1;
-    const float scale = (float)(1.0 / sqrt((double)HD));  // f32(1/sqrt(dim/heads)), llama.go:306
-    const uint32_t chunk = min((Tn + S - 1) / S, p.chunk_cap);
-    const uint32_t items = p.heads * S;
-    float *scores = scores_all + (size_t)half * p.chunk_cap;
-    float4 *pv = sh.pv + half * RG_HALF;
-    const uint32_t kg = ht / LANES, dl = ht % LANES;
-    for (uint32_t item = blockIdx.x * 2 + half; item < items; item += gridDim.x * 2) {
-        const uint32_t h = item / S, sp = item % S;
-        const uint32_t t0 = min(sp * chunk, Tn), t1 = min(t0 + chunk, Tn), nk = t1 - t0;
-        float *Kh = L.Kc + (size_t)h * HD;
-        float *Vh = L.Vc + (size_t)h * HD;
-        float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (lane < LANES) {
-            const float4 qr = ldcg4(p.qkv + (size_t)h * HD + lane * 4);
-            const double c0 = sh.rope_cs[lane * 2][0], s0 = sh.rope_cs[lane * 2][1];
-            const double c1 = sh.rope_cs[lane * 2 + 1][0], s1 = sh.rope_cs[lane * 2 + 1][1];
-            qv.x = (float)(__dsub_rn(__dmul_rn((double)qr.x, c0), __dmul_rn((double)qr.y, s0)));
-            qv.y = (float)(__dadd_rn(__dmul_rn((double)qr.x, s0), __dmul_rn((double)qr.y, c0)));
-            qv.z = (float)(__dsub_rn(__dmul_rn((double)qr.z, c1), __dmul_rn((double)qr.w, s1)));
-            qv.w = (float)(__dadd_rn(__dmul_rn((double)qr.z, s1), __dmul_rn((double)qr.w, c1)));
-            if (hwarp == 0 && past >= t0 && past < t1) {
-                const float4 kr = ldcg4(p.qkv + dim + (size_t)h * HD + lane * 4);
-                float4 ko;
-                ko.x = (float)(__dsub_rn(__dmul_rn((double)kr.x, c0), __dmul_rn((double)kr.y, s0)));
-                ko.y = (float)(__dadd_rn(__dmul_rn((double)kr.x, s0), __dmul_rn((double)kr.y, c0)));
-                ko.z = (float)(__dsub_rn(__dmul_rn((double)kr.z, c1), __dmul_rn((double)kr.w, s1)));
-                ko.w = (float)(__dadd_rn(__dmul_rn((double)kr.z, s1), __dmul_rn((double)kr.w, c1)));
-                *reinterpret_cast<float4 *>(Kh + (size_t)past * dim + lane * 4) = ko;
-                *reinterpret_cast<float4 *>(Vh + (size_t)past * dim + lane * 4) = ldcg4(p.qkv + 2 * dim + (size_t)h * HD + lane * 4);
-            }
-        }
-        hsync(half);
-        for (uint32_t i = hwarp; i < nk; i += HW * AU) {
-            float4 kk[AU];
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                kk[u] = (ii < nk && lane < LANES) ? ldcg4(Kh + (size_t)(t0 + ii) * dim + lane * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                float dd = kk[u].x * qv.x;
-                dd = fmaf(kk[u].y, qv.y, dd); dd = fmaf(kk[u].z, qv.z, dd); dd = fmaf(kk[u].w, qv.w, dd);
-                dd = warp_sum(dd);
-                if (lane == 0 && ii < nk) scores[ii] = __fmul_rn(dd, scale);
-            }
-        }
-        float4 vf[AU];
-#pragma unroll
-        for (int u = 0; u < AU; u++) {
-            const uint32_t key = kg + u * KG;
-            vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        hsync(half);
-        float m = -INFINITY;
-        for (uint32_t i = ht; i < nk; i += RG_HALF) m = fmaxf(m, scores[i]);
-        m = warp_max(m);
-        if (lane == 0) sh.fred[half][hwarp] = m;
-        hsync(half);
-        if (ht == 0) {
-            float tt = sh.fred[half][0];
-            for (int i = 1; i < HW; i++) tt = fmaxf(tt, sh.fred[half][i]);
-            sh.hbcast[half] = tt;
-        }
-        hsync(half);
-        m = sh.hbcast[half];
-        float l = 0.f;
-        for (uint32_t i = ht; i < nk; i += RG_HALF) {
-            float e = (float)exp((double)__fsub_rn(scores[i], m));
-            scores[i] = e;
-            l += e;
-        }
-        l = warp_sum(l);
-        hsync(half);
-        if (lane == 0) sh.fred[half][hwarp] = l;
-        hsync(half);
-        if (ht == 0) {
-            float tt = 0.f;
-            for (int i = 0; i < HW; i++) tt += sh.fred[half][i];
-            p.part_ml[((size_t)h * S + sp) * 2 + 0] = m;
-            p.part_ml[((size_t)h * S + sp) * 2 + 1] = tt;
-        }
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (uint32_t base = 0; base < nk; base += KG * AU) {
-            if (base) {
-#pragma unroll
-                for (int u = 0; u < AU; u++) {
-                    const uint32_t key = base + kg + u * KG;
-                    vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t key = base + kg + u * KG;
-                if (key < nk) {
-                    const float sc = scores[key];
-                    acc.x = fmaf(vf[u].x, sc, acc.x); acc.y = fmaf(vf[u].y, sc, acc.y);
-                    acc.z = fmaf(vf[u].z, sc, acc.z); acc.w = fmaf(vf[u].w, sc, acc.w);
-                }
-            }
-        }
-        pv[ht] = acc;
-        hsync(half);
-        if (ht < HD) {
-            const float *pvf = reinterpret_cast<const float *>(pv);
-            float r = 0.f;
-            for (int i = 0; i < KG; i++) r += pvf[i * HD + ht];
-            p.part_o[((size_t)h * S + sp) * HD + ht] = r;
-        }
-        hsync(half);
-    }
-}
-
 // dynamic shared memory: [ring: n_slots x RG_SLOT][scores: 2 x chunk_cap floats][RingShared]
 template <typename WT, int HD, int ND, int NF>
 __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingParams p) {
@@ -646,7 +434,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
     __syncthreads();   // the only CTA-wide barrier: after it the producer warp and the consumers never meet again
 
     RingPos pos;        // the producer's next slot to fill / the consumers' next slot to read
-    pos.slot = 0; pos.par = 0;
+    pos.slot = 0; pos.phase = 0;
     const uint32_t ring_base = smem_u32(ring);
     if (producer) {
         if (threadIdx.x != RG_CTHREADS) return;   // one thread drives the copy engine
@@ -679,7 +467,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             if (p.p2p_wait_in) p2p_wait(p.p2p_flags + 0, p2p_seq + 1);
             if (p.p2p_x_out) p2p_wait(p.p2p_flags + 1, p2p_seq);
         }
-        ccsync();
+        csync<RG_CTHREADS>();
     }
     const float *xin = p.x;
     if (p.tok_embeddings) xin = p.tok_embeddings + (size_t)p.tokens[p.state[1]] * dim;  // GetRows, llama.go:244
@@ -704,12 +492,12 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             consume<WT, 1, 0, ND>(dim, xs, p.qkv, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 2);
-        grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 0));
+        grid_barrier<RG_CTHREADS>(p.barrier, target, gridDim.x, false, arr(li, 0));
         stamp(li, 3);
         // ---- P2: RoPE, KV store, split attention partials (llama.go:274-333)
-        attention_phase<HD>(p, L, past, sh, scores);
+        attention_phase<HD, RG_CTHREADS>(p, L, past, sh, scores);
         stamp(li, 4);
-        grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 1));
+        grid_barrier<RG_CTHREADS>(p.barrier, target, gridDim.x, false, arr(li, 1));
         stamp(li, 5);
         {   // ---- P3: merge the attention splits, wo + residual (llama.go:336-340)
             float4 xs[ND][2];
@@ -717,7 +505,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             consume<WT, 1, 1, ND>(dim, xs, p.y, xin, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 6);
-        grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 2));
+        grid_barrier<RG_CTHREADS>(p.barrier, target, gridDim.x, false, arr(li, 2));
         stamp(li, 7);
         {   // ---- P4: rmsnorm * ffn_norm, silu(w1.)*(w3.) (llama.go:346-361)
             float4 xs[ND][2];
@@ -726,7 +514,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             consume<WT, 2, 0, ND>(dim, xs, p.act, nullptr, pos, phidx++, ring_base, sh, n_slots, p.spin_ns);
         }
         stamp(li, 9);
-        grid_barrier(p.barrier, target, gridDim.x, false, arr(li, 3));
+        grid_barrier<RG_CTHREADS>(p.barrier, target, gridDim.x, false, arr(li, 3));
         stamp(li, 10);
         {   // ---- P5: w2 + residual (llama.go:363-366); the stage's last layer writes the residual into the next stage's x
             float4 xf[NF][2];
@@ -735,7 +523,7 @@ __global__ void __launch_bounds__(RG_THREADS, 1) decode_ring_kernel(const RingPa
             consume<WT, 1, 1, NF>(ff, xf, to_peer ? p.p2p_x_out : p.x, p.y, pos, phidx++, ring_base, sh, n_slots, p.spin_ns, to_peer);
         }
         stamp(li, 11);
-        grid_barrier(p.barrier, target, gridDim.x, p.p2p_x_out != nullptr && li + 1 == p.n_layers, arr(li, 4));
+        grid_barrier<RG_CTHREADS>(p.barrier, target, gridDim.x, p.p2p_x_out != nullptr && li + 1 == p.n_layers, arr(li, 4));
         stamp(li, 12);
         xin = p.x;
     }

@@ -19,7 +19,8 @@
 //     memory, refilled synchronously by the consumers while the ring keeps the HBM stream going); per (tile,
 //     pass) the 16 warps' partial 16 x 8 tiles are combined through shared memory in a fixed order
 //     (deterministic) and accumulated across passes.
-// Attention / RMSNorm / RoPE numerics: kernels_mega.cu.
+// Attention / RMSNorm / RoPE numerics: kernels_mega.cu; the attention phase (attention_pods), merge statistics, grid
+// barrier and PTX wrappers are shared with the other decode kernels (megakernel.cuh).
 #include <cooperative_groups.h>
 #include <cuda.h>
 #include <stdlib.h>
@@ -27,16 +28,15 @@
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "megakernel.cuh"
 
 namespace lb {
 namespace k {
 namespace {
 
 constexpr int RP_CWARPS = 16;
-constexpr int RP_WARPS = RP_CWARPS;                // (name used by the attention code)
 constexpr int RP_CTHREADS = RP_CWARPS * 32;
 constexpr int RP_ALL_THREADS = RP_CTHREADS + 32;   // + the producer warp
-constexpr int RP_HALF = RP_CTHREADS / 2;
 constexpr int RP_MAXB = 8;
 constexpr int RP_SEG = 256;                        // floats of K per slot row
 constexpr int RP_ROWS = 16;
@@ -47,62 +47,6 @@ constexpr uint32_t RP_PASS_SEGS = 8;               // segments per K pass
 constexpr uint32_t RP_XS_F4 = RP_PASS_SEGS * 16 * 32;   // float4 slots of the activation stage (64 KB): [chunk][pod][t]
 constexpr int RP_MAX_ITEMS = 2 * kNumSMs + 64;
 constexpr int RP_MAX_TILES = 16;                   // 16-row tiles of a CTA per matrix (x2 for the w1/w3 pair)
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ccsync() { asm volatile("bar.sync 1, %0;" ::"n"(RP_CTHREADS) : "memory"); }   // consumers only
-__device__ __forceinline__ void hsync(int half) { asm volatile("bar.sync %0, %1;" ::"r"(2 + half), "n"(RP_HALF) : "memory"); }
-__device__ __forceinline__ float4 ldcg4(const float *p) { return __ldcg(reinterpret_cast<const float4 *>(p)); }
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// (try_wait suspends the thread in hardware for a bounded time; the spin counter only exists so that a pipeline bug traps
-//  instead of hanging the box — no clock read per iteration: ncu r02n counted 3.5-6.5 % CS2R instructions in the ring kernels)
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t spins = 0;
-    while (true) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (++spins > (1u << 24)) __trap();
-    }
-}
-// 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (TMA engine, no tensor map)
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-
-
-
-// D(16x8, f32) += A(16x8, tf32, row) * B(8x8, tf32, col)
-__device__ __forceinline__ void mma_tf32(float (&d)[4], float a0, float a1, float a2, float a3, float b0, float b1) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(__float_as_uint(a0)), "r"(__float_as_uint(a1)), "r"(__float_as_uint(a2)), "r"(__float_as_uint(a3)),
-          "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
-// v - trunc_tf32(v): exact in FP32 (the tensor core reads only the upper 19 bits of an operand register)
-__device__ __forceinline__ float tf32_lo(float v) { return v - __uint_as_float(__float_as_uint(v) & 0xFFFFE000u); }
-__device__ __forceinline__ float4 tf32_lo4(float4 v) { return make_float4(tf32_lo(v.x), tf32_lo(v.y), tf32_lo(v.z), tf32_lo(v.w)); }
 
 // 3-D tiled load (k, row, layer) -> dense [16][256] floats in shared memory, ONE instruction per slot: 1-D bulk copies
 // of 1 KB per row were measured copy-engine bound (~75 clk per copy instruction, 4 TB/s; profiles/README.md)
@@ -195,27 +139,6 @@ struct RPShared {
     float mrg_m[RP_MAX_ITEMS], mrg_l[RP_MAX_ITEMS], mrg_w[RP_MAX_ITEMS], mrg_inv[RP_MAX_ITEMS];
 };
 
-__device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned &target, unsigned nctas) {
-    target += nctas;
-    ccsync();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(bar, 1u);
-        const long long t0 = clock64();
-        while (ld_acquire_u32(bar) < target) {
-            if (clock64() - t0 > 4000000000LL) __trap();
-        }
-        __threadfence();
-    }
-    ccsync();
-}
-struct RingPos {
-    uint32_t slot, phase;
-    __device__ __forceinline__ void next(uint32_t n_slots) {
-        if (++slot == n_slots) { slot = 0; phase ^= 1; }
-    }
-};
-
 // ---------------------------------------------------------------------------------------------------------
 // producer: for K pass, for tile, for segment of the pass (, for matrix): one slot
 // ---------------------------------------------------------------------------------------------------------
@@ -233,7 +156,7 @@ __device__ __forceinline__ void produce(const CUtensorMap *mapA, const CUtensorM
 #pragma unroll
                 for (int m = 0; m < NM; m++) {
                     const uint32_t fb = smem_u32(&sh.full[pos.slot]);
-                    mbar_wait(smem_u32(&sh.empty[pos.slot]), pos.phase ^ 1);
+                    mbar_wait<(1u << 24)>(smem_u32(&sh.empty[pos.slot]), pos.phase ^ 1);
                     mbar_expect_tx(fb, RP_SLOT);   // rows past the matrix end are zero-filled by the copy engine and still counted
                     if (rp.chunk != 0xFFFFFFFFu)
                         tma_load_4d(ring_base + pos.slot * RP_SLOT, m == 0 ? chunkA : chunkB, fb, (int)(seg * RP_SEG), (int)(tile - r0), (int)rp.chunk, layer);
@@ -309,7 +232,7 @@ __device__ __forceinline__ void fill_pass(float4 *xs, const float *src, uint32_t
             }
         }
     }
-    ccsync();
+    csync<RP_CTHREADS>();
 }
 
 // RMSNorm scales of the B rows sh.xrow[] (f64 sums of squares of FP32 products, ml.go:1788-1808)
@@ -336,41 +259,14 @@ __device__ __forceinline__ void rms_scales(uint32_t K, uint32_t B, RPShared &sh)
     acc += __shfl_xor_sync(0xffffffffu, acc, 1);
     acc += __shfl_xor_sync(0xffffffffu, acc, 2);
     if (t == 0) sh.red[warp][pod] = acc;
-    ccsync();
+    csync<RP_CTHREADS>();
     if (threadIdx.x < RP_MAXB) {
         double s = 0.0;
 #pragma unroll
         for (int i = 0; i < RP_CWARPS; i++) s += sh.red[i][threadIdx.x];
         sh.scale[threadIdx.x] = (float)(1.0 / sqrt(s / (double)K + 1e-5));
     }
-    ccsync();
-}
-
-// statistics of the attention splits (S > 1) for the merge done by fill_pass<2>
-__device__ __forceinline__ void merge_stats(const RPParams &p, RPShared &sh) {
-    const uint32_t S = p.splits, BH = p.B * p.heads, items = BH * S;
-    for (uint32_t i = threadIdx.x; i < items; i += RP_CTHREADS) {
-        const float2 ml = __ldcg(reinterpret_cast<const float2 *>(p.part_ml) + i);
-        sh.mrg_m[i] = ml.x;
-        sh.mrg_l[i] = ml.y;
-    }
-    ccsync();
-    for (uint32_t bh = threadIdx.x; bh < BH; bh += RP_CTHREADS) {
-        float M = -INFINITY;
-        for (uint32_t s = 0; s < S; s++) M = fmaxf(M, sh.mrg_m[bh * S + s]);
-        float Lsum = 0.f;
-        for (uint32_t s = 0; s < S; s++) {
-            const float l = sh.mrg_l[bh * S + s];
-            float wgt = 0.f;
-            if (l > 0.f) {
-                wgt = expf(__fsub_rn(sh.mrg_m[bh * S + s], M));
-                Lsum = fmaf(l, wgt, Lsum);
-            }
-            sh.mrg_w[bh * S + s] = wgt;
-        }
-        sh.mrg_inv[bh] = __fdiv_rn(1.0f, Lsum);
-    }
-    ccsync();
+    csync<RP_CTHREADS>();
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -404,7 +300,7 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const float *xsr
                 const float4 xl = tf32_lo4(xv);
 #pragma unroll
                 for (int m = 0; m < NM; m++) {
-                    mbar_wait(smem_u32(&sh.full[pos.slot]), pos.phase);
+                    mbar_wait<(1u << 24)>(smem_u32(&sh.full[pos.slot]), pos.phase);
                     const uint8_t *sl = ring + (size_t)pos.slot * RP_SLOT + wofs;
                     const float4 wa = *reinterpret_cast<const float4 *>(sl);
                     const float4 wb = *reinterpret_cast<const float4 *>(sl + 8 * RP_PITCH);
@@ -429,7 +325,7 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const float *xsr
                 *reinterpret_cast<float2 *>(pw + g * 8 + 2 * t) = make_float2(d0, d1);         // (row g,     pods 2t, 2t+1)
                 *reinterpret_cast<float2 *>(pw + (g + 8) * 8 + 2 * t) = make_float2(d2, d3);   // (row g + 8, pods 2t, 2t+1)
             }
-            ccsync();
+            csync<RP_CTHREADS>();
             if (threadIdx.x < 128) {
                 const uint32_t row = tile + (threadIdx.x >> 3), pod = threadIdx.x & 7;
                 float s1v = 0.f, s3v = 0.f;
@@ -456,142 +352,12 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const float *xsr
                     out[(size_t)pod * ldo + row] = v;
                 }
             }
-            if (NM == 2) ccsync();   // single-buffered partials in the two-matrix phase
+            if (NM == 2) csync<RP_CTHREADS>();   // single-buffered partials in the two-matrix phase
             else buf ^= 1;
         }
-        if (ps + 1 < npass) ccsync();   // every warp is done with this pass's activation stage before it is refilled
+        if (ps + 1 < npass) csync<RP_CTHREADS>();   // every warp is done with this pass's activation stage before it is refilled
     }
 }
-
-template <int HD>
-__device__ __forceinline__ void attention_pods(const RPParams &p, size_t layer_off, RPShared &sh, float *scores_all) {
-    constexpr int LANES = HD / 4;
-    constexpr int HW = RP_WARPS / 2;
-    constexpr int KG = RP_HALF / LANES;
-    constexpr int AU = 8;
-    const int half = threadIdx.x / RP_HALF, ht = threadIdx.x % RP_HALF;
-    const int hwarp = ht >> 5, lane = threadIdx.x & 31;
-    const uint32_t dim = p.dim, S = p.splits;
-    const float scale = (float)(1.0 / sqrt((double)HD));  // f32(1/sqrt(dim/heads)), llama.go:306
-    const uint32_t items = p.B * p.heads * S;
-    float *scores = scores_all + (size_t)half * p.chunk_cap;
-    float4 *pv = sh.pv + half * RP_HALF;
-    const uint32_t kg = ht / LANES, dl = ht % LANES;
-    for (uint32_t item = blockIdx.x * 2 + half; item < items; item += gridDim.x * 2) {
-        const uint32_t sp = item % S, bh = item / S, h = bh % p.heads, b = bh / p.heads;
-        const uint32_t past = p.pasts[b], Tn = past + 1;
-        const uint32_t chunk = min((Tn + S - 1) / S, p.chunk_cap);
-        const uint32_t t0 = min(sp * chunk, Tn), t1 = min(t0 + chunk, Tn), nk = t1 - t0;
-        float *Kh = p.Kb[b] + layer_off + (size_t)h * HD;
-        float *Vh = p.Vb[b] + layer_off + (size_t)h * HD;
-        const float *qkv = p.qkv + (size_t)b * 3 * dim;
-        float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (lane < LANES) {
-            const float4 qr = ldcg4(qkv + (size_t)h * HD + lane * 4);
-            const double c0 = sh.rope_cs[b][lane * 2][0], s0 = sh.rope_cs[b][lane * 2][1];
-            const double c1 = sh.rope_cs[b][lane * 2 + 1][0], s1 = sh.rope_cs[b][lane * 2 + 1][1];
-            qv.x = (float)(__dsub_rn(__dmul_rn((double)qr.x, c0), __dmul_rn((double)qr.y, s0)));
-            qv.y = (float)(__dadd_rn(__dmul_rn((double)qr.x, s0), __dmul_rn((double)qr.y, c0)));
-            qv.z = (float)(__dsub_rn(__dmul_rn((double)qr.z, c1), __dmul_rn((double)qr.w, s1)));
-            qv.w = (float)(__dadd_rn(__dmul_rn((double)qr.z, s1), __dmul_rn((double)qr.w, c1)));
-            if (hwarp == 0 && past >= t0 && past < t1) {  // the item that owns position `past` stores the new K (rotated) and V rows
-                const float4 kr = ldcg4(qkv + dim + (size_t)h * HD + lane * 4);
-                float4 ko;
-                ko.x = (float)(__dsub_rn(__dmul_rn((double)kr.x, c0), __dmul_rn((double)kr.y, s0)));
-                ko.y = (float)(__dadd_rn(__dmul_rn((double)kr.x, s0), __dmul_rn((double)kr.y, c0)));
-                ko.z = (float)(__dsub_rn(__dmul_rn((double)kr.z, c1), __dmul_rn((double)kr.w, s1)));
-                ko.w = (float)(__dadd_rn(__dmul_rn((double)kr.z, s1), __dmul_rn((double)kr.w, c1)));
-                *reinterpret_cast<float4 *>(Kh + (size_t)past * dim + lane * 4) = ko;
-                *reinterpret_cast<float4 *>(Vh + (size_t)past * dim + lane * 4) = ldcg4(qkv + 2 * dim + (size_t)h * HD + lane * 4);
-            }
-        }
-        hsync(half);
-        for (uint32_t i = hwarp; i < nk; i += HW * AU) {
-            float4 kk[AU];
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                kk[u] = (ii < nk && lane < LANES) ? ldcg4(Kh + (size_t)(t0 + ii) * dim + lane * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                float dd = kk[u].x * qv.x;
-                dd = fmaf(kk[u].y, qv.y, dd); dd = fmaf(kk[u].z, qv.z, dd); dd = fmaf(kk[u].w, qv.w, dd);
-                dd = warp_sum(dd);
-                if (lane == 0 && ii < nk) scores[ii] = __fmul_rn(dd, scale);
-            }
-        }
-        float4 vf[AU];
-#pragma unroll
-        for (int u = 0; u < AU; u++) {
-            const uint32_t key = kg + u * KG;
-            vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        hsync(half);
-        float m = -INFINITY;
-        for (uint32_t i = ht; i < nk; i += RP_HALF) m = fmaxf(m, scores[i]);
-        m = warp_max(m);
-        if (lane == 0) sh.fred[half][hwarp] = m;
-        hsync(half);
-        if (ht == 0) {
-            float tt = sh.fred[half][0];
-            for (int i = 1; i < HW; i++) tt = fmaxf(tt, sh.fred[half][i]);
-            sh.hbcast[half] = tt;
-        }
-        hsync(half);
-        m = sh.hbcast[half];
-        float l = 0.f;
-        for (uint32_t i = ht; i < nk; i += RP_HALF) {
-            float e = (float)exp((double)__fsub_rn(scores[i], m));
-            scores[i] = e;
-            l += e;
-        }
-        l = warp_sum(l);
-        hsync(half);
-        if (lane == 0) sh.fred[half][hwarp] = l;
-        hsync(half);
-        if (ht == 0) {
-            float tt = 0.f;
-            for (int i = 0; i < HW; i++) tt += sh.fred[half][i];
-            sh.hbcast[half] = tt;
-            if (S > 1) {
-                p.part_ml[((size_t)bh * S + sp) * 2 + 0] = m;
-                p.part_ml[((size_t)bh * S + sp) * 2 + 1] = tt;
-            }
-        }
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (uint32_t base = 0; base < nk; base += KG * AU) {
-            if (base) {
-#pragma unroll
-                for (int u = 0; u < AU; u++) {
-                    const uint32_t key = base + kg + u * KG;
-                    vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t key = base + kg + u * KG;
-                if (key < nk) {
-                    const float sc = scores[key];
-                    acc.x = fmaf(vf[u].x, sc, acc.x); acc.y = fmaf(vf[u].y, sc, acc.y);
-                    acc.z = fmaf(vf[u].z, sc, acc.z); acc.w = fmaf(vf[u].w, sc, acc.w);
-                }
-            }
-        }
-        pv[ht] = acc;
-        hsync(half);  // also publishes hbcast = l
-        if (ht < HD) {
-            const float *pvf = reinterpret_cast<const float *>(pv);
-            float r = 0.f;
-            for (int i = 0; i < KG; i++) r += pvf[i * HD + ht];
-            if (S > 1) p.part_o[((size_t)bh * S + sp) * HD + ht] = r;
-            else p.attn[(size_t)b * dim + (size_t)h * HD + ht] = __fmul_rn(r, __fdiv_rn(1.0f, sh.hbcast[half]));  // p = e * f32(1/sum), ml.go:2493-2499
-        }
-        hsync(half);
-    }
-}
-
 
 // dynamic shared memory: [ring: n_slots x RP_SLOT][xs: 64 KB (attention scores overlay it)][RPShared]
 template <int HD>
@@ -657,39 +423,39 @@ __global__ void __launch_bounds__(RP_ALL_THREADS, 1) decode_ring_pods_kernel(con
         stamp(li, 1);
         consume<1, 0, 1, HD>(dim, 3 * dim, nullptr, 0, L.attention_norm, p.qkv, 3 * dim, nullptr, 0, ph, pos, ring, xs, p, sh);
         stamp(li, 2);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RP_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 3);
         // ---- P2: RoPE, KV store, attention (llama.go:274-333)
-        attention_pods<HD>(p, layer_off, sh, scores);
+        attention_pods<HD, RP_CTHREADS>(p, layer_off, sh, scores);
         stamp(li, 4);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RP_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 5);
         // ---- P3: wo + residual (llama.go:336-340)
         if (p.splits > 1) {
-            merge_stats(p, sh);
+            merge_stats<RP_CTHREADS>(p, p.B * p.heads, sh);
             consume<1, 1, 2, HD>(dim, dim, nullptr, 0, nullptr, p.y, dim, nullptr, 0, ph, pos, ring, xs, p, sh);
         } else {
             consume<1, 1, 0, HD>(dim, dim, p.attn, dim, nullptr, p.y, dim, nullptr, 0, ph, pos, ring, xs, p, sh);
         }
         stamp(li, 6);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RP_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 7);
         // ---- P4: rmsnorm * ffn_norm, silu(w1.)*(w3.) (llama.go:346-361)
         if (threadIdx.x < RP_MAXB) sh.xrow[threadIdx.x] = threadIdx.x < B ? p.y + (size_t)threadIdx.x * dim : nullptr;
-        ccsync();
+        csync<RP_CTHREADS>();
         rms_scales(dim, B, sh);
         stamp(li, 8);
         consume<2, 0, 1, HD>(dim, ff, nullptr, 0, L.ffn_norm, p.act, ff, nullptr, 0, ph, pos, ring, xs, p, sh);
         stamp(li, 9);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RP_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 10);
         // ---- P5: w2 + residual (llama.go:363-366)
         consume<1, 1, 0, HD>(ff, dim, p.act, ff, nullptr, p.x, dim, p.y, dim, ph, pos, ring, xs, p, sh);
         stamp(li, 11);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RP_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 12);
         if (threadIdx.x < RP_MAXB) sh.xrow[threadIdx.x] = threadIdx.x < B ? p.x + (size_t)threadIdx.x * dim : nullptr;
-        ccsync();
+        csync<RP_CTHREADS>();
     }
     if (p.final_norm) {  // final norm + lm_head (llama.go:374-384)
         rms_scales(dim, B, sh);

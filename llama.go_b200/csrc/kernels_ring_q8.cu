@@ -19,13 +19,15 @@
 //     ~24 instructions per 512 weights instead of ~1800.
 // The result differs from "the FP32 path on the dequantised weights d*q" (the parity target, tests/test_gpu_q8.py)
 // only by summation order and the 2^-28 digit truncation.
-// Attention / RMSNorm / RoPE numerics: kernels_mega.cu.
+// Attention / RMSNorm / RoPE numerics: kernels_mega.cu; the attention phase, grid barrier and PTX wrappers are shared
+// with the other decode kernels (megakernel.cuh).
 #include <cooperative_groups.h>
 #include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
 #include "kernels.cuh"
+#include "megakernel.cuh"
 
 namespace lb {
 namespace k {
@@ -34,7 +36,6 @@ namespace {
 constexpr int RQ_CWARPS = 16;
 constexpr int RQ_CTHREADS = RQ_CWARPS * 32;
 constexpr int RQ_THREADS = RQ_CTHREADS + 32;       // + the producer warp
-constexpr int RQ_HALF = RQ_CTHREADS / 2;
 constexpr uint32_t RQ_SEGK = 1024;                 // k per slot row
 constexpr uint32_t RQ_ROWS = 16;
 constexpr uint32_t RQ_BLKQ = RQ_ROWS * 32;                     // int8 bytes of one 32-column block of a tile: [16 rows][32]
@@ -45,49 +46,6 @@ constexpr int RQ_MAX_SLOTS = 10;
 constexpr int RQ_MAX_ITEMS = 2 * kNumSMs;
 constexpr int RQ_MAX_HEADS = 256;
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ccsync() { asm volatile("bar.sync 1, %0;" ::"n"(RQ_CTHREADS) : "memory"); }   // consumers only
-__device__ __forceinline__ void hsync(int half) { asm volatile("bar.sync %0, %1;" ::"r"(2 + half), "n"(RQ_HALF) : "memory"); }
-__device__ __forceinline__ float4 ldcg4(const float *p) { return __ldcg(reinterpret_cast<const float4 *>(p)); }
-__device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-// (try_wait suspends the thread in hardware for a bounded time; the spin counter only exists so that a pipeline bug traps
-//  instead of hanging the box — no clock read per iteration: ncu r02n counted 3.5-6.5 % CS2R instructions in the ring kernels)
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, uint32_t backoff_ns = 0) {
-    uint32_t spins = 0;
-    while (true) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (backoff_ns) __nanosleep(backoff_ns);   // 16 warps polling one mbarrier compete with the producer's and the copy engine's updates of it
-        if (++spins > (1u << 24)) __trap();
-    }
-}
-
-// 1-D bulk copy global -> shared, completion counted in bytes on an mbarrier (TMA engine, no tensor map)
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
 // D(16x8, s32) = A(16x32, s8, row) * B(32x8, s8, col)
 __device__ __forceinline__ void mma_s8(int (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
     asm volatile(
@@ -137,24 +95,6 @@ struct RQShared {
     float mrg_m[RQ_MAX_ITEMS], mrg_l[RQ_MAX_ITEMS], mrg_w[RQ_MAX_ITEMS], mrg_inv[RQ_MAX_HEADS];
 };
 
-// ---- grid barrier among the consumer threads of all CTAs (the producer warps never take part)
-__device__ __forceinline__ void grid_barrier(unsigned *bar, unsigned &target, unsigned nctas) {
-    target += nctas;
-    ccsync();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(bar, 1u);
-        const long long t0 = clock64();
-        while (ld_acquire_u32(bar) < target) {
-            if (clock64() - t0 > 4000000000LL) __trap();
-        }
-        __threadfence();
-    }
-    ccsync();
-}
-
-
-
 // Rows of an M-row matrix owned by this CTA in MulMat phase number `ph`: whole 16-row tiles (a TMA box never fetches
 // rows the CTA does not use), ceil(M/16) tiles dealt out evenly; WHICH CTAs get the extra tile rotates with the phase
 // number, and the run-ahead of the ring lets a CTA that is short one tile in this phase start on the next phase's
@@ -197,13 +137,6 @@ __device__ __forceinline__ void cta_rows(uint32_t M, uint32_t ph, uint32_t &r0, 
     rq_rows_of(M, (blockIdx.x + ph * 37u) % gridDim.x, gridDim.x, r0, r1);
 }
 
-struct RingPos {
-    uint32_t slot, phase;
-    __device__ __forceinline__ void next(uint32_t n_slots) {
-        if (++slot == n_slots) { slot = 0; phase ^= 1; }
-    }
-};
-
 // ---------------------------------------------------------------------------------------------------------
 // producer (one thread): for tile, for segment (, for matrix): one contiguous record of the tile-major plane per slot
 // ---------------------------------------------------------------------------------------------------------
@@ -222,7 +155,7 @@ __device__ __forceinline__ void produce(const uint8_t *PA, const uint8_t *PB, ui
 #pragma unroll
             for (int m = 0; m < NM; m++) {
                 const uint32_t fb = smem_u32(&sh.full[pos.slot]);
-                mbar_wait(smem_u32(&sh.empty[pos.slot]), pos.phase ^ 1);
+                mbar_wait<(1u << 24)>(smem_u32(&sh.empty[pos.slot]), pos.phase ^ 1);
                 mbar_expect_tx(fb, bytes);
                 bulk_g2s(ring_base + pos.slot * RQ_SLOT, (m == 0 ? PA : PB) + tbase + (size_t)seg * (RQ_SEGK / 32) * rt * 36u, bytes, fb);
                 pos.next(n_slots);
@@ -305,7 +238,7 @@ __device__ __forceinline__ void norm_digits(const float *x, const float *w, uint
     }
     acc = warp_sum(acc);
     if (lane == 0) sh.red[warp] = acc;
-    ccsync();
+    csync<RQ_CTHREADS>();
     double t = 0.0;
 #pragma unroll
     for (int i = 0; i < RQ_CWARPS; i++) t += sh.red[i];
@@ -322,7 +255,7 @@ __device__ __forceinline__ void norm_digits(const float *x, const float *w, uint
     for (uint32_t f = threadIdx.x + R * RQ_CTHREADS; f < K / 4; f += RQ_CTHREADS)
         emit4(f, nrm(ldcg4(x + (size_t)f * 4), __ldg(reinterpret_cast<const float4 *>(w) + f)), dig, xsc);
     zero_blocks(K / 32, kp / 32, dig, xsc);
-    ccsync();   // also orders sh.red against its next use
+    csync<RQ_CTHREADS>();   // also orders sh.red against its next use
 }
 __device__ __forceinline__ void plain_digits(const float *x, uint32_t K, uint32_t kp, int8_t *dig, float *xsc) {
     constexpr int PB = 6;   // float4 per thread per batch of loads: one L2 round trip per 12288 elements
@@ -340,34 +273,13 @@ __device__ __forceinline__ void plain_digits(const float *x, uint32_t K, uint32_
         }
     }
     zero_blocks(K / 32, kp / 32, dig, xsc);
-    ccsync();
+    csync<RQ_CTHREADS>();
 }
-// digits of the merged attention output (see kernels_mega.cu::merged_attention_slice): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s)
+// digits of the merged attention output (statistics: merge_stats, megakernel.cuh): out = (sum_s O_s w_s) * f32(1 / sum_s l_s w_s)
 template <int HD>
 __device__ __forceinline__ void merge_digits(const RQParams &p, uint32_t kp, int8_t *dig, float *xsc, RQShared &sh) {
-    const uint32_t S = p.splits, items = p.heads * S;
-    for (uint32_t i = threadIdx.x; i < items; i += RQ_CTHREADS) {
-        const float2 ml = __ldcg(reinterpret_cast<const float2 *>(p.part_ml) + i);
-        sh.mrg_m[i] = ml.x;
-        sh.mrg_l[i] = ml.y;
-    }
-    ccsync();
-    for (uint32_t h = threadIdx.x; h < p.heads; h += RQ_CTHREADS) {
-        float M = -INFINITY;
-        for (uint32_t s2 = 0; s2 < S; s2++) M = fmaxf(M, sh.mrg_m[h * S + s2]);
-        float Lsum = 0.f;
-        for (uint32_t s2 = 0; s2 < S; s2++) {
-            const float l = sh.mrg_l[h * S + s2];
-            float wgt = 0.f;
-            if (l > 0.f) {
-                wgt = expf(__fsub_rn(sh.mrg_m[h * S + s2], M));
-                Lsum = fmaf(l, wgt, Lsum);
-            }
-            sh.mrg_w[h * S + s2] = wgt;
-        }
-        sh.mrg_inv[h] = __fdiv_rn(1.0f, Lsum);
-    }
-    ccsync();
+    const uint32_t S = p.splits;
+    merge_stats<RQ_CTHREADS>(p, p.heads, sh);
     constexpr int MB = 12;   // splits per batch of loads (a per-split loop of L2 reads costs one round trip per split)
     for (uint32_t f = threadIdx.x; f < p.dim / 4; f += RQ_CTHREADS) {
         const uint32_t e = f * 4, h = e / HD, d = e % HD;
@@ -390,7 +302,7 @@ __device__ __forceinline__ void merge_digits(const RQParams &p, uint32_t kp, int
         emit4(f, make_float4(__fmul_rn(o.x, inv), __fmul_rn(o.y, inv), __fmul_rn(o.z, inv), __fmul_rn(o.w, inv)), dig, xsc);
     }
     zero_blocks(p.dim / 32, kp / 32, dig, xsc);
-    ccsync();
+    csync<RQ_CTHREADS>();
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -458,7 +370,7 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const int8_t *di
             const bool fast = full_tile && nb == RQ_SEGK / 32;
 #pragma unroll
             for (int m = 0; m < NM; m++) {
-                mbar_wait(smem_u32(&sh.full[pos.slot]), pos.phase, spin_ns);
+                mbar_wait<(1u << 24)>(smem_u32(&sh.full[pos.slot]), pos.phase, spin_ns);
                 const uint32_t sl = ring_s + pos.slot * RQ_SLOT;
                 uint2 qa[2], qb[2];
                 float da[2], db[2];
@@ -519,7 +431,7 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const int8_t *di
                 sh.part[buf][m][warp][g + 8] = acc[m][1];
             }
         }
-        ccsync();
+        csync<RQ_CTHREADS>();
         if (threadIdx.x < RQ_ROWS) {
             const uint32_t row = tile + threadIdx.x;
             float s1 = 0.f, s3 = 0.f;
@@ -538,131 +450,7 @@ __device__ __forceinline__ void consume(uint32_t K, uint32_t M, const int8_t *di
         }
         buf ^= 1;
     }
-    ccsync();   // the last tile's partials are read before the next phase's prologue reuses shared memory
-}
-
-// ---- attention phase: identical to kernels_mega.cu::attention_phase (items (head, split), two per CTA at a time)
-template <int HD>
-__device__ __forceinline__ void attention_phase(const RQParams &p, const MegaLayerHost &L, uint32_t past, RQShared &sh, float *scores_all) {
-    constexpr int LANES = HD / 4;
-    constexpr int HW = RQ_CWARPS / 2;
-    constexpr int KG = RQ_HALF / LANES;
-    constexpr int AU = 8;
-    const int half = threadIdx.x / RQ_HALF, ht = threadIdx.x % RQ_HALF;
-    const int hwarp = ht >> 5, lane = threadIdx.x & 31;
-    const uint32_t dim = p.dim, S = p.splits, Tn = past + 1;
-    const float scale = (float)(1.0 / sqrt((double)HD));  // f32(1/sqrt(dim/heads)), llama.go:306
-    const uint32_t chunk = min((Tn + S - 1) / S, p.chunk_cap);
-    const uint32_t items = p.heads * S;
-    float *scores = scores_all + (size_t)half * p.chunk_cap;
-    float4 *pv = sh.pv + half * RQ_HALF;
-    const uint32_t kg = ht / LANES, dl = ht % LANES;
-    for (uint32_t item = blockIdx.x * 2 + half; item < items; item += gridDim.x * 2) {
-        const uint32_t h = item / S, sp = item % S;
-        const uint32_t t0 = min(sp * chunk, Tn), t1 = min(t0 + chunk, Tn), nk = t1 - t0;
-        float *Kh = L.Kc + (size_t)h * HD;
-        float *Vh = L.Vc + (size_t)h * HD;
-        float4 qv = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (lane < LANES) {
-            const float4 qr = ldcg4(p.qkv + (size_t)h * HD + lane * 4);
-            const double c0 = sh.rope_cs[lane * 2][0], s0 = sh.rope_cs[lane * 2][1];
-            const double c1 = sh.rope_cs[lane * 2 + 1][0], s1 = sh.rope_cs[lane * 2 + 1][1];
-            qv.x = (float)(__dsub_rn(__dmul_rn((double)qr.x, c0), __dmul_rn((double)qr.y, s0)));
-            qv.y = (float)(__dadd_rn(__dmul_rn((double)qr.x, s0), __dmul_rn((double)qr.y, c0)));
-            qv.z = (float)(__dsub_rn(__dmul_rn((double)qr.z, c1), __dmul_rn((double)qr.w, s1)));
-            qv.w = (float)(__dadd_rn(__dmul_rn((double)qr.z, s1), __dmul_rn((double)qr.w, c1)));
-            if (hwarp == 0 && past >= t0 && past < t1) {
-                const float4 kr = ldcg4(p.qkv + dim + (size_t)h * HD + lane * 4);
-                float4 ko;
-                ko.x = (float)(__dsub_rn(__dmul_rn((double)kr.x, c0), __dmul_rn((double)kr.y, s0)));
-                ko.y = (float)(__dadd_rn(__dmul_rn((double)kr.x, s0), __dmul_rn((double)kr.y, c0)));
-                ko.z = (float)(__dsub_rn(__dmul_rn((double)kr.z, c1), __dmul_rn((double)kr.w, s1)));
-                ko.w = (float)(__dadd_rn(__dmul_rn((double)kr.z, s1), __dmul_rn((double)kr.w, c1)));
-                *reinterpret_cast<float4 *>(Kh + (size_t)past * dim + lane * 4) = ko;
-                *reinterpret_cast<float4 *>(Vh + (size_t)past * dim + lane * 4) = ldcg4(p.qkv + 2 * dim + (size_t)h * HD + lane * 4);
-            }
-        }
-        hsync(half);
-        for (uint32_t i = hwarp; i < nk; i += HW * AU) {
-            float4 kk[AU];
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                kk[u] = (ii < nk && lane < LANES) ? ldcg4(Kh + (size_t)(t0 + ii) * dim + lane * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t ii = i + u * HW;
-                float dd = kk[u].x * qv.x;
-                dd = fmaf(kk[u].y, qv.y, dd); dd = fmaf(kk[u].z, qv.z, dd); dd = fmaf(kk[u].w, qv.w, dd);
-                dd = warp_sum(dd);
-                if (lane == 0 && ii < nk) scores[ii] = __fmul_rn(dd, scale);
-            }
-        }
-        float4 vf[AU];
-#pragma unroll
-        for (int u = 0; u < AU; u++) {
-            const uint32_t key = kg + u * KG;
-            vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        hsync(half);
-        float m = -INFINITY;
-        for (uint32_t i = ht; i < nk; i += RQ_HALF) m = fmaxf(m, scores[i]);
-        m = warp_max(m);
-        if (lane == 0) sh.fred[half][hwarp] = m;
-        hsync(half);
-        if (ht == 0) {
-            float tt = sh.fred[half][0];
-            for (int i = 1; i < HW; i++) tt = fmaxf(tt, sh.fred[half][i]);
-            sh.hbcast[half] = tt;
-        }
-        hsync(half);
-        m = sh.hbcast[half];
-        float l = 0.f;
-        for (uint32_t i = ht; i < nk; i += RQ_HALF) {
-            float e = (float)exp((double)__fsub_rn(scores[i], m));
-            scores[i] = e;
-            l += e;
-        }
-        l = warp_sum(l);
-        hsync(half);
-        if (lane == 0) sh.fred[half][hwarp] = l;
-        hsync(half);
-        if (ht == 0) {
-            float tt = 0.f;
-            for (int i = 0; i < HW; i++) tt += sh.fred[half][i];
-            p.part_ml[((size_t)h * S + sp) * 2 + 0] = m;
-            p.part_ml[((size_t)h * S + sp) * 2 + 1] = tt;
-        }
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (uint32_t base = 0; base < nk; base += KG * AU) {
-            if (base) {
-#pragma unroll
-                for (int u = 0; u < AU; u++) {
-                    const uint32_t key = base + kg + u * KG;
-                    vf[u] = key < nk ? ldcg4(Vh + (size_t)(t0 + key) * dim + dl * 4) : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < AU; u++) {
-                const uint32_t key = base + kg + u * KG;
-                if (key < nk) {
-                    const float sc = scores[key];
-                    acc.x = fmaf(vf[u].x, sc, acc.x); acc.y = fmaf(vf[u].y, sc, acc.y);
-                    acc.z = fmaf(vf[u].z, sc, acc.z); acc.w = fmaf(vf[u].w, sc, acc.w);
-                }
-            }
-        }
-        pv[ht] = acc;
-        hsync(half);
-        if (ht < HD) {
-            const float *pvf = reinterpret_cast<const float *>(pv);
-            float r = 0.f;
-            for (int i = 0; i < KG; i++) r += pvf[i * HD + ht];
-            p.part_o[((size_t)h * S + sp) * HD + ht] = r;
-        }
-        hsync(half);
-    }
+    csync<RQ_CTHREADS>();   // the last tile's partials are read before the next phase's prologue reuses shared memory
 }
 
 // dynamic shared memory: [ring: n_slots x RQ_SLOT][xs: kpad floats, digit planes in place][xsc: kpad/32 floats][scores][RQShared]
@@ -686,12 +474,7 @@ __global__ void __launch_bounds__(RQ_THREADS, 1) decode_ring_q8_kernel(const RQP
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     const uint32_t past = p.state[0];
-    if (threadIdx.x < HD / 2) {  // RoPE table of this token's position (f64 pow/cos/sin, ml.go:2307-2310)
-        double sn, cs;
-        sincos((double)past * pow(10000.0, ((double)(-(int)(2 * threadIdx.x))) / (double)HD), &sn, &cs);
-        sh.rope_cs[threadIdx.x][0] = cs;
-        sh.rope_cs[threadIdx.x][1] = sn;
-    }
+    rope_table<HD>(sh, past);
     __syncthreads();   // the only CTA-wide barrier
 
     RingPos pos;
@@ -729,31 +512,31 @@ __global__ void __launch_bounds__(RQ_THREADS, 1) decode_ring_q8_kernel(const RQP
         stamp(li, 1);
         consume<1, 0, 0>(dim, 3 * dim, dig, xsc, p.qkv, nullptr, ph, pos, ring, sh, n_slots, p.spin_ns);
         stamp(li, 2);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RQ_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 3);
         // ---- P2: RoPE, KV store, split attention partials (llama.go:274-333)
-        attention_phase<HD>(p, L, past, sh, scores);
+        attention_phase<HD, RQ_CTHREADS>(p, L, past, sh, scores);
         stamp(li, 4);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RQ_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 5);
         // ---- P3: merge the attention splits, wo + residual (llama.go:336-340)
         merge_digits<HD>(p, kp_dim, dig, xsc, sh);
         consume<1, 1, 0>(dim, dim, dig, xsc, p.y, xin, ph, pos, ring, sh, n_slots, p.spin_ns);
         stamp(li, 6);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RQ_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 7);
         // ---- P4: rmsnorm * ffn_norm, silu(w1.)*(w3.) (llama.go:346-361)
         norm_digits(p.y, L.ffn_norm, dim, kp_dim, dig, xsc, sh);
         stamp(li, 8);
         consume<2, 0, 0>(dim, ff, dig, xsc, p.act, nullptr, ph, pos, ring, sh, n_slots, p.spin_ns);
         stamp(li, 9);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RQ_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 10);
         // ---- P5: w2 + residual (llama.go:363-366)
         plain_digits(p.act, ff, kp_ff, dig, xsc);
         consume<1, 1, 0>(ff, dim, dig, xsc, p.x, p.y, ph, pos, ring, sh, n_slots, p.spin_ns);
         stamp(li, 11);
-        grid_barrier(p.barrier, target, gridDim.x);
+        grid_barrier<RQ_CTHREADS>(p.barrier, target, gridDim.x);
         stamp(li, 12);
         xin = p.x;
     }

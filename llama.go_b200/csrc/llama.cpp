@@ -355,9 +355,6 @@ void Context::forward(uint32_t n, bool tokens_indirect, bool all_rows, const flo
         mp.tokens = tokens_dev; mp.state = state_dev;
         mp.final_norm = model->has_head() ? model->norm : nullptr;
         mp.output = model->has_head() ? model->output : nullptr;
-        mp.q_output = model->has_head() ? model->output8.q : nullptr;
-        mp.d_output = model->has_head() ? model->output8.d : nullptr;
-        mp.q8 = model->q8();
         mp.f16 = model->f16();
         mp.h_output = model->has_head() ? model->outputh : nullptr;
         mp.x = x; mp.y = y; mp.qkv = qkv; mp.attn = attn; mp.act = act; mp.logits = logits;
