@@ -174,6 +174,21 @@ LB_API int       lb_batch_eval(lb_batch *b, const uint32_t *tokens, const uint32
 /* `steps` tokens per pod (tokens [n][steps], teacher-forced) enqueued back to back; ms_out = CUDA-event time */
 LB_API int       lb_batch_decode_resident(lb_batch *b, const uint32_t *tokens, uint32_t steps, const uint32_t *pasts, float *ms_out);
 LB_API int       lb_batch_read_logits(lb_batch *b, float *logits_out);    /* [n][vocab] of the last step */
+/* lb_sample_top_p_top_k for every pod at once, one CTA per pod on row b of the batch's last logits, with the same
+ * arithmetic (candidate set and pick bit-identical to the single-context sampler on the same row): last_n_tokens
+ * [n][n_last], seeds [n]; tokens_out [n]; cand_ids_out / cand_probs_out ([n][top_k]) and n_cand_out ([n]) optional. */
+LB_API int       lb_batch_sample(lb_batch *b, const uint32_t *last_n_tokens, uint32_t n_last, uint32_t top_k, float top_p, float temp,
+                                 float repeat_penalty, const uint64_t *seeds, uint32_t *cand_ids_out, float *cand_probs_out,
+                                 uint32_t *n_cand_out, uint32_t *tokens_out);
+/* lb_generate for every pod of the batch at once: server.Engine's --pods jobs (pkg/server/server.go:84-237) as one call.
+ * Pod b's prompt is the next n_prompts[b] ids of `prompts` (concatenated), its seed seeds[b]; predict and the sampling
+ * parameters are shared.  Each prompt goes through its pod's own context in batches of batch_size, with the same context
+ * swap as lb_generate; then every generated token is one batched device sample + one pod-batch step (one pass over the
+ * weights for all pods), with no host round trip except where a pod's context swap is due (:158-172).  out_tokens
+ * receives [n][predict] ids; decode_ms_out (optional) the CUDA-event time of the decode phase (first sample to last). */
+LB_API int       lb_batch_generate(lb_batch *b, const uint32_t *prompts, const uint32_t *n_prompts, uint32_t predict, uint32_t top_k,
+                                   float top_p, float temp, float repeat_penalty, uint32_t keep_count, uint32_t batch_size,
+                                   const uint64_t *seeds, uint32_t *out_tokens, float *decode_ms_out);
 /* profiling aid, like lb_context_mega_trace: 13 globaltimer stamps per layer of the last pod-batch step (LB_MEGA_TRACE=1) */
 LB_API int       lb_batch_mega_trace(lb_batch *b, uint64_t *out, uint32_t n);
 

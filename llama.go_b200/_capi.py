@@ -70,6 +70,10 @@ _SIGS = {
     "lb_batch_decode_resident": (C.c_int, [_vp, _u32p, C.c_uint32, _u32p, _f32p]),
     "lb_batch_read_logits": (C.c_int, [_vp, _f32p]),
     "lb_batch_mega_trace": (C.c_int, [_vp, C.POINTER(C.c_uint64), C.c_uint32]),
+    "lb_batch_sample": (C.c_int, [_vp, _u32p, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float, C.POINTER(C.c_uint64), _u32p,
+                                  _f32p, _u32p, _u32p]),
+    "lb_batch_generate": (C.c_int, [_vp, _u32p, _u32p, C.c_uint32, C.c_uint32, C.c_float, C.c_float, C.c_float, C.c_uint32, C.c_uint32,
+                                    C.POINTER(C.c_uint64), _u32p, _f32p]),
     "lb_comm_unique_id": (C.c_int, [_vp]),
     "lb_comm_init": (C.c_int, [_vp, C.c_int, C.c_int, C.c_int]),
     "lb_comm_destroy": (None, []),

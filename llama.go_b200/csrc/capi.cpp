@@ -244,6 +244,21 @@ int lb_batch_mega_trace(lb_batch *b, uint64_t *out, uint32_t n) {
                LB_CUDA(cudaMemcpy(out, x->mega_trace, (size_t)n * sizeof(uint64_t), cudaMemcpyDeviceToHost)));
 }
 int lb_batch_read_logits(lb_batch *b, float *logits_out) { LB_TRY_INT(LB_CHECK(b && logits_out, "nil argument"); b->b->read_logits(logits_out)); }
+int lb_batch_sample(lb_batch *b, const uint32_t *last_n_tokens, uint32_t n_last, uint32_t top_k, float top_p, float temp,
+                    float repeat_penalty, const uint64_t *seeds, uint32_t *cand_ids_out, float *cand_probs_out, uint32_t *n_cand_out,
+                    uint32_t *tokens_out) {
+    LB_TRY_INT(LB_CHECK(b, "nil batch");
+               b->b->sample(last_n_tokens, n_last, top_k, top_p, temp, repeat_penalty, seeds, cand_ids_out, cand_probs_out, n_cand_out,
+                            tokens_out));
+}
+int lb_batch_generate(lb_batch *b, const uint32_t *prompts, const uint32_t *n_prompts, uint32_t predict, uint32_t top_k, float top_p,
+                      float temp, float repeat_penalty, uint32_t keep_count, uint32_t batch_size, const uint64_t *seeds,
+                      uint32_t *out_tokens, float *decode_ms_out) {
+    LB_TRY_INT(LB_CHECK(b, "nil batch");
+               float ms = b->b->generate(prompts, n_prompts, predict, top_k, top_p, temp, repeat_penalty, keep_count, batch_size, seeds,
+                                         out_tokens);
+               if (decode_ms_out) *decode_ms_out = ms);
+}
 
 // ---- multi-GPU pipeline ----
 int lb_comm_unique_id(void *out128) { LB_TRY_INT(LB_CHECK(out128, "nil argument"); pipe::unique_id(out128)); }

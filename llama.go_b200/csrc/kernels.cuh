@@ -115,6 +115,22 @@ size_t sample_top_p_top_k_smem(uint32_t V, uint32_t top_k);
 void sample_top_p_top_k(const float *logits, uint32_t V, const uint32_t *last_n_dev, uint32_t n_last, uint32_t top_k, float top_p,
                         float temp, float penalty, uint64_t seed, uint32_t *out_ids, float *out_probs, uint32_t *out_n_token,
                         cudaStream_t st);
+// device state of the pods generate loop (every pointer device memory; all nullptr for a one-shot batch sample)
+struct PodSampleState {
+    uint32_t *ring = nullptr;       // [B][n_last] last-N ids (the sampler's last_n rows): the pick is appended at ring_pos
+    uint32_t *ring_pos = nullptr;   // [B]
+    uint32_t *produced = nullptr;   // [B] ids sampled so far: seed offset and column of `out`
+    uint32_t *out = nullptr;        // [B][out_stride]
+    uint32_t out_stride = 0;
+    uint32_t *tokens = nullptr;     // [B][tok_stride]: the pick goes to column state[1], read by the next pod step
+    uint32_t tok_stride = 0;
+    const uint32_t *state = nullptr;
+};
+// the same sampler on B rows of logits ([B][V]), one CTA per pod: last_n rows n_last apart, pod b seeded with
+// seeds_dev[b] (+ g.produced[b]); out_ids/out_probs [B][top_k], out_n/out_tok [B] (all optional)
+void sample_top_p_top_k_pods(const float *logits, uint32_t V, uint32_t B, const uint32_t *last_n_dev, uint32_t n_last, uint32_t top_k,
+                             float top_p, float temp, float penalty, const uint64_t *seeds_dev, uint32_t *out_ids, float *out_probs,
+                             uint32_t *out_n, uint32_t *out_tok, const PodSampleState &g, cudaStream_t st);
 // state[0] (= past) += dp; state[1] (= step) += ds; if seq != nullptr, *seq += 1 (pipeline hand-off step counter)
 void advance_state(uint32_t *state, uint32_t dp, uint32_t ds, cudaStream_t st, uint32_t *seq = nullptr);
 

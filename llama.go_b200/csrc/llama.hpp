@@ -179,17 +179,36 @@ struct PodBatch {
     std::vector<uint8_t> tmaps;         // TMA tensor maps of the weight matrices (k::ring_pods_make_maps)
     const void *tmaps_ptr = nullptr;
     void *mega_trace = nullptr;         // LB_MEGA_TRACE=1: per-phase globaltimer stamps of CTA 0 (TMA-ring variant)
+    // batched sampler (allocated on first use): generate loop state [B][ctx] ring, [B] ring position / produced count,
+    // [B][out_cap] sampled ids; one-shot sample inputs / outputs
+    uint32_t *ring_dev = nullptr, *ring_pos_dev = nullptr, *produced_dev = nullptr, *out_dev = nullptr;
+    uint32_t out_cap = 0;
+    uint64_t *seeds_dev = nullptr;
+    uint32_t *smp_last_dev = nullptr, *smp_ids_dev = nullptr, *smp_n_dev = nullptr, *smp_tok_dev = nullptr;
+    float *smp_probs_dev = nullptr;
+    uint32_t smp_last_cap = 0;
 
     explicit PodBatch(const std::vector<Context *> &ctxs);
     ~PodBatch();
     void eval(const uint32_t *tokens, const uint32_t *pasts, float *logits_out);          // one token per pod, host buffers
     float decode_resident(const uint32_t *tokens, uint32_t steps, const uint32_t *pasts);  // teacher-forced, device timed
     void read_logits(float *out);
+    // Context::sample for every pod at once, on the batch's last logits: last_n [B][n_last], seeds [B]; tokens_out [B];
+    // ids_out / probs_out ([B][top_k]) and n_out ([B]) optional, as in Context::sample
+    void sample(const uint32_t *last_n, uint32_t n_last, uint32_t top_k, float top_p, float temp, float repeat_penalty,
+                const uint64_t *seeds, uint32_t *ids_out, float *probs_out, uint32_t *n_out, uint32_t *tokens_out);
+    // Context::generate (server.Do's loop) for every pod: pod b's prompt is the next n_prompts[b] ids of `prompts`, its
+    // seed seeds[b]; the prompts go through each pod's own Context, then every step is one batched sample + one pod step
+    // with no host round trip, except where a pod's context swap is due.  out_tokens [B][predict]; returns the CUDA-event
+    // time of the decode phase in ms
+    float generate(const uint32_t *prompts, const uint32_t *n_prompts, uint32_t predict, uint32_t top_k, float top_p, float temp,
+                   float repeat_penalty, uint32_t keep_count, uint32_t batch_size, const uint64_t *seeds, uint32_t *out_tokens);
 
    private:
     void forward();
     void ensure_graph();
     void stage_inputs(const uint32_t *tokens, uint32_t steps, const uint32_t *pasts);
+    void ensure_sampler(uint32_t predict);
 };
 
 }  // namespace llama

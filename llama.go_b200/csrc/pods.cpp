@@ -210,5 +210,176 @@ void PodBatch::read_logits(float *out) {
     LB_CUDA(cudaMemcpy(out, logits, (size_t)B * model->hp.vocab * sizeof(float), cudaMemcpyDeviceToHost));
 }
 
+void PodBatch::ensure_sampler(uint32_t predict) {
+    const uint32_t V = model->hp.vocab;
+    if (!ring_dev) {
+        ring_dev = mem.dmalloc<uint32_t>((size_t)B * ctx_size);
+        ring_pos_dev = mem.dmalloc<uint32_t>(B);
+        produced_dev = mem.dmalloc<uint32_t>(B);
+        seeds_dev = mem.dmalloc<uint64_t>(B);
+        smp_ids_dev = mem.dmalloc<uint32_t>((size_t)B * V);
+        smp_probs_dev = mem.dmalloc<float>((size_t)B * V);
+        smp_n_dev = mem.dmalloc<uint32_t>(B);
+        smp_tok_dev = mem.dmalloc<uint32_t>(B);
+    }
+    if (predict > out_cap) {
+        out_cap = predict;
+        out_dev = mem.dmalloc<uint32_t>((size_t)B * out_cap, false);
+    }
+}
+
+void PodBatch::sample(const uint32_t *last_n, uint32_t n_last, uint32_t top_k, float top_p, float temp, float repeat_penalty,
+                      const uint64_t *seeds, uint32_t *ids_out, float *probs_out, uint32_t *n_out, uint32_t *tokens_out) {
+    LB_CHECK(last_n || !n_last, "SampleTopPTopK : nil lastNTokens");
+    LB_CHECK(seeds && tokens_out, "pod batch: nil argument");
+    LB_CHECK(top_k >= 1 && top_k <= model->hp.vocab, "SampleTopPTopK : topK must be in 1..vocab");
+    LB_CUDA(cudaSetDevice(model->device));
+    ensure_sampler(0);
+    if (n_last > smp_last_cap) {
+        smp_last_cap = n_last;
+        smp_last_dev = mem.dmalloc<uint32_t>((size_t)B * smp_last_cap, false);
+    }
+    LB_CUDA(cudaStreamSynchronize(stream));   // the previous call's buffers are idle before they are overwritten
+    if (n_last) LB_CUDA(cudaMemcpyAsync(smp_last_dev, last_n, (size_t)B * n_last * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    LB_CUDA(cudaMemcpyAsync(seeds_dev, seeds, B * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    k::sample_top_p_top_k_pods(logits, model->hp.vocab, B, smp_last_dev, n_last, top_k, top_p, temp, repeat_penalty, seeds_dev,
+                               smp_ids_dev, smp_probs_dev, smp_n_dev, smp_tok_dev, k::PodSampleState(), stream);
+    std::vector<uint32_t> n(B);
+    LB_CUDA(cudaMemcpyAsync(n.data(), smp_n_dev, B * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    LB_CUDA(cudaMemcpyAsync(tokens_out, smp_tok_dev, B * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    if (ids_out) LB_CUDA(cudaMemcpyAsync(ids_out, smp_ids_dev, (size_t)B * top_k * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    if (probs_out) LB_CUDA(cudaMemcpyAsync(probs_out, smp_probs_dev, (size_t)B * top_k * sizeof(float), cudaMemcpyDeviceToHost, stream));
+    LB_CUDA(cudaStreamSynchronize(stream));
+    if (n_out) memcpy(n_out, n.data(), B * sizeof(uint32_t));
+}
+
+// server.Do (server.go:127-237) for B jobs at once.  Context::generate's loop, restated per pod:
+//   prompt phase: each pod's prompt in batch_size chunks through its own Context, with the same context_swap; the last
+//     row of logits is copied into row b of the batch logits, so every pod's first sample is a batched one;
+//   decode phase: [batched sample] then (predict - 1) x [pod step, batched sample].  A pod step evaluates each pod's
+//     pending token at its own position, and every position grows by one per step, so the host knows the first step at
+//     which some pod's pending token would land at past == ctx_size.  Every step up to there is enqueued as one segment
+//     with no host synchronisation (segments also restart at kTokensCap steps, the token buffer's width).
+//   context swap (server.go:165-172) of a pod that is due: its device ring, oldest first, goes through context_swap with
+//     embd = [pending]; the re-fed prefix (which ends with the pending id itself, as in the reference) is evaluated
+//     through the pod's Context at keep_count in one eval, and its past becomes keep_count + n_front.  The next pod step
+//     then evaluates the pending id: the same tokens at the same positions as the reference's single Eval(embd).
+// The last sampled id is never evaluated (server.go:153-237).
+float PodBatch::generate(const uint32_t *prompts, const uint32_t *n_prompts, uint32_t predict, uint32_t top_k, float top_p, float temp,
+                         float repeat_penalty, uint32_t keep_count, uint32_t batch_size, const uint64_t *seeds, uint32_t *out_tokens) {
+    const HParams &hp = model->hp;
+    const uint32_t V = hp.vocab;
+    LB_CHECK(prompts && n_prompts && seeds && out_tokens && predict >= 1 && batch_size >= 1, "generate : bad arguments");
+    std::vector<size_t> first(B);
+    size_t off = 0;
+    for (uint32_t b = 0; b < B; b++) {
+        LB_CHECK(n_prompts[b] >= 1, "generate : bad arguments");
+        first[b] = off;
+        for (uint32_t i = 0; i < n_prompts[b]; i++) LB_CHECK(prompts[off + i] < V, "generate : token id out of range");
+        off += n_prompts[b];
+    }
+    LB_CHECK(top_k >= 1 && top_k <= V, "SampleTopPTopK : topK must be in 1..vocab");
+    LB_CHECK(temp > 0.f, "SampleTopPTopK : temp must be > 0 (the reference replaces 0 by 0.5, main.go:379-381)");
+    LB_CHECK(keep_count < ctx_size, "generate : keep_count must be smaller than the context size");
+    LB_CUDA(cudaSetDevice(model->device));
+    ensure_sampler(predict);
+    LB_CUDA(cudaStreamSynchronize(stream));
+
+    // ---- prompt phase, per pod (Context::generate until its first sample)
+    std::vector<uint32_t> ring((size_t)B * ctx_size, 0u), ring_pos(B, 0u), past(B, 0u), produced(B, 0u);
+    std::vector<uint32_t> embd, tmp((size_t)ctx_size * 2 + batch_size);
+    for (uint32_t b = 0; b < B; b++) {
+        uint32_t *rb = ring.data() + (size_t)b * ctx_size;
+        const uint32_t *prompt = prompts + first[b];
+        uint32_t consumed = 0;
+        embd.clear();
+        for (;;) {
+            if (!embd.empty()) {
+                if ((uint64_t)past[b] + embd.size() > ctx_size) {   // server.go:165-172
+                    std::vector<uint32_t> h(ctx_size);
+                    for (uint32_t i = 0; i < ctx_size; i++) h[i] = rb[(ring_pos[b] + i) % ctx_size];
+                    const int64_t n = context_swap(ctx_size, keep_count, h.data(), ctx_size, &past[b], embd.data(), (uint32_t)embd.size(),
+                                                   tmp.data(), (uint32_t)tmp.size());
+                    embd.assign(tmp.begin(), tmp.begin() + n);
+                }
+                ctxs[b]->eval(embd.data(), (uint32_t)embd.size(), past[b], nullptr, false);   // synchronous
+            }
+            past[b] += (uint32_t)embd.size();
+            embd.clear();
+            if (consumed == n_prompts[b]) break;
+            while (consumed < n_prompts[b] && embd.size() < batch_size) {
+                embd.push_back(prompt[consumed]);
+                rb[ring_pos[b]] = prompt[consumed];
+                ring_pos[b] = (ring_pos[b] + 1) % ctx_size;
+                consumed++;
+            }
+        }
+        LB_CUDA(cudaMemcpyAsync(logits + (size_t)b * V, ctxs[b]->logits, V * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+    }
+    // pageable sources: each copy returns once its data is staged, in stream order before the sampler
+    LB_CUDA(cudaMemcpyAsync(ring_dev, ring.data(), ring.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    LB_CUDA(cudaMemcpyAsync(ring_pos_dev, ring_pos.data(), B * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    LB_CUDA(cudaMemcpyAsync(produced_dev, produced.data(), B * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    LB_CUDA(cudaMemcpyAsync(seeds_dev, seeds, B * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    pasts_host[8] = 0; pasts_host[9] = 0;   // state {unused, step}: the first sample writes token column 0
+    LB_CUDA(cudaMemcpyAsync(state_dev, pasts_host + 8, 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    LB_CUDA(cudaStreamSynchronize(stream));
+
+    // ---- decode phase
+    k::PodSampleState g;
+    g.ring = ring_dev; g.ring_pos = ring_pos_dev; g.produced = produced_dev; g.out = out_dev; g.out_stride = out_cap;
+    g.tokens = tokens_dev; g.tok_stride = kTokensCap; g.state = state_dev;
+    auto sample_all = [&]() {
+        k::sample_top_p_top_k_pods(logits, V, B, ring_dev, ctx_size, top_k, top_p, temp, repeat_penalty, seeds_dev, nullptr, nullptr,
+                                   nullptr, nullptr, g, stream);
+    };
+    LB_CUDA(cudaEventRecord(ev0, stream));
+    sample_all();
+    const uint32_t steps = predict - 1;
+    uint32_t done = 0, col = 0;   // col = token column holding the pending ids (= state[1] on the device)
+    while (done < steps) {
+        LB_CUDA(cudaStreamSynchronize(stream));
+        for (uint32_t b = 0; b < B; b++) {
+            if (past[b] < ctx_size) continue;
+            std::vector<uint32_t> rb(ctx_size), h(ctx_size);
+            uint32_t pos = 0;
+            LB_CUDA(cudaMemcpy(rb.data(), ring_dev + (size_t)b * ctx_size, ctx_size * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+            LB_CUDA(cudaMemcpy(&pos, ring_pos_dev + b, sizeof(uint32_t), cudaMemcpyDeviceToHost));
+            for (uint32_t i = 0; i < ctx_size; i++) h[i] = rb[(pos + i) % ctx_size];
+            const uint32_t pending = h[ctx_size - 1];   // the ring already ends with the pending id (server.go:207-211)
+            const int64_t n = context_swap(ctx_size, keep_count, h.data(), ctx_size, &past[b], &pending, 1, tmp.data(), (uint32_t)tmp.size());
+            if (n > 1) ctxs[b]->eval(tmp.data(), (uint32_t)(n - 1), past[b], nullptr, false);
+            past[b] += (uint32_t)(n - 1);
+        }
+        uint32_t seg = steps - done < kTokensCap - 1 ? steps - done : kTokensCap - 1;
+        for (uint32_t b = 0; b < B; b++) seg = ctx_size - past[b] < seg ? ctx_size - past[b] : seg;
+        if (col) {   // move the pending ids to column 0 and restart the step counter
+            LB_CUDA(cudaMemcpy2DAsync(tokens_dev, kTokensCap * sizeof(uint32_t), tokens_dev + col, kTokensCap * sizeof(uint32_t),
+                                      sizeof(uint32_t), B, cudaMemcpyDeviceToDevice, stream));
+            col = 0;
+        }
+        for (uint32_t b = 0; b < B; b++) pasts_host[b] = past[b];
+        pasts_host[8] = 0; pasts_host[9] = 0;
+        LB_CUDA(cudaMemcpyAsync(pasts_dev, pasts_host, B * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+        LB_CUDA(cudaMemcpyAsync(state_dev, pasts_host + 8, 2 * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+        ensure_graph();   // first use: an eager run of this very step, then capture (ensure_graph restores pasts / state)
+        for (uint32_t i = 0; i < seg; i++) {
+            LB_CUDA(cudaGraphLaunch(graph, stream));
+            count_launch(use_mega ? 2 : model->layers.size() * 8 + 4);
+            sample_all();
+        }
+        for (uint32_t b = 0; b < B; b++) past[b] += seg;
+        col = seg;
+        done += seg;
+    }
+    LB_CUDA(cudaEventRecord(ev1, stream));
+    LB_CUDA(cudaMemcpy2DAsync(out_tokens, predict * sizeof(uint32_t), out_dev, out_cap * sizeof(uint32_t), predict * sizeof(uint32_t), B,
+                              cudaMemcpyDeviceToHost, stream));
+    LB_CUDA(cudaStreamSynchronize(stream));
+    float ms = 0.f;
+    LB_CUDA(cudaEventElapsedTime(&ms, ev0, ev1));
+    return ms;
+}
+
 }  // namespace llama
 }  // namespace lb

@@ -230,6 +230,48 @@ class PodBatch:
         check(lib().lb_batch_read_logits(self._h, out.ctypes.data_as(_f32p)))
         return out
 
+    def _seeds(self, seeds, what):
+        s = np.ascontiguousarray(range(len(self.ctxs)) if seeds is None else seeds, dtype=np.uint64).reshape(-1)
+        if s.size != len(self.ctxs):
+            raise ValueError(f"PodBatch.{what}: need one seed per pod")
+        return s, s.ctypes.data_as(C.POINTER(C.c_uint64))
+
+    def SampleTopPTopK(self, lastN, topK: int = 40, topP: float = 0.95, temp: float = 0.8, repeatPenalty: float = 1.10, seeds=None):
+        """SampleTopPTopK for every pod on the batch's last logits (row b with lastN[b] and seeds[b], default b).  Returns
+        (tokens [n], candidate ids per pod, candidate probabilities per pod), as llama.SampleTopPTopK does for one context."""
+        n = len(self.ctxs)
+        last = np.ascontiguousarray(lastN, dtype=np.uint32)
+        if last.ndim != 2 or last.shape[0] != n:
+            raise ValueError("PodBatch.SampleTopPTopK: lastN must be [pods][n_last]")
+        s, sp = self._seeds(seeds, "SampleTopPTopK")
+        ids = np.zeros((n, topK), np.uint32)
+        probs = np.zeros((n, topK), np.float32)
+        cnt = np.zeros(n, np.uint32)
+        toks = np.zeros(n, np.uint32)
+        check(lib().lb_batch_sample(self._h, last.ctypes.data_as(_u32p), last.shape[1], topK, topP, temp, repeatPenalty, sp,
+                                    ids.ctypes.data_as(_u32p), probs.ctypes.data_as(_f32p), cnt.ctypes.data_as(_u32p),
+                                    toks.ctypes.data_as(_u32p)))
+        return toks.tolist(), [ids[b, :cnt[b]].copy() for b in range(n)], [probs[b, :cnt[b]].copy() for b in range(n)]
+
+    def Generate(self, prompts, predict: int, topK: int = 40, topP: float = 0.95, temp: float = 0.8, repeatPenalty: float = 1.10,
+                 keepCount: int = 0, batchSize: int | None = None, seeds=None, return_ms: bool = False):
+        """llama.Generate for every pod at once (pkg/server.Do per job, server.go:127-237): prompts[b] on pod b with
+        seeds[b] (default b).  Returns one list of `predict` ids per pod (and the decode phase's CUDA-event ms if
+        return_ms)."""
+        n = len(self.ctxs)
+        if len(prompts) != n:
+            raise ValueError("PodBatch.Generate: need one prompt per pod")
+        lens = np.asarray([len(p) for p in prompts], np.uint32)
+        cat = np.ascontiguousarray(np.concatenate([np.asarray(p, np.uint32).reshape(-1) for p in prompts]), dtype=np.uint32)
+        s, sp = self._seeds(seeds, "Generate")
+        out = np.zeros((n, predict), np.uint32)
+        ms = C.c_float(0)
+        check(lib().lb_batch_generate(self._h, cat.ctypes.data_as(_u32p), lens.ctypes.data_as(_u32p), predict, topK, topP, temp,
+                                      repeatPenalty, keepCount, self.ctxs[0].ctx_size if batchSize is None else batchSize, sp,
+                                      out.ctypes.data_as(_u32p), C.byref(ms)))
+        toks = [row.tolist() for row in out]
+        return (toks, ms.value) if return_ms else toks
+
     def free(self):
         if self._h:
             lib().lb_batch_free(self._h)
